@@ -3,6 +3,7 @@
 edges/sec; aggregation GB/s against the measured roofs of the box; transforms against the tensor peak).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode fp32|bf16] [--quick]
+                    [--dump-outputs DIR]
 
 One *step* = train-mode ``DrugDiseaseModel.forward`` on the full graph + BCEWithLogits + ``backward()``
 (reference src/train.py:291-306; optimiser, clipping and sampling excluded, SURVEY.md §8d).
@@ -27,6 +28,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 import torch.nn.functional as F
 
@@ -45,6 +47,7 @@ PARITY = ("operator restated, not PyG-pinned (torch_geometric is not installable
 # SURVEY.md §8d: algorithmic bytes of one cfg2 step in the reference's (dense) formulation
 CFG2_STEP_BYTES = 2_406.3e6
 PART = dict(nodes_per_gpu=1_250_000, edges_per_gpu=50_000_000, relations=30, layers=3, embedding=64, hidden=128, batch=2048)
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
 
 
 def measured_peaks():
@@ -125,6 +128,30 @@ def make_workload(rank: int):
     kg = synth.primekg_subgraph(CFG["num_edges"], seed=CFG["seed"])
     batch = synth.link_batch(kg, CFG["batch_pos"], seed=CFG["seed"] + 1000 * rank)   # a different mini-batch per rank
     return kg, batch
+
+
+def rewind_dropout_counters(model):
+    """Set the device-side step counters of the fused dropout (the layers' and the decoder's) back to 0.  A step's masks
+    hash (seed, counter, element) and the untimed pre-roll runs as many steps as fit its time window, so without this
+    the masks of the timed steps, and every output of them, would change from run to run."""
+    for m in model.modules():
+        ctr = getattr(m, "_drop_ctr", None)
+        if ctr is not None:
+            ctr.zero_()
+        rng = getattr(m, "_drop_rng", None)
+        if rng is not None:
+            rng[1].zero_()
+
+
+def dump_outputs(out_dir, gstep, model):
+    """What the last step handed its caller, as float32 ``out_dir/<name>.npy``: the loss, the scores of the batch's
+    pairs and every parameter gradient (``grad.<parameter name>``)."""
+    arrays = {"loss": gstep.loss, "scores": gstep.scores}
+    arrays.update((f"grad.{k}", p.grad) for k, p in model.named_parameters() if p.grad is not None)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def algorithmic_bytes(E, N, R, d_in):
@@ -574,6 +601,9 @@ def run_ours(args, rank, world, local_rank):
     params = [p for p in model.parameters()]
     flush = Flusher(dev)
     d_batch = [t.to(dev) for t in (heads, tails, rels, labels)]
+    dump_bytes = 4 * (1 + d_batch[0].numel() + sum(p.numel() for p in params))     # loss, scores, gradients
+    if args.dump_outputs and dump_bytes > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {dump_bytes} bytes of outputs exceed the {DUMP_LIMIT_BYTES} byte limit")
 
     def eager_step(b):
         for p in params:
@@ -700,11 +730,14 @@ def run_ours(args, rank, world, local_rank):
         for _ in range(20):
             gstep(); allreduce_grads()
         torch.cuda.synchronize()
+    rewind_dropout_counters(model)
     barrier()
     t_wall0 = time.perf_counter()
     ms_per_step = timed(lambda: (gstep(), allreduce_grads()), args.steps)
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gstep, model)
     value = world * kg.num_edges / (ms_per_step * 1e-3)
     dp_exchange_ok = None
     if peer_ar:
@@ -895,7 +928,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-partitioned", action="store_true", help="skip the node-range partitioned record")
     ap.add_argument("--quick", action="store_true", help="headline + roofline only (no other configs, no library baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, scores and parameter gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

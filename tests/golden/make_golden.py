@@ -1,7 +1,7 @@
-"""Generates the golden fixtures in this directory.  Runs ONLY in the build container, where
-/root/reference exists; the fixtures it writes are committed and travel to the GPU box.
+"""Generates the golden fixtures in this directory.  Needs a checkout of the original
+PrimeKG-RGCN-LinkPrediction project in ``$PRIMEKG_RGCN_REFERENCE``; the fixtures it writes are committed.
 
-It imports the UNMODIFIED reference ``/root/reference/src/models/rgcn.py``.  That file imports
+It imports the UNMODIFIED reference ``$PRIMEKG_RGCN_REFERENCE/src/models/rgcn.py``.  That file imports
 ``torch_geometric.nn.RGCNConv`` (third party, not installable here), so a stub module provides
 ``RGCNConv = oracle.rgcn_ref.RGCNConvRef`` — everything else (encoder wiring, ReLU/dropout placement,
 DistMult decoder, composite forward, predict_all_tails) is executed by the reference's own code.
@@ -20,7 +20,9 @@ import torch.nn.functional as F
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("PRIMEKG_RGCN_REFERENCE", "")
+if not REF or not os.path.isfile(os.path.join(REF, "src", "models", "rgcn.py")):
+    sys.exit("set PRIMEKG_RGCN_REFERENCE to a checkout of the original PrimeKG-RGCN-LinkPrediction project")
 
 from oracle import rgcn_ref  # noqa: E402
 

@@ -1,6 +1,7 @@
 """Generates tests/golden/ref_call_sequence.json: the sequence of model-API calls the reference's UNMODIFIED
 src/train.py (main(), two epochs) and src/evaluate.py (load_model, ModelEvaluator scoring + ranking loops) make on the
-drop-in module trio, recorded on this CPU box (kernels = tests/cpu_ops_emulation.py).  Needs /root/reference.
+drop-in module trio, recorded on the CPU (kernels = tests/cpu_ops_emulation.py).  Needs a checkout of the original
+project in ``$PRIMEKG_RGCN_REFERENCE``.
 
     python tests/golden/make_ref_calls.py
 """

@@ -1,8 +1,10 @@
-"""TEST INFRASTRUCTURE: drives the reference's OWN scripts (``/root/reference/src/train.py``, ``src/evaluate.py``,
-loaded from where they lie, never copied) on top of this repo's drop-in ``src/models/rgcn.py``, and records the sequence
-of model-API calls they make.  Used by ``tests/test_reference_scripts.py`` (CPU box: kernels replaced by
-``tests/cpu_ops_emulation.py``) and by ``tests/golden/make_ref_calls.py`` (writes ``tests/golden/ref_call_sequence.json``,
-which ``tests/test_gpu_reference_calls.py`` replays against the real kernels on the B200)."""
+"""TEST INFRASTRUCTURE: drives the reference's OWN scripts (``src/train.py``, ``src/evaluate.py`` of the checkout of the
+original PrimeKG-RGCN-LinkPrediction project named by ``$PRIMEKG_RGCN_REFERENCE``, loaded from where they lie, never
+copied) on top of this repo's drop-in ``src/models/rgcn.py``, and records the sequence of model-API calls they make.
+Used by ``tests/test_reference_scripts.py`` (CPU: kernels replaced by ``tests/cpu_ops_emulation.py``) and by
+``tests/golden/make_ref_calls.py`` (writes ``tests/golden/ref_call_sequence.json``, which
+``tests/test_reference_call_replay.py`` drives through the drop-in on the CPU and ``tests/test_gpu_reference_calls.py``
+replays against the real kernels on the B200)."""
 import contextlib
 import importlib.util
 import os
@@ -11,11 +13,12 @@ import types
 
 import torch
 
-REF = "/root/reference"
+# the original project is not part of this repository: the tests that run its scripts skip without it
+REF = os.environ.get("PRIMEKG_RGCN_REFERENCE", "")
 
 
 def reference_present() -> bool:
-    return os.path.isfile(os.path.join(REF, "src", "train.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "src", "train.py"))
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -87,7 +90,7 @@ def _stub_plotting_modules():
 
 
 def load_reference_script(name: str):
-    """Import /root/reference/src/<name>.py as a module.  Its ``from src.models.rgcn import DrugDiseaseModel`` finds this
+    """Import the reference's src/<name>.py as a module.  Its ``from src.models.rgcn import DrugDiseaseModel`` finds this
     repo's ``src`` package, which is imported (and therefore in ``sys.modules``) first."""
     import src.models.rgcn as shim                       # this repo's drop-in
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -100,7 +103,7 @@ def load_reference_script(name: str):
     try:
         spec.loader.exec_module(mod)
     finally:
-        sys.path[:] = before                             # the script prepends /root/reference to sys.path
+        sys.path[:] = before                             # the script prepends the reference root to sys.path
     assert mod.DrugDiseaseModel is shim.DrugDiseaseModel
     return mod
 

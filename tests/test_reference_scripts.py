@@ -1,5 +1,6 @@
 """The north_star boundary claim, exercised: the reference's OWN ``src/train.py`` and ``src/evaluate.py`` — imported
-from /root/reference where they lie, unmodified — run on top of this repo's drop-in ``src/models/rgcn.py``.
+from the checkout of the original project named by ``$PRIMEKG_RGCN_REFERENCE``, where they lie, unmodified — run on
+top of this repo's drop-in ``src/models/rgcn.py``.
 
 No GPU here, so the kernels under the module trio are the CPU stand-ins of tests/cpu_ops_emulation.py (same role as in
 tests/test_dist.py); everything above them — constructors, ``.to(device)``, the graph cache, autograd wiring of both
@@ -16,7 +17,8 @@ import torch
 import ref_harness as H
 from conftest import GOLDEN
 
-pytestmark = pytest.mark.skipif(not H.reference_present(), reason="/root/reference is not present on this machine")
+pytestmark = pytest.mark.skipif(not H.reference_present(),
+                                reason="needs a checkout of the original project: set PRIMEKG_RGCN_REFERENCE")
 
 
 @pytest.fixture(scope="module")
