@@ -2,10 +2,12 @@
 
 Per step: positives in -> negatives drawn on the device -> full-graph 2-layer RGCN forward -> fused decoder + BCE loss +
 accuracy -> backward, all replayed as ONE CUDA graph (``GraphedTrainStep`` with a ``NegativeSampler``), then the
-reference's own clipping and Adam step (src/train.py:311-318).  Loss and accuracy stay on the device and are read once per
-logging interval instead of twice per step (src/train.py:322, :325).
+reference's own clipping and Adam step (src/train.py:311-318).  ``--optimizer fused`` passes a ``FusedAdam(max_grad_norm=1.0)``
+into the graphed step instead: clipping and Adam become the last kernels of the same graph, one replay per iteration.
+Loss and accuracy stay on the device and are read once per logging interval instead of twice per step (src/train.py:322,
+:325).
 
-    python examples/train_synthetic.py [--steps 300] [--hidden 128] [--batch 1024]
+    python examples/train_synthetic.py [--steps 300] [--hidden 128] [--batch 1024] [--optimizer torch|fused]
 """
 import argparse
 import os
@@ -26,6 +28,7 @@ def main():
     ap.add_argument("--batch", type=int, default=1024)
     ap.add_argument("--lr", type=float, default=0.01)
     ap.add_argument("--edges", type=int, default=849_456)
+    ap.add_argument("--optimizer", choices=("torch", "fused"), default="torch")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     torch.manual_seed(42)
@@ -33,9 +36,12 @@ def main():
     ei, et = kg.edge_index.to(dev), kg.edge_type.to(dev)
     model = pkg.DrugDiseaseModel(kg.num_nodes, kg.num_relations, 64, args.hidden, dropout=0.5, decoder_dropout=0.1).to(dev)
     model.train()
-    opt = torch.optim.Adam(model.parameters(), lr=args.lr)
+    fused = args.optimizer == "fused"
+    opt = (pkg.FusedAdam(model.parameters(), lr=args.lr, max_grad_norm=1.0) if fused
+           else torch.optim.Adam(model.parameters(), lr=args.lr))
     sampler = pkg.NegativeSampler(kg.num_nodes, 1)
-    step = pkg.GraphedTrainStep(model, ei, et, batch_size=2 * args.batch, sampler=sampler)
+    step = pkg.GraphedTrainStep(model, ei, et, batch_size=2 * args.batch, sampler=sampler,
+                                optimizer=opt if fused else None)
     params = [p for p in model.parameters()]
     perm = torch.randperm(kg.num_edges, device=dev)
     loss_sum = torch.zeros((), device=dev)
@@ -46,8 +52,9 @@ def main():
         lo = (it * args.batch) % (kg.num_edges - args.batch)
         idx = perm[lo:lo + args.batch]
         loss = step.run_positives(ei[0, idx], ei[1, idx], et[idx])           # src/train.py:276-306 as one graph replay
-        torch.nn.utils.clip_grad_norm_(params, 1.0)                            # src/train.py:311-315
-        opt.step()                                                             # src/train.py:317
+        if not fused:                                                          # (fused: inside the replay)
+            torch.nn.utils.clip_grad_norm_(params, 1.0)                        # src/train.py:311-315
+            opt.step()                                                         # src/train.py:317
         loss_sum += loss
         correct_sum += step.correct
         if (it + 1) % 50 == 0:                                                 # one host read per logging interval

@@ -607,6 +607,50 @@ int rgcn_link_loss_bwd_rows(const float* emb, int64_t ld, const int64_t* head, c
 int rgcn_check_pairs(const int64_t* head, const int64_t* tail, const int64_t* rel, int64_t n_pairs,
                      int64_t n_nodes, int32_t n_rel, int32_t* flag, rgcn_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Optimiser step.  Replaces torch.nn.utils.clip_grad_norm_(params, max_norm) + torch.optim.Adam / AdamW .step()
+ * (reference src/train.py:311-318) with two kernels (one without clipping) over a table of parameter segments.
+ *
+ *   clipping (max_grad_norm >= 0): total_norm = ||all grads||_2 (per-block partial sums, fp64, reduced in a fixed
+ *     order: bitwise run-to-run deterministic), clip_coef = min(max_grad_norm / (total_norm + 1e-6), 1);
+ *     *grad_norm = total_norm (nullable).  The clipped gradient is used on the fly; grad is NOT written.
+ *   update, per element, in the order of torch.optim.Adam's single-tensor path (fp32; the per-step scalars in fp64
+ *     from the segment's step + 1, rounded to fp32):
+ *     g = grad * clip_coef;  decoupled ? p *= 1 - lr*wd : g += wd*p  (when wd != 0);  m = lerp(m, g, 1 - beta1);
+ *     v = beta2*v + (1 - beta2)*g*g;  p -= lr / (1 - beta1^t) * m / (sqrt(v) / sqrt(1 - beta2^t) + eps);
+ *     and every segment's *step += 1 once all blocks have read it.
+ *
+ *   segments_host : host array of n_segments (at most RGCN_ADAM_MAX_SEGMENTS) descriptors, passed to the kernels BY
+ *                   VALUE (a captured CUDA graph keeps the pointers; no table copy).  param / exp_avg / exp_avg_sq /
+ *                   grad are fp32 [numel]; step is one fp32 (torch's state['step']); group indexes hparams.
+ *   hparams       : DEVICE array of n_groups rgcn_adam_hparams, read by every launch (an lr change between replays of
+ *                   a captured step takes effect without re-capturing).
+ *   workspace     : rgcn_adam_workspace_bytes(total numel of the segments, n_segments) bytes, ZEROED once before first
+ *                   use (it holds two arrival counters that every call leaves at zero).
+ * n_segments == 0 enqueues nothing; it loads the kernels, so that a later call under stream capture loads no module.
+ * ------------------------------------------------------------------------------------------ */
+#define RGCN_ADAM_MAX_SEGMENTS 64
+
+typedef struct rgcn_adam_segment {
+  float* param;
+  const float* grad;
+  float* exp_avg;
+  float* exp_avg_sq;
+  float* step;
+  int64_t numel;
+  int32_t group;
+} rgcn_adam_segment;
+
+typedef struct rgcn_adam_hparams {
+  double lr, beta1, beta2, eps, weight_decay;
+  int32_t decoupled_weight_decay; /* 1: AdamW's p *= 1 - lr*wd; 0: Adam's L2 term g += wd*p */
+} rgcn_adam_hparams;
+
+size_t rgcn_adam_workspace_bytes(int64_t total_numel, int32_t n_segments);
+int rgcn_adam_step(const rgcn_adam_segment* segments_host, int32_t n_segments, const rgcn_adam_hparams* hparams,
+                   int32_t n_groups, float max_grad_norm, float* grad_norm, void* workspace, size_t workspace_bytes,
+                   rgcn_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

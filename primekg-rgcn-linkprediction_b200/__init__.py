@@ -11,8 +11,9 @@ from .graphed import GraphedTrainStep
 from .rank import rank_true_tails, ranking_metrics, score_all_pairs, topk_all_pairs
 from .modules import DrugDiseaseModel, DrugDiseaseRGCN, LinkPredictor
 from .sampler import NegativeSampler
+from .optim import FusedAdam, FusedAdamW
 
 __all__ = ["RGCNConv", "DrugDiseaseRGCN", "LinkPredictor", "DrugDiseaseModel", "RelGraph", "get_graph",
            "clear_graph_cache", "default_mode", "GraphedTrainStep", "graph_state", "graph_from_state", "register_graph", "rank_true_tails", "ranking_metrics", "score_all_pairs", "topk_all_pairs",
-           "NegativeSampler"]
+           "NegativeSampler", "FusedAdam", "FusedAdamW"]
 __version__ = "0.1.0"

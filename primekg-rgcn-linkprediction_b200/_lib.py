@@ -63,6 +63,20 @@ class LayerBwdArgs(C.Structure):
                 ("next_G", C.POINTER(MaskedPlanesOut)), ("g_ready", i32), ("n_colsum_ready", i32), ("slot_ready", i32),
                 ("w_planes", p), ("a_compact", i32), ("csr_fwd", PCSR), ("src_flag", p)]
 
+ADAM_MAX_SEGMENTS = 64   # RGCN_ADAM_MAX_SEGMENTS
+
+
+class AdamSegment(C.Structure):
+    """Mirror of ``rgcn_adam_segment`` (include/rgcn_b200.h)."""
+    _fields_ = [("param", p), ("grad", p), ("exp_avg", p), ("exp_avg_sq", p), ("step", p), ("numel", i64),
+                ("group", i32)]
+
+
+class AdamHparams(C.Structure):
+    """Mirror of ``rgcn_adam_hparams`` (include/rgcn_b200.h)."""
+    _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
+                ("weight_decay", C.c_double), ("decoupled_weight_decay", i32)]
+
 # name -> (restype, argtypes); must list every symbol of include/rgcn_b200.h
 PROTOTYPES = {
     "rgcn_abi_version": (C.c_int, []),
@@ -134,6 +148,8 @@ PROTOTYPES = {
     "rgcn_link_loss_bwd_rows": (C.c_int, [p, i64, p, p, p, p, p, p, p, p, i64, i32, C.c_float, u32, p, i64, i32, p, i64, p,
                                           p, p, p, i32, p, sz, p]),
     "rgcn_check_pairs": (C.c_int, [p, p, p, i64, i64, i32, p, p]),
+    "rgcn_adam_workspace_bytes": (sz, [i64, i32]),
+    "rgcn_adam_step": (C.c_int, [C.POINTER(AdamSegment), i32, p, i32, C.c_float, p, p, sz, p]),
 }
 
 

@@ -5,7 +5,8 @@ limiter.  ``GraphedTrainStep`` captures one step — ``model(edge_index, edge_ty
 ``BCEWithLogitsLoss`` -> ``backward()`` (reference src/train.py:291-306) — into a CUDA graph over static input buffers
 and replays it; gradients land in the parameters' ``.grad`` as usual (each replay OVERWRITES them: the step owns the
 buffers, so gradient accumulation over several batches needs ``flat_grads=True`` and a caller-side sum), so the
-optimiser / clipping code of the caller (src/train.py:309-318) stays as it is.  Dropout masks are re-drawn on every replay: the fused dropout is a counter-based hash of (seed, device-side
+optimiser / clipping code of the caller (src/train.py:309-318) stays as it is — or, with ``optimizer=FusedAdam(...)``
+(optim.py), the clipping and the Adam update become the last kernels of the captured step.  Dropout masks are re-drawn on every replay: the fused dropout is a counter-based hash of (seed, device-side
 step counter, element index) and the counter is advanced by a kernel of the captured step itself (csrc/transform.cu,
 csrc/decoder.cu; statistical quality: tests/test_gpu_parity.py::test_fused_dropout_hash_statistics).
 
@@ -24,7 +25,7 @@ from .ops import bce_with_logits
 class GraphedTrainStep:
     def __init__(self, model: torch.nn.Module, edge_index: torch.Tensor, edge_type: torch.Tensor, batch_size: int,
                  loss_fn: Optional[Callable] = None, warmup: int = 3, flat_grads: bool = False, sampler=None,
-                 host_io: bool = False, allreduce: Optional[str] = None):
+                 host_io: bool = False, allreduce: Optional[str] = None, optimizer=None):
         """``host_io``: the captured graph starts with the host-to-device copy of the batch from a pinned staging block
         (``self.host_batch``, int64 [4, B] in ``pack_batch`` layout) and ends with the device-to-host copy of the loss
         and the correct-count into pinned memory (``self.host_loss``, ``self.host_correct``): one graph launch per step
@@ -40,6 +41,13 @@ class GraphedTrainStep:
         data-parallel replicas — the backward kernels write the parameter gradients into a peer-visible flat buffer and the
         LAST kernels of the captured step average it over the ranks (``peer.PeerAllReduce``: our two-shot all-reduce over
         NVLink, no collective call); ``p.grad`` then are views of the averaged buffer.  Every rank must replay in step."""
+        """``optimizer`` (an ``optim.FusedAdam`` / ``FusedAdamW`` over parameters of ``model``): its clipping and update
+        kernels are captured as the last compute of the step (after the peer all-reduce, before the ``host_io`` copies),
+        so one replay is the whole training iteration.  The warm-up steps run without it (construction moves neither
+        the parameters nor the optimiser state).  Every replay first copies changed group hyperparameters (an LR
+        scheduler's ``lr``) to the device and afterwards bumps the parameters' in-place versions; ``step.grad_norm`` is
+        the optimiser's device-side total gradient norm.  The optimiser's state tensors must keep their addresses
+        (``FusedAdam.load_state_dict`` loads into them)."""
         if not edge_index.is_cuda:
             raise RuntimeError("GraphedTrainStep needs CUDA tensors")
         dev = edge_index.device
@@ -69,6 +77,17 @@ class GraphedTrainStep:
             self.pos_tails = torch.zeros(n_pos, dtype=torch.int64, device=dev)
             self.pos_rels = torch.zeros(n_pos, dtype=torch.int64, device=dev)
         self.params = [p for p in model.parameters() if p.requires_grad]
+        self.optimizer = optimizer
+        self._capturing = False
+        if optimizer is not None:
+            from .optim import FusedAdam
+            if not isinstance(optimizer, FusedAdam):
+                raise TypeError("optimizer must be a FusedAdam / FusedAdamW (its kernels are what the graph captures)")
+            mine = {id(p) for p in self.params}
+            if any(id(p) not in mine for g in optimizer.param_groups for p in g["params"]):
+                raise ValueError("the optimizer holds a parameter that is not a trainable parameter of the model")
+            optimizer.prepare_capture()        # state, workspace, hyperparameters: nothing is allocated under capture
+            self._opt_params = [p for g in optimizer.param_groups for p in g["params"]]
         self.flat_grad = None
         self.arena = None
         self.peer_ar = None
@@ -114,8 +133,12 @@ class GraphedTrainStep:
         # capture on the stream the warm-up ran on: the per-stream workspaces (ops._workspace, the fused loss's ticket
         # buffer) exist already, so no allocation — and no zero-fill node — ends up inside the graph
         self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph, stream=side):
-            self.loss, self.scores = self._step()
+        self._capturing = True
+        try:
+            with torch.cuda.graph(self.graph, stream=side):
+                self.loss, self.scores = self._step()
+        finally:
+            self._capturing = False
         if self.arena is not None:
             lo, hi = self.arena.buf.data_ptr(), self.arena.buf.data_ptr() + self.arena.buf.numel() * 4
             inside = all(g is not None and lo <= g.data_ptr() < hi for g in self._grads)
@@ -123,11 +146,7 @@ class GraphedTrainStep:
                 self.flat_grad = self.arena.used        # every parameter gradient lives inside: all-reduce this one tensor
             # else (e.g. basis layers, whose gradients autograd assembles): p.grad are ordinary tensors, flat_grad stays None
             if self.peer_ar is not None:
-                if not inside:
-                    raise RuntimeError("allreduce='peer': a parameter gradient was not written into the arena")
-                # the averaged gradients: same offsets, in the exchange's output buffer
-                self._avg = [self.peer_ar.out[(g.data_ptr() - lo) // 4: (g.data_ptr() - lo) // 4 + g.numel()].view_as(g)
-                             for g in self._grads]
+                self._avg = self._step_grads()
                 self.flat_grad = self.peer_ar.out[: self.arena.off]
         self._bind_grads()
 
@@ -148,6 +167,9 @@ class GraphedTrainStep:
         out = self._step_compute()
         if self.peer_ar is not None:
             self.peer_ar(self.arena.off)               # gradient exchange = the last kernels of the (captured) step
+        if self.optimizer is not None and self._capturing:
+            # every rank applies the same deterministic update to the same averaged gradients
+            self.optimizer._launch(list(zip(self.params, self._step_grads())))
         if self.host_io:
             self.host_loss.copy_(out[0].reshape(1), non_blocking=True)
             if self.correct is not None:
@@ -172,6 +194,31 @@ class GraphedTrainStep:
                 self._one = torch.ones((), dtype=loss.dtype, device=loss.device)     # the seed gradient: no fill kernel per step
             self._grads = torch.autograd.grad(loss, self.params, grad_outputs=self._one, allow_unused=True)
         return loss.detach(), scores.detach()
+
+    def _step_grads(self):
+        """The gradients the step leaves, one per parameter (None: unused), before ``_bind_grads`` publishes them."""
+        if self.peer_ar is not None:
+            # the averaged gradients: same offsets as in the arena, in the exchange's output buffer
+            lo = self.arena.buf.data_ptr()
+            if any(g is None or not lo <= g.data_ptr() < lo + self.arena.buf.numel() * 4 for g in self._grads):
+                raise RuntimeError("allreduce='peer': a parameter gradient was not written into the arena")
+            return [self.peer_ar.out[(g.data_ptr() - lo) // 4: (g.data_ptr() - lo) // 4 + g.numel()].view_as(g)
+                    for g in self._grads]
+        if self.flat_grad is not None and self.arena is None:
+            return [p.grad for p in self.params]
+        return list(self._grads)
+
+    @property
+    def grad_norm(self) -> Optional[torch.Tensor]:
+        """Total gradient norm of the last replay (device scalar; NaN when the optimizer does not clip)."""
+        return None if self.optimizer is None else self.optimizer.grad_norm
+
+    def _replay(self) -> None:
+        if self.optimizer is not None:
+            self.optimizer.sync_hparams()
+        self.graph.replay()
+        if self.optimizer is not None:
+            torch.autograd.graph.increment_version(self._opt_params)
 
     def _bind_grads(self) -> None:
         if self.peer_ar is not None and getattr(self, "_avg", None) is not None:
@@ -211,7 +258,7 @@ class GraphedTrainStep:
         if self.sampler is not None:
             raise RuntimeError("this step draws its own negatives: call run_positives(pos_heads, pos_tails, pos_rels)")
         self.load_packed(packed)
-        self.graph.replay()
+        self._replay()
         self._bind_grads()
         return self.loss
 
@@ -220,7 +267,7 @@ class GraphedTrainStep:
         Returns the pinned loss tensor (valid after a synchronisation)."""
         if not self.host_io:
             raise RuntimeError("replay_host needs a GraphedTrainStep built with host_io=True")
-        self.graph.replay()
+        self._replay()
         self._bind_grads()
         return self.host_loss
 
@@ -231,7 +278,7 @@ class GraphedTrainStep:
         self.pos_heads.copy_(pos_heads, non_blocking=non_blocking)
         self.pos_tails.copy_(pos_tails, non_blocking=non_blocking)
         self.pos_rels.copy_(pos_rels, non_blocking=non_blocking)
-        self.graph.replay()
+        self._replay()
         self._bind_grads()
         return self.loss
 
@@ -241,6 +288,6 @@ class GraphedTrainStep:
             if self.sampler is not None:
                 raise RuntimeError("this step draws its own negatives: call run_positives(pos_heads, pos_tails, pos_rels)")
             self.load_batch(heads, tails, rels, labels)
-        self.graph.replay()
+        self._replay()
         self._bind_grads()          # (a caller may have set .grad to None, e.g. optimizer.zero_grad())
         return self.loss
