@@ -83,6 +83,10 @@ __global__ void __launch_bounds__(256) distmult_bwd_kernel(const float* __restri
   }
 }
 
+// The accuracy decision of reference src/train.py:321-322, sigmoid(x) > 0.5 in fp32, given e = expf(-|x|): not the same
+// as x > 0, since 1 / (1 + expf(-x)) rounds to 0.5 for 0 < x < ~9e-8.  False for x <= 0 and for NaN.
+__device__ __forceinline__ bool sigmoid_above_half(float x, float e) { return x > 0.f && 1.f / (1.f + e) > 0.5f; }
+
 // loss = mean_i [ max(x,0) - x*y + log1p(exp(-|x|)) ]   (= torch BCEWithLogitsLoss, reference src/train.py:139, :300)
 // one block, fixed-order tree => deterministic; also counts sigmoid(x) > 0.5 == y (the accuracy of src/train.py:321-322)
 __global__ void __launch_bounds__(1024) bce_logits_fwd_kernel(const float* __restrict__ x, const float* __restrict__ y,
@@ -95,8 +99,9 @@ __global__ void __launch_bounds__(1024) bce_logits_fwd_kernel(const float* __res
   int cor = 0;
   for (int64_t i = threadIdx.x; i < n; i += 1024) {
     const float v = x[i], t = y[i];
-    acc += fmaxf(v, 0.f) - v * t + log1pf(expf(-fabsf(v)));
-    cor += ((v > 0.f) ? 1.f : 0.f) == t;
+    const float e = expf(-fabsf(v));
+    acc += fmaxf(v, 0.f) - v * t + log1pf(e);
+    cor += (sigmoid_above_half(v, e) ? 1.f : 0.f) == t;
   }
   for (int o = 16; o; o >>= 1) {
     acc += __shfl_xor_sync(0xffffffffu, acc, o);
@@ -235,8 +240,9 @@ __global__ void __launch_bounds__(256) link_loss_fwd_kernel(const LinkLossParams
     }
     if (q.labels) {                                  // NULL: scores only (LinkPredictor.score_pairs)
       const float y = q.labels[p];
-      l = fmaxf(s, 0.f) - s * y + log1pf(expf(-fabsf(s)));
-      ok = (((s > 0.f) ? 1.f : 0.f) == y) ? 1 : 0;
+      const float e = expf(-fabsf(s));
+      l = fmaxf(s, 0.f) - s * y + log1pf(e);
+      ok = ((sigmoid_above_half(s, e) ? 1.f : 0.f) == y) ? 1 : 0;
     }
     if (lane == 0) q.score[p] = s;
   }
@@ -778,13 +784,21 @@ extern "C" int rgcn_link_loss_bwd_rows(const float* emb, int64_t ld, const int64
   size_t smem = (size_t)((2 * n_pairs + 127) / 128 * 128) * sizeof(int);
   b.rows_in_smem = smem <= 200 * 1024 ? 1 : 0;       // (larger batches scan the list in global memory)
   if (!b.rows_in_smem) smem = 0;
-  if (smem > 48 * 1024) {
+  if (smem > 0) {
+    // the default limit is 48 KB of static + dynamic shared memory, and the kernel's own static arrays count against
+    // it: ask the runtime what is left rather than comparing with 48 KB.  Cached per device, so that a captured step
+    // (whose eager warm-up ran the same batch size first) makes no attribute call.
     static size_t granted[64] = {0};
     int dev = 0;
     RGCN_CUDA(cudaGetDevice(&dev));
     if (dev >= 0 && dev < 64 && granted[dev] < smem) {
-      RGCN_CUDA(cudaFuncSetAttribute(link_gather_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      granted[dev] = 200 * 1024;
+      cudaFuncAttributes fa{};
+      RGCN_CUDA(cudaFuncGetAttributes(&fa, link_gather_kernel));
+      granted[dev] = (size_t)fa.maxDynamicSharedSizeBytes;
+      if (granted[dev] < smem) {
+        RGCN_CUDA(cudaFuncSetAttribute(link_gather_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        granted[dev] = 200 * 1024;
+      }
     }
   }
   RGCN_CUDA(launch_pdl(link_gather_kernel, dim3((unsigned)(b.n_owner_blocks + b.n_zero_blocks + b.n_tab_blocks)), dim3(256),

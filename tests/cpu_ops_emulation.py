@@ -124,7 +124,7 @@ def pair_scores(emb, rel_table, head, tail, rel, p_drop=0.0, seed=0, counter=Non
 def link_loss(emb, rel_table, head, tail, rel, labels, p_drop=0.0, seed=0, counter=None):
     s = pair_scores(emb, rel_table, head, tail, rel, p_drop)
     loss = torch.nn.functional.binary_cross_entropy_with_logits(s, labels)
-    return loss, s.detach(), ((s.detach() > 0).float() == labels).sum().to(torch.int32)
+    return loss, s.detach(), ((torch.sigmoid(s.detach()) > 0.5).float() == labels).sum().to(torch.int32)
 
 
 def rank_prep(emb, idx, rel_table, rel, normalize):

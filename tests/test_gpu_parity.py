@@ -728,19 +728,43 @@ def test_cfg3_full_size_basis_forward_backward(pkg):
         assert rel < 1e-4, (name, rel)
 
 
+def _bce_logits(kind):
+    if kind == "random":
+        torch.manual_seed(8)
+        return torch.randn(2048, device=DEV) * 6, (torch.rand(2048, device=DEV) < 0.5).float()
+    if kind == "band":
+        # sigmoid(x) rounds to 0.5 in fp32 for 0 < x < ~9e-8, where x > 0 and sigmoid(x) > 0.5 disagree; labels 1, 0, 0,
+        # 1, 0, 0, ... so that the two labels do not cancel in the count; then +-0, +- the smallest subnormal and +-1e4
+        sweep = torch.linspace(-2e-7, 2e-7, 40_001, device=DEV)
+        special = torch.tensor([0.0, -0.0, 2.0 ** -149, -(2.0 ** -149), 1e4, -1e4], device=DEV).repeat(2)
+        return (torch.cat([sweep, special]),
+                torch.cat([(torch.arange(sweep.numel(), device=DEV) % 3 == 0).float(),
+                           torch.tensor([1.0] * 6 + [0.0] * 6, device=DEV)]))
+    g = torch.Generator(device=DEV).manual_seed(9)                  # long: the single block's per-thread loop
+    return (torch.randn(1_000_000, device=DEV, generator=g) * 4,
+            (torch.rand(1_000_000, device=DEV, generator=g) < 0.5).float())
+
+
 def test_fused_bce_matches_torch(pkg):
+    """Loss, gradient and accuracy count against torch, for each set of logits of ``_bce_logits``."""
     from primekg_rgcn_linkprediction_b200 import ops
-    torch.manual_seed(8)
-    x = (torch.randn(2048, device=DEV) * 6).requires_grad_()
-    y = (torch.rand(2048, device=DEV) < 0.5).float()
-    xr = x.detach().clone().requires_grad_()
-    loss, correct = ops.bce_with_logits(x, y, with_accuracy=True)
-    (loss * 3.0).backward()
-    ref = F.binary_cross_entropy_with_logits(xr, y)
-    (ref * 3.0).backward()
-    torch.testing.assert_close(loss, ref, rtol=1e-6, atol=1e-7)
-    torch.testing.assert_close(x.grad, xr.grad, rtol=1e-5, atol=1e-9)
-    assert int(correct) == int(((torch.sigmoid(xr) > 0.5).float() == y).sum())      # reference src/train.py:321-322
+    for kind in ("random", "band", "long"):
+        x, y = _bce_logits(kind)
+        x.requires_grad_()
+        n = x.numel()
+        xr = x.detach().clone().requires_grad_()
+        loss, correct = ops.bce_with_logits(x, y, with_accuracy=True)
+        (loss * 3.0).backward()
+        ref = F.binary_cross_entropy_with_logits(xr, y)
+        (ref * 3.0).backward()
+        torch.testing.assert_close(loss, ref, rtol=1e-6, atol=1e-7, msg=lambda m: f"{kind} logits: {m}")
+        torch.testing.assert_close(x.grad, xr.grad, rtol=1e-5, atol=1e-9, msg=lambda m: f"{kind} logits: {m}")
+        want = int(((torch.sigmoid(xr) > 0.5).float() == y).sum())                 # reference src/train.py:321-322
+        assert int(correct) == want, f"{kind} logits: accuracy count {int(correct)} != {want}"
+        # against float64: each thread adds n / 1024 terms in order, then two 32-wide butterflies
+        x64 = x.detach().double()
+        l64 = x64.clamp_min(0) - x64 * y.double() + torch.log1p(torch.exp(-x64.abs()))
+        assert abs(float(loss) - float(l64.mean())) <= (n / 1024 + 40) * 2.0 ** -24 * float(l64.abs().mean()), kind
 
 
 # ------------------------------------------------------------------------------------------------
