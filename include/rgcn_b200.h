@@ -528,8 +528,10 @@ int rgcn_rank_count(const float* scores, int64_t ld, int64_t nq, int64_t n_cand,
  *   rgcn_scores_topk_w : per query the k <= 16 best candidates, value alpha * s + beta (alpha > 0) and position in the
  *                        candidate list, sorted by value (ties: lower position first): the cosine sweeps + top-k /
  *                        threshold filters of src/compare_methods.py:384-397, src/medical_validation.py:222-239,
- *                        src/case_studies.py:260-274.  Scratch: cand_val / cand_idx [n_q, n_slots, 16] with n_slots =
- *                        rgcn_scores_topk_slots(n_q, n_cand), slot_ctr [n_q] (cleared by the call). */
+ *                        src/case_studies.py:260-274.  Scratch: cand_val / cand_idx [n_q, n_slots, 16] with n_slots >=
+ *                        rgcn_scores_topk_slots(n_q, n_cand), slot_ctr [n_q] (cleared by the call).  The slot count is
+ *                        the number of partial lists a row can receive (two per CTA run over its row tile, at most
+ *                        2 (#SMs + 1)); fewer slots are rejected. */
 int rgcn_scores_diag_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* tail_planes, int64_t n_q,
                        float* thr, rgcn_stream_t stream);
 int rgcn_scores_rank_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes, int64_t n_cand,

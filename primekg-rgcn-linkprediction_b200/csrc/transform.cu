@@ -939,14 +939,14 @@ extern "C" int rgcn_reduce_partials(const float* part, int64_t n_part, int32_t n
 extern "C" int rgcn_split_planes(const float* x, int64_t ldx, const float* relu_mask, int64_t ldm, int64_t rows,
                                  int32_t cols, void* hi, void* lo, int64_t ldp, float* colsum_partial,
                                  float mask_scale, float* out_f32, int64_t ld_f32, rgcn_stream_t stream) {
-  RGCN_CHECK_ARG(!out_f32 || (((uintptr_t)out_f32 & 15) == 0 && ld_f32 % 4 == 0), "split_planes: fp32 output misaligned");
   RGCN_CHECK_ARG(rows >= 0 && cols >= 4 && cols % 4 == 0 && cols <= 1024, "split_planes: cols=%d must be a multiple of 4 in [4, 1024]", cols);
+  if (rows == 0) return RGCN_OK;                 // nothing is read or written (an empty tensor may have a null pointer)
+  RGCN_CHECK_ARG(!out_f32 || (((uintptr_t)out_f32 & 15) == 0 && ld_f32 % 4 == 0), "split_planes: fp32 output misaligned");
   RGCN_CHECK_ARG(x && ((uintptr_t)x & 15) == 0 && ldx % 4 == 0, "split_planes: x must be 16-byte aligned, ld %% 4 == 0");
   RGCN_CHECK_ARG(!relu_mask || (((uintptr_t)relu_mask & 15) == 0 && ldm % 4 == 0), "split_planes: mask misaligned");
   RGCN_CHECK_ARG(hi && ((uintptr_t)hi & 7) == 0 && (!lo || ((uintptr_t)lo & 7) == 0) && ldp % 4 == 0,
                  "split_planes: planes must be 8-byte aligned, ld %% 4 == 0");
   RGCN_CHECK_ARG(!colsum_partial || ((uintptr_t)colsum_partial & 15) == 0, "split_planes: colsum_partial misaligned");
-  if (rows == 0) return RGCN_OK;
   const int64_t nb = rgcn_split_planes_blocks(rows, cols);
   const int rpp = 256 / (cols / 4) > 0 ? 256 / (cols / 4) : 1;
   const int64_t rows_per_block = ((rows + nb - 1) / nb + rpp - 1) / rpp * rpp;
@@ -1071,11 +1071,14 @@ extern "C" int rgcn_transform_wgrad(const void* A_hi, const void* A_lo, int64_t 
   RGCN_CHECK_ARG(K1 % 4 == 0 && K2 % 4 == 0 && d_out % 4 == 0, "transform_wgrad: K1, K2, d_out must be multiples of 4");
   RGCN_CHECK_ARG(mode == 0 || mode == 1, "transform_wgrad: mode must be 0 (fp32) or 1 (bf16)");
   RGCN_CHECK_ARG(n_rows < (1ll << 31), "transform_wgrad: too many rows for one call");
-  int rc = check_plane(A_hi, lda, "A_hi"); if (rc) return rc;
-  rc = check_plane(G_hi, ldg, "G_hi"); if (rc) return rc;
-  if (mode == 0) {
-    rc = check_plane(A_lo, lda, "A_lo"); if (rc) return rc;
-    rc = check_plane(G_lo, ldg, "G_lo"); if (rc) return rc;
+  int rc;
+  if (n_rows > 0) {                           // no rows: the planes are not read (the outputs are zero)
+    rc = check_plane(A_hi, lda, "A_hi"); if (rc) return rc;
+    rc = check_plane(G_hi, ldg, "G_hi"); if (rc) return rc;
+    if (mode == 0) {
+      rc = check_plane(A_lo, lda, "A_lo"); if (rc) return rc;
+      rc = check_plane(G_lo, ldg, "G_lo"); if (rc) return rc;
+    }
   }
   RGCN_CHECK_ARG(gW1 && (K2 == 0 || gW2), "transform_wgrad: null outputs");
   RGCN_CHECK_ARG(!gbias || (colsum_partial && n_colsum >= 0), "transform_wgrad: g_bias needs the column-sum partials");
@@ -1257,8 +1260,9 @@ extern "C" int rgcn_transform_dgrad_w(const void* G_hi, const void* G_lo, int64_
 //                        (i, true_pos[i]) and exact ties with other candidates are counted as ties
 //   rgcn_scores_rank_w : greater[i] / equal[i] += #{j != true_pos[i] : s_ij > / == thr[i]}   (zero them first)
 //   rgcn_scores_topk_w : per query the k <= 16 best candidates (alpha * s + beta, index), sorted by value then index;
-//                        every epilogue lane keeps a 16-entry list per row across its run of column tiles, the partial
-//                        lists (n_slots per row, rgcn_scores_topk_slots) are merged by a second small kernel
+//                        every epilogue lane keeps a 16-entry list per row across its run of column tiles and stores it
+//                        in one of the row's n_slots partial lists (rgcn_scores_topk_slots: one per CTA run and column
+//                        half that touches the row, uncapped); a second small kernel merges them 256 candidates at a time
 // Replaces score_all_tails + the per-row argsort of src/evaluate.py:260-276 and the cosine sweeps + top-k / threshold
 // filters of src/compare_methods.py:384-397, src/medical_validation.py:222-239, src/case_studies.py:260-274.
 // ------------------------------------------------------------------------------------------------
@@ -1276,38 +1280,51 @@ __global__ void __launch_bounds__(256) topk_merge_kernel(const float* __restrict
   const int total = used * kTopK;
   const float* cv = cand_val + (size_t)row * n_slots * kTopK;
   const int32_t* ci = cand_idx + (size_t)row * n_slots * kTopK;
-  constexpr int PER = 8;                              // up to 256 candidates per row (16 slots)
-  float v[PER];
-  int id[PER];
+  constexpr int PER = 8;                              // candidates per lane and pass: the partial lists in chunks of 256
+  // running top-k of the chunks merged so far: lane j < k holds entry j (value descending, then index ascending)
+  float lv = -INFINITY;
+  int li = -1;
+  for (int base = 0; base < total; base += PER * 32) {
+    float v[PER];
+    int id[PER];
 #pragma unroll
-  for (int u = 0; u < PER; ++u) {
-    const int e = u * 32 + lane;
-    const bool ok = e < total;
-    v[u] = ok ? cv[e] : -INFINITY;
-    id[u] = ok ? ci[e] : -1;
-    if (id[u] < 0) v[u] = -INFINITY;
+    for (int u = 0; u < PER; ++u) {
+      const int e = base + u * 32 + lane;
+      const bool ok = e < total;
+      v[u] = ok ? cv[e] : -INFINITY;
+      id[u] = ok ? ci[e] : -1;
+      if (id[u] < 0) v[u] = -INFINITY;
+    }
+    float nv = -INFINITY;
+    int ni = -1;
+    for (int j = 0; j < k; ++j) {
+      // warp arg-max over the chunk and the running list by (value desc, index asc)
+      float bv = -INFINITY;
+      int bi = 0x7fffffff;
+      if (li >= 0 && (lv > bv || (lv == bv && li < bi))) { bv = lv; bi = li; }
+#pragma unroll
+      for (int u = 0; u < PER; ++u)
+        if (id[u] >= 0 && (v[u] > bv || (v[u] == bv && id[u] < bi))) { bv = v[u]; bi = id[u]; }
+#pragma unroll
+      for (int o = 16; o; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+      }
+      if (bi == 0x7fffffff) break;                    // (warp-uniform) nothing left
+      // an index occurs once: the partial lists cover disjoint column ranges
+      if (li == bi) { li = -1; lv = -INFINITY; }
+#pragma unroll
+      for (int u = 0; u < PER; ++u)
+        if (id[u] == bi) { id[u] = -1; v[u] = -INFINITY; }
+      if (lane == j) { nv = bv; ni = bi; }
+    }
+    lv = nv;
+    li = ni;
   }
-  for (int j = 0; j < k; ++j) {
-    // warp arg-max by (value desc, index asc)
-    float bv = -INFINITY;
-    int bi = 0x7fffffff;
-#pragma unroll
-    for (int u = 0; u < PER; ++u)
-      if (id[u] >= 0 && (v[u] > bv || (v[u] == bv && id[u] < bi))) { bv = v[u]; bi = id[u]; }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-      const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-      const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
-    }
-#pragma unroll
-    for (int u = 0; u < PER; ++u)
-      if (id[u] == bi) { id[u] = -1; v[u] = -INFINITY; }      // (an index occurs once: column ranges are disjoint)
-    if (lane == 0) {
-      const bool have = bi != 0x7fffffff;
-      out_val[row * k + j] = have ? alpha * bv + beta : -INFINITY;
-      out_idx[row * k + j] = have ? (int64_t)bi : -1;
-    }
+  if (lane < k) {
+    out_val[row * k + lane] = li >= 0 ? alpha * lv + beta : -INFINITY;
+    out_idx[row * k + lane] = li >= 0 ? (int64_t)li : -1;
   }
 }
 }  // namespace rgcn
@@ -1357,8 +1374,8 @@ extern "C" int32_t rgcn_scores_topk_slots(int64_t n_q, int64_t n_cand) {
   const int64_t tiles = n_tiles * m_tiles;
   const int64_t grid = tiles < sm_count() ? tiles : sm_count();
   const int64_t per = (tiles + grid - 1) / grid;
-  int64_t slots = 2 * ((n_tiles + per - 1) / per + 1);           // CTA runs touching one row tile x two column halves
-  return (int32_t)(slots > 16 ? 16 : slots);
+  // CTA runs touching one row tile x two column halves: at most 2 (#SMs + 1), whatever the shape
+  return (int32_t)(2 * ((n_tiles + per - 1) / per + 1));
 }
 
 extern "C" int rgcn_scores_topk_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
@@ -1370,8 +1387,7 @@ extern "C" int rgcn_scores_topk_w(const void* Q_hi, const void* Q_lo, int64_t ld
   if (rc) return rc;
   RGCN_CHECK_ARG(n_cand > 0 && n_cand < (1ll << 31) && k >= 1 && k <= kTopK && alpha > 0.f, "scores_topk_w: 1 <= k <= %d, alpha > 0", kTopK);
   RGCN_CHECK_ARG(cand_val && cand_idx && slot_ctr && out_val && out_idx, "scores_topk_w: null argument");
-  RGCN_CHECK_ARG(n_slots >= rgcn_scores_topk_slots(n_q, n_cand) || n_slots == 16, "scores_topk_w: too few slots (rgcn_scores_topk_slots)");
-  RGCN_CHECK_ARG(rgcn_scores_topk_slots(n_q, n_cand) <= 16 && 2 * ((n_cand + KBN - 1) / KBN) + 2 >= 0, "scores_topk_w: bad sizes");
+  RGCN_CHECK_ARG(n_slots >= rgcn_scores_topk_slots(n_q, n_cand), "scores_topk_w: too few slots (rgcn_scores_topk_slots)");
   if (n_q == 0) return RGCN_OK;
   cudaStream_t st = (cudaStream_t)stream;
   RGCN_CUDA(cudaMemsetAsync(slot_ctr, 0, (size_t)n_q * sizeof(int32_t), st));

@@ -330,7 +330,8 @@ def split_planes(x: torch.Tensor, planes, col0: int = 0, relu_mask: Optional[tor
     part = None
     if colsum:
         nb = lib.rgcn_split_planes_blocks(rows, cols)
-        part = torch.empty(max(nb, 1), cols, dtype=torch.float32, device=x.device)
+        # no rows: the kernel writes no partial, so the one row handed on must be zero (a sum over nothing)
+        part = (torch.empty if nb > 0 else torch.zeros)(max(nb, 1), cols, dtype=torch.float32, device=x.device)
     hi_v = hi[:, col0:col0 + cols]
     lo_v = None if lo is None else lo[:, col0:col0 + cols]
     _lib.check(lib.rgcn_split_planes(_ptr(x), x.stride(0), _ptr(relu_mask), 0 if relu_mask is None else relu_mask.stride(0),
@@ -736,7 +737,7 @@ def p2p_reduce_split(part_ptrs, row0: int, ld_part: int, rows: int, cols: int, d
     part = None
     if colsum:
         nb = lib.rgcn_split_planes_blocks(rows, cols)
-        part = torch.empty(max(nb, 1), cols, dtype=torch.float32, device=device)
+        part = (torch.empty if nb > 0 else torch.zeros)(max(nb, 1), cols, dtype=torch.float32, device=device)
     _lib.check(lib.rgcn_p2p_reduce_split(_ptr_array(part_ptrs), len(part_ptrs), int(row0), int(ld_part), _ptr(extra),
                                          0 if extra is None else extra.stride(0), _ptr(relu_mask),
                                          0 if relu_mask is None else relu_mask.stride(0), float(mask_scale), rows, cols,

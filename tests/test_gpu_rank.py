@@ -102,37 +102,52 @@ def test_all_pairs_drug_disease_sweep(pkg, method):
     torch.testing.assert_close(gotc, wantc, rtol=1e-5, atol=1e-5 if method == "simt" else 2e-5)
 
 
+# (queries, candidates): BASELINE cfg4 (5,593 diseases x 6,282 drugs), then few queries against many candidates, where a
+# row receives a partial list from every CTA run over its row tile (up to 2 (#SMs + 1) lists), and fewer candidates than k
+TOPK_SHAPES = [(5593, 6282), (1, 1025), (100, 5593), (128, 30926), (1000, 30926), (2048, 30926), (7, 5)]
+
+
+@pytest.mark.parametrize("nq,ncand", TOPK_SHAPES)
 @pytest.mark.parametrize("cosine", [False, True])
 @pytest.mark.parametrize("k", [1, 10, 16])
-def test_fused_topk_matches_sorted_score_matrix(pkg, cosine, k):
+def test_fused_topk_matches_sorted_score_matrix(pkg, cosine, k, nq, ncand):
     """``topk_all_pairs`` (score block consumed in the GEMM epilogue) against a sort of the materialised tensor-core score
-    matrix: same values bit for bit, same candidates, ties broken by the lower position; BASELINE cfg4 shape."""
+    matrix: same values bit for bit, same candidates, ties broken by the lower position; missing entries (fewer
+    candidates than k) are -inf / -1."""
     torch.manual_seed(4)
     emb = torch.randn(30926, 128, device=DEV)
-    emb[7000] = emb[6000]                                # duplicate candidates => exact ties
-    drugs = torch.arange(5593, 11875, device=DEV)
-    diseases = torch.arange(0, 5593, device=DEV)
+    c0 = 5593 if ncand == 6282 else 0
+    queries = torch.arange(nq, device=DEV) + (0 if c0 else 30926 - nq)
+    cands = torch.arange(c0, c0 + ncand, device=DEV)
+    if ncand >= 3:
+        emb[cands[2 * ncand // 3]] = emb[cands[ncand // 3]]          # duplicate candidates => exact ties
     rel = torch.randn(128, device=DEV)
     kw = dict(cosine=True) if cosine else dict(rel_vec=rel)
-    val, ids = pkg.topk_all_pairs(emb, diseases, drugs, k=k, **kw)
-    S = pkg.score_all_pairs(emb, diseases, drugs, **kw)
-    assert val.shape == (5593, k) and ids.shape == (5593, k)
-    # reference order: value descending, position ascending
-    order = torch.argsort(S, dim=1, descending=True, stable=True)[:, :k]
-    want_val = S.gather(1, order)
-    if k > 1:
-        assert torch.all(val[:, :-1] >= val[:, 1:])
+    val, ids = pkg.topk_all_pairs(emb, queries, cands, k=k, **kw)
+    S = pkg.score_all_pairs(emb, queries, cands, **kw)
+    assert val.shape == (nq, k) and ids.shape == (nq, k)
+    # reference order: value descending, position ascending; entries beyond the candidate count are -inf / -1
+    kk = min(k, ncand)
+    order = torch.argsort(S, dim=1, descending=True, stable=True)[:, :kk]
+    want_val = torch.full((nq, k), float("-inf"), device=DEV)
+    want_ids = torch.full((nq, k), -1, dtype=torch.int64, device=DEV)
+    want_val[:, :kk] = S.gather(1, order)
+    want_ids[:, :kk] = cands[order]
+    assert torch.equal(ids[:, kk:], want_ids[:, kk:]) and torch.equal(val[:, kk:], want_val[:, kk:])
+    if kk > 1:
+        assert torch.all(val[:, :kk - 1] >= val[:, 1:kk])
     if not cosine:
         # DistMult: the sweep and the matrix are the same products in the same order => the same bits, and exact ties
         # (the duplicated candidate) are broken like the stable sort: lower position first
         assert torch.equal(val, want_val)
-        assert torch.equal(ids, drugs[order])
+        assert torch.equal(ids, want_ids)
     else:
         # cosine: the matrix folds (s + 1) / 2 into the contraction, the fused form applies it to the accumulator
-        torch.testing.assert_close(val, want_val, rtol=0, atol=2e-6)
-        pos = ids - 5593
-        torch.testing.assert_close(S.gather(1, pos), val, rtol=0, atol=2e-6)      # the returned candidates carry these scores
-        assert bool(((pos[:, :-1] != pos[:, 1:]).all())) if k > 1 else True
+        torch.testing.assert_close(val[:, :kk], want_val[:, :kk], rtol=0, atol=2e-6)
+        pos = ids[:, :kk] - c0
+        assert bool(((pos >= 0) & (pos < ncand)).all())
+        torch.testing.assert_close(S.gather(1, pos), val[:, :kk], rtol=0, atol=2e-6)   # the candidates carry these scores
+        assert bool((pos.sort(1).values[:, 1:] != pos.sort(1).values[:, :-1]).all()) if kk > 1 else True
 
 
 def test_fused_rank_matches_block_rank_at_evaluate_size(pkg):
