@@ -516,6 +516,19 @@ int rgcn_allpairs_rank(const float* A, int64_t lda, int64_t nq, const float* B, 
  * excluded by index.  thr (optional) receives the thresholds. */
 int rgcn_rank_count(const float* scores, int64_t ld, int64_t nq, int64_t n_cand, const int64_t* true_pos,
                     float* thr, int32_t* greater, int32_t* equal, rgcn_stream_t stream);
+/* Exclusion lists (filtered ranking, top-k of novel links): row i of the queries excludes the candidate positions
+ * excl_pos[excl_begin[i] .. excl_end[i]) (int32, sorted ascending and distinct within each range; positions >= n_cand are
+ * ignored; ranges of different rows may overlap or share storage).  The excluding entry points take the three pointers
+ * together: all null (no filter) or none.
+ *   rgcn_rank_excl_correct : turns the counts of rgcn_rank_count / rgcn_allpairs_rank into filtered counts: for every
+ *                            excluded j != true_pos[i] it subtracts [s_ij > thr[i]] from greater[i] and [s_ij == thr[i]]
+ *                            from equal[i].  s_ij is read from the score block `scores` (ld) when it is given, else
+ *                            recomputed as rgcn_allpairs_rank computes it (A, B, b_idx, d: fmaf in ascending k).  thr is the
+ *                            counting pass's threshold (its thr output). */
+int rgcn_rank_excl_correct(const float* scores, int64_t ld, const float* A, int64_t lda, const float* B, int64_t ldb,
+                           const int64_t* b_idx, int32_t d, int64_t nq, int64_t n_cand, const int64_t* true_pos,
+                           const float* thr, const int64_t* excl_begin, const int64_t* excl_end, const int32_t* excl_pos,
+                           int32_t* greater, int32_t* equal, rgcn_stream_t stream);
 /* The same sweeps on the tensor cores WITHOUT the [queries, candidates] matrix: the tcgen05 kernel's epilogue consumes the
  * accumulator (three bf16 products, fp32 accumulation, as the fp32 mode of the transforms).
  *   Q_hi / Q_lo     : the prepared query rows (rgcn_rows_prepare) as bf16 planes [n_q, d] (rgcn_split_planes)
@@ -531,7 +544,11 @@ int rgcn_rank_count(const float* scores, int64_t ld, int64_t nq, int64_t n_cand,
  *                        src/case_studies.py:260-274.  Scratch: cand_val / cand_idx [n_q, n_slots, 16] with n_slots >=
  *                        rgcn_scores_topk_slots(n_q, n_cand), slot_ctr [n_q] (cleared by the call).  The slot count is
  *                        the number of partial lists a row can receive (two per CTA run over its row tile, at most
- *                        2 (#SMs + 1)); fewer slots are rejected. */
+ *                        2 (#SMs + 1)); fewer slots are rejected.
+ *   rgcn_scores_rank_excl_w / rgcn_scores_topk_excl_w : the same with exclusion lists (format above rgcn_rank_excl_correct;
+ *                        all three null = the unfiltered call).  rank: an excluded column counts in neither greater nor
+ *                        equal (the true tail stays excluded by index; listing it changes nothing).  top-k: an excluded
+ *                        column is never a candidate; a row with fewer than k admissible columns ends in -inf / -1. */
 int rgcn_scores_diag_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* tail_planes, int64_t n_q,
                        float* thr, rgcn_stream_t stream);
 int rgcn_scores_rank_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes, int64_t n_cand,
@@ -541,6 +558,15 @@ int32_t rgcn_scores_topk_slots(int64_t n_q, int64_t n_cand);
 int rgcn_scores_topk_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes, int64_t n_cand,
                        int64_t n_q, int32_t k, float alpha, float beta, float* cand_val, int32_t* cand_idx,
                        int32_t* slot_ctr, int32_t n_slots, float* out_val, int64_t* out_idx, rgcn_stream_t stream);
+int rgcn_scores_rank_excl_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
+                            int64_t n_cand, int64_t n_q, const float* thr, const int64_t* true_pos, int32_t* greater,
+                            int32_t* equal, const int64_t* excl_begin, const int64_t* excl_end, const int32_t* excl_pos,
+                            rgcn_stream_t stream);
+int rgcn_scores_topk_excl_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
+                            int64_t n_cand, int64_t n_q, int32_t k, float alpha, float beta, float* cand_val,
+                            int32_t* cand_idx, int32_t* slot_ctr, int32_t n_slots, float* out_val, int64_t* out_idx,
+                            const int64_t* excl_begin, const int64_t* excl_end, const int32_t* excl_pos,
+                            rgcn_stream_t stream);
 /* ------------------------------------------------------------------------------------------
  * Fused link-prediction loss.  Replaces nn.BCEWithLogitsLoss (mean) over the batch logits and the
  * sigmoid > 0.5 accuracy count (src/train.py:139, :300, :321-322):

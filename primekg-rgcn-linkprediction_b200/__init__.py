@@ -8,12 +8,12 @@ A from-scratch implementation of the one hot path of arnold117/PrimeKG-RGCN-Link
 from .conv import RGCNConv, default_mode
 from .graph import RelGraph, clear_graph_cache, get_graph, graph_from_state, graph_state, register_graph
 from .graphed import GraphedTrainStep
-from .rank import rank_true_tails, ranking_metrics, score_all_pairs, topk_all_pairs
+from .rank import KnownTriples, rank_true_tails, ranking_metrics, score_all_pairs, topk_all_pairs
 from .modules import DrugDiseaseModel, DrugDiseaseRGCN, LinkPredictor
 from .sampler import NegativeSampler
 from .optim import FusedAdam, FusedAdamW
 
 __all__ = ["RGCNConv", "DrugDiseaseRGCN", "LinkPredictor", "DrugDiseaseModel", "RelGraph", "get_graph",
-           "clear_graph_cache", "default_mode", "GraphedTrainStep", "graph_state", "graph_from_state", "register_graph", "rank_true_tails", "ranking_metrics", "score_all_pairs", "topk_all_pairs",
+           "clear_graph_cache", "default_mode", "GraphedTrainStep", "graph_state", "graph_from_state", "register_graph", "KnownTriples", "rank_true_tails", "ranking_metrics", "score_all_pairs", "topk_all_pairs",
            "NegativeSampler", "FusedAdam", "FusedAdamW"]
 __version__ = "0.1.0"

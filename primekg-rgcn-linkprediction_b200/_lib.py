@@ -138,6 +138,10 @@ PROTOTYPES = {
     "rgcn_scores_rank_w": (C.c_int, [p, p, i64, i32, p, i64, i64, p, p, p, p, p]),
     "rgcn_scores_topk_slots": (i32, [i64, i64]),
     "rgcn_scores_topk_w": (C.c_int, [p, p, i64, i32, p, i64, i64, i32, C.c_float, C.c_float, p, p, p, i32, p, p, p]),
+    "rgcn_rank_excl_correct": (C.c_int, [p, i64, p, i64, p, i64, p, i32, i64, i64, p, p, p, p, p, p, p, p]),
+    "rgcn_scores_rank_excl_w": (C.c_int, [p, p, i64, i32, p, i64, i64, p, p, p, p, p, p, p, p]),
+    "rgcn_scores_topk_excl_w": (C.c_int, [p, p, i64, i32, p, i64, i64, i32, C.c_float, C.c_float, p, p, p, i32, p, p,
+                                          p, p, p, p]),
     "rgcn_bce_logits_fwd": (C.c_int, [p, p, i64, p, p, p]),
     "rgcn_bce_logits_bwd": (C.c_int, [p, p, i64, p, p, p]),
     "rgcn_link_batch": (C.c_int, [p, p, p, i64, i32, i64, u32, p, p, p, p, p, p]),

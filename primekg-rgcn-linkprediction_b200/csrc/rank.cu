@@ -246,3 +246,71 @@ extern "C" int rgcn_rank_count(const float* scores, int64_t ld, int64_t nq, int6
   return RGCN_OK;
 }
 
+// ---- filtered ranks from an unfiltered count -------------------------------------------------------------------------
+// After rgcn_rank_count (materialised block) or rgcn_allpairs_rank (fp32 FMA tiles): every excluded position j != t_i of
+// row i whose score is > / == thr[i] is taken back out of greater[i] / equal[i].  The score carries the counting pass's
+// own bits: read from the block, or recomputed with the tile kernel's accumulation (fmaf, k ascending).  One warp per
+// row, integer updates: deterministic.
+namespace rgcn {
+__global__ void __launch_bounds__(256) rank_excl_correct_kernel(const float* __restrict__ s, int64_t lds,
+                                                                const float* __restrict__ A, int64_t lda,
+                                                                const float* __restrict__ B, int64_t ldb,
+                                                                const int64_t* __restrict__ b_idx, int32_t d, int64_t nq,
+                                                                int64_t n_cand, const int64_t* __restrict__ true_pos,
+                                                                const float* __restrict__ thr,
+                                                                const int64_t* __restrict__ excl_begin,
+                                                                const int64_t* __restrict__ excl_end,
+                                                                const int32_t* __restrict__ excl_pos,
+                                                                int32_t* __restrict__ greater, int32_t* __restrict__ equal) {
+  pdl_enter();
+  const int lane = threadIdx.x & 31;
+  const int64_t i = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (i >= nq) return;
+  const int64_t t = true_pos[i];
+  const float th = thr[i];
+  int g = 0, e = 0;
+  for (int64_t x = excl_begin[i] + lane; x < excl_end[i]; x += 32) {
+    const int64_t j = excl_pos[x];
+    if (j == t || j < 0 || j >= n_cand) continue;
+    float v;
+    if (s) {
+      v = s[i * lds + j];
+    } else {
+      const float* a = A + i * lda;
+      const float* b = B + (b_idx ? b_idx[j] : j) * ldb;
+      float acc = 0.f;
+      for (int k = 0; k < d; ++k) acc = fmaf(a[k], b[k], acc);
+      v = acc;
+    }
+    g += v > th;
+    e += v == th;
+  }
+  for (int o = 16; o; o >>= 1) {
+    g += __shfl_xor_sync(0xffffffffu, g, o);
+    e += __shfl_xor_sync(0xffffffffu, e, o);
+  }
+  if (lane == 0) { greater[i] -= g; equal[i] -= e; }
+}
+}  // namespace rgcn
+
+extern "C" int rgcn_rank_excl_correct(const float* scores, int64_t ld, const float* A, int64_t lda, const float* B,
+                                      int64_t ldb, const int64_t* b_idx, int32_t d, int64_t nq, int64_t n_cand,
+                                      const int64_t* true_pos, const float* thr, const int64_t* excl_begin,
+                                      const int64_t* excl_end, const int32_t* excl_pos, int32_t* greater, int32_t* equal,
+                                      rgcn_stream_t stream) {
+  RGCN_CHECK_ARG(nq >= 0 && n_cand >= 0, "rank_excl_correct: negative size");
+  if (nq == 0) return RGCN_OK;
+  RGCN_CHECK_ARG(true_pos && thr && excl_begin && excl_end && excl_pos && greater && equal,
+                 "rank_excl_correct: null argument");
+  if (scores) {
+    RGCN_CHECK_ARG(ld >= n_cand, "rank_excl_correct: ld < n_cand");
+  } else {
+    RGCN_CHECK_ARG(A && B && d > 0, "rank_excl_correct: needs the score block or the operands A, B");
+  }
+  RGCN_CUDA(launch_pdl(rgcn::rank_excl_correct_kernel, dim3((unsigned)((nq + 7) / 8)), dim3(256), 0, (cudaStream_t)stream,
+                       scores, ld, A, lda, B, ldb, b_idx, d, nq, n_cand, true_pos, thr, excl_begin, excl_end, excl_pos,
+                       greater, equal));
+  RGCN_LAUNCH_CHECK();
+  return RGCN_OK;
+}
+

@@ -23,6 +23,7 @@
 //   MMA warp : one thread issues tcgen05.mma.cta_group::1.kind::f16 (M=128, N=BN, K=16) and tcgen05.commit
 //   epilogue : tcgen05.ld -> bias / ReLU -> staging tile in the idle operand smem -> coalesced 128-bit row stores
 #include <cuda.h>
+#include <limits.h>
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -170,6 +171,10 @@ struct GemmKParams {
   // matrix are clipped by the copy engine
   int tma_store;
   alignas(64) CUtensorMap tm_out;
+  // EPI_RANK / EPI_TOPK with exclusion (the EXCL instantiations): row i skips the candidate positions
+  // excl_pos[excl_begin[i] .. excl_end[i]), sorted ascending and distinct.  (Last, so that the fields above keep their
+  // offsets: the unfiltered rank / top-k instantiations compile to the same SASS.)
+  const int64_t* excl_begin; const int64_t* excl_end; const int32_t* excl_pos;
 };
 
 enum { EPI_STORE = 0, EPI_RANK = 1, EPI_THR = 2, EPI_TOPK = 3 };
@@ -211,7 +216,10 @@ struct KStage {
 // ceil(BN / 64) chunks of 64 k-rows x 128 B, the layout of the weight-gradient kernel's operands.
 // XF (EPI_STORE only) specialises the store loop, which is where an epilogue-bound launch spends its instructions:
 // 0 = plain store, 1 = + fused dropout, 2 = everything decided at run time (bf16 copy, peer stores, scattered rows)
-template <bool SPLIT, bool B_MN, int EPI = EPI_STORE, int BNT = 128, int XF = 2>
+// EXCL (EPI_RANK / EPI_TOPK only): skip each row's excluded candidate positions (p.excl_*).  A lane visits its row's
+// columns in ascending order (a CTA run walks its column tiles in order, the warp its half of each tile chunk by chunk),
+// so one cursor per lane walks the sorted list: one comparison per element, a load only when the cursor advances.
+template <bool SPLIT, bool B_MN, int EPI = EPI_STORE, int BNT = 128, int XF = 2, bool EXCL = false>
 __global__ void __launch_bounds__((epi_warps(EPI) + 2) * 32, 1)
 gemm_kmajor_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                    const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo,
@@ -299,6 +307,10 @@ gemm_kmajor_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
     uint2* tbuf = reinterpret_cast<uint2*>(patch);
     int bcnt = 0;
     float kth = -INFINITY;                                    // the list's last entry as of the last drain
+    // exclusion cursor (EXCL): x_next = excl_pos[x_cur], or INT_MAX past the end of the row's list
+    int64_t x_cur = 0, x_end = 0;
+    int x_next = INT_MAX;
+    auto x_advance = [&]() { ++x_cur; x_next = x_cur < x_end ? p.excl_pos[x_cur] : INT_MAX; };
     auto drain = [&]() {
       const int mx = __reduce_max_sync(0xffffffffu, bcnt);
       for (int e = 0; e < mx; ++e) {
@@ -360,6 +372,19 @@ gemm_kmajor_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
           kth = -INFINITY;
           bcnt = 0;
         }
+        if (EXCL) {
+          // the run may enter the row tile mid-row: start at the lower bound of the first column this warp visits
+          int64_t lo = 0, hi = 0;
+          if (row < p.M) { lo = p.excl_begin[row]; hi = x_end = p.excl_end[row]; }
+          else x_end = 0;
+          const int first = n0 + c_lo;
+          while (lo < hi) {
+            const int64_t mid = lo + ((hi - lo) >> 1);
+            if (p.excl_pos[mid] < first) lo = mid + 1; else hi = mid;
+          }
+          x_cur = lo;
+          x_next = x_cur < x_end ? p.excl_pos[x_cur] : INT_MAX;
+        }
       }
       mbar_wait(&tfull_bar[a], (uint32_t)((iter >> 1) & 1));
       fence_after_sync();
@@ -370,12 +395,18 @@ gemm_kmajor_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
         tmem_ld_wait();
         if (EPI != EPI_STORE) {
           const int64_t row = m0 + quarter * 32 + lane;
+          if (EXCL) {
+            // entries below this chunk: columns of the other half, or of tiles this run does not visit
+            while (x_next < n0 + cc) x_advance();
+          }
           if (EPI == EPI_RANK) {
 #pragma unroll
             for (int j = 0; j < 16; ++j) {
               const int64_t col = n0 + cc + j;
               const float v = __uint_as_float(r[j]);
-              if (row < p.M && col < p.n_cols_valid && col != tpos) { cnt_g += v > thr; cnt_e += v == thr; }
+              bool skip = false;
+              if (EXCL && x_next == n0 + cc + j) { skip = true; x_advance(); }
+              if (row < p.M && col < p.n_cols_valid && col != tpos && !skip) { cnt_g += v > thr; cnt_e += v == thr; }
             }
           } else if (EPI == EPI_THR) {
             // the diagonal element of this lane's row, if it lies in this warp's 16 columns
@@ -396,7 +427,9 @@ gemm_kmajor_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_con
               for (int j = j0; j < j0 + 4; ++j) {
                 const int col = n0 + cc + j;
                 const float v = __uint_as_float(r[j]);
-                if (row < p.M && col < p.n_cols_valid && v > kth) {
+                bool skip = false;
+                if (EXCL && x_next == col) { skip = true; x_advance(); }
+                if (row < p.M && col < p.n_cols_valid && v > kth && !skip) {
                   tbuf[lane + 32 * bcnt] = make_uint2(r[j], (uint32_t)col);
                   ++bcnt;
                 }
@@ -867,12 +900,13 @@ static int wide_bn() {
   return v;
 }
 
-template <bool SPLIT, bool B_MN, int EPI>
+template <bool SPLIT, bool B_MN, int EPI, bool EXCL = false>
 static int launch_kmajor_e(const GemmKParams& p, const CUtensorMap& ahi, const CUtensorMap& alo, const CUtensorMap& mhi,
                            const CUtensorMap& mlo, unsigned grid, cudaStream_t st) {
-  int rc = set_smem(gemm_kmajor_kernel<SPLIT, B_MN, EPI>, KStage<SPLIT>::SMEM);
+  auto kern = gemm_kmajor_kernel<SPLIT, B_MN, EPI, 128, 2, EXCL>;
+  int rc = set_smem(kern, KStage<SPLIT>::SMEM);
   if (rc) return rc;
-  RGCN_CUDA(launch_pdl(gemm_kmajor_kernel<SPLIT, B_MN, EPI>, dim3(grid), dim3(K_THREADS), KStage<SPLIT>::SMEM, st, ahi, alo, mhi, mlo, p));
+  RGCN_CUDA(launch_pdl(kern, dim3(grid), dim3(K_THREADS), KStage<SPLIT>::SMEM, st, ahi, alo, mhi, mlo, p));
   RGCN_LAUNCH_CHECK();
   return RGCN_OK;
 }
@@ -895,9 +929,12 @@ static int launch_kmajor(GemmKParams p, const void* a_hi, const void* a_lo, int6
   if (epi != EPI_STORE) {
     // the consuming epilogues serve the all-pairs scorers: K-major candidates, three-product (fp32) mode
     if (b_mn || !split) { set_error("transform: the scoring epilogues need K-major candidates in fp32 mode"); return RGCN_EINVAL; }
-    if (epi == EPI_RANK) return launch_kmajor_e<true, false, EPI_RANK>(p, ahi, alo, mhi, mlo, grid, st);
+    const bool excl = p.excl_pos != nullptr;
+    if (epi == EPI_RANK) return excl ? launch_kmajor_e<true, false, EPI_RANK, true>(p, ahi, alo, mhi, mlo, grid, st)
+                                     : launch_kmajor_e<true, false, EPI_RANK>(p, ahi, alo, mhi, mlo, grid, st);
     if (epi == EPI_THR) return launch_kmajor_e<true, false, EPI_THR>(p, ahi, alo, mhi, mlo, grid, st);
-    return launch_kmajor_e<true, false, EPI_TOPK>(p, ahi, alo, mhi, mlo, grid, st);
+    return excl ? launch_kmajor_e<true, false, EPI_TOPK, true>(p, ahi, alo, mhi, mlo, grid, st)
+                : launch_kmajor_e<true, false, EPI_TOPK>(p, ahi, alo, mhi, mlo, grid, st);
   }
   if (split) return b_mn ? launch_kmajor_t<true, true>(p, ahi, alo, mhi, mlo, grid, st)
                          : launch_kmajor_t<true, false>(p, ahi, alo, mhi, mlo, grid, st);
@@ -1352,16 +1389,34 @@ extern "C" int rgcn_scores_diag_w(const void* Q_hi, const void* Q_lo, int64_t ld
   return launch_kmajor(p, Q_hi, Q_lo, ldq, d, bhi, blo, n_q, d, wplane_ld(d), false, 1, true, (cudaStream_t)stream, EPI_THR);
 }
 
+// the exclusion lists come as a triple: all null (no filter) or none
+static int check_excl(const int64_t* excl_begin, const int64_t* excl_end, const int32_t* excl_pos, const char* what) {
+  const int n_null = (excl_begin == nullptr) + (excl_end == nullptr) + (excl_pos == nullptr);
+  RGCN_CHECK_ARG(n_null == 0 || n_null == 3, "%s: excl_begin, excl_end and excl_pos are all null or none is", what);
+  return RGCN_OK;
+}
+
 extern "C" int rgcn_scores_rank_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
                                   int64_t n_cand, int64_t n_q, const float* thr, const int64_t* true_pos, int32_t* greater,
                                   int32_t* equal, rgcn_stream_t stream) {
+  return rgcn_scores_rank_excl_w(Q_hi, Q_lo, ldq, d, cand_planes, n_cand, n_q, thr, true_pos, greater, equal, nullptr,
+                                 nullptr, nullptr, stream);
+}
+
+extern "C" int rgcn_scores_rank_excl_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
+                                       int64_t n_cand, int64_t n_q, const float* thr, const int64_t* true_pos,
+                                       int32_t* greater, int32_t* equal, const int64_t* excl_begin, const int64_t* excl_end,
+                                       const int32_t* excl_pos, rgcn_stream_t stream) {
+  int rc = check_excl(excl_begin, excl_end, excl_pos, "scores_rank_excl_w");
+  if (rc) return rc;
   GemmKParams p{};
-  int rc = scores_common(p, Q_hi, Q_lo, ldq, d, cand_planes, n_q, "scores_rank_w");
+  rc = scores_common(p, Q_hi, Q_lo, ldq, d, cand_planes, n_q, "scores_rank_w");
   if (rc) return rc;
   RGCN_CHECK_ARG(n_cand > 0 && n_cand < (1ll << 31) && thr && true_pos && greater && equal, "scores_rank_w: null argument");
   if (n_q == 0) return RGCN_OK;
   p.N = (int)n_cand; p.n_cols_valid = n_cand; p.tile_contig = 1;
   p.thr_in = thr; p.true_pos = true_pos; p.greater = greater; p.equal = equal;
+  p.excl_begin = excl_begin; p.excl_end = excl_end; p.excl_pos = excl_pos;
   const int n_tiles = (int)((n_cand + KBN - 1) / KBN);
   const __nv_bfloat16* bhi = (const __nv_bfloat16*)cand_planes;
   const __nv_bfloat16* blo = (const __nv_bfloat16*)((const char*)cand_planes + wplane_bytes((int)n_cand, d));
@@ -1382,8 +1437,19 @@ extern "C" int rgcn_scores_topk_w(const void* Q_hi, const void* Q_lo, int64_t ld
                                   int64_t n_cand, int64_t n_q, int32_t k, float alpha, float beta, float* cand_val,
                                   int32_t* cand_idx, int32_t* slot_ctr, int32_t n_slots, float* out_val, int64_t* out_idx,
                                   rgcn_stream_t stream) {
+  return rgcn_scores_topk_excl_w(Q_hi, Q_lo, ldq, d, cand_planes, n_cand, n_q, k, alpha, beta, cand_val, cand_idx, slot_ctr,
+                                 n_slots, out_val, out_idx, nullptr, nullptr, nullptr, stream);
+}
+
+extern "C" int rgcn_scores_topk_excl_w(const void* Q_hi, const void* Q_lo, int64_t ldq, int32_t d, const void* cand_planes,
+                                       int64_t n_cand, int64_t n_q, int32_t k, float alpha, float beta, float* cand_val,
+                                       int32_t* cand_idx, int32_t* slot_ctr, int32_t n_slots, float* out_val,
+                                       int64_t* out_idx, const int64_t* excl_begin, const int64_t* excl_end,
+                                       const int32_t* excl_pos, rgcn_stream_t stream) {
+  int rc = check_excl(excl_begin, excl_end, excl_pos, "scores_topk_excl_w");
+  if (rc) return rc;
   GemmKParams p{};
-  int rc = scores_common(p, Q_hi, Q_lo, ldq, d, cand_planes, n_q, "scores_topk_w");
+  rc = scores_common(p, Q_hi, Q_lo, ldq, d, cand_planes, n_q, "scores_topk_w");
   if (rc) return rc;
   RGCN_CHECK_ARG(n_cand > 0 && n_cand < (1ll << 31) && k >= 1 && k <= kTopK && alpha > 0.f, "scores_topk_w: 1 <= k <= %d, alpha > 0", kTopK);
   RGCN_CHECK_ARG(cand_val && cand_idx && slot_ctr && out_val && out_idx, "scores_topk_w: null argument");
@@ -1393,6 +1459,7 @@ extern "C" int rgcn_scores_topk_w(const void* Q_hi, const void* Q_lo, int64_t ld
   RGCN_CUDA(cudaMemsetAsync(slot_ctr, 0, (size_t)n_q * sizeof(int32_t), st));
   p.N = (int)n_cand; p.n_cols_valid = n_cand; p.tile_contig = 1;
   p.alpha = alpha; p.beta = beta; p.cand_val = cand_val; p.cand_idx = cand_idx; p.slot_ctr = slot_ctr; p.n_slots = n_slots;
+  p.excl_begin = excl_begin; p.excl_end = excl_end; p.excl_pos = excl_pos;
   const int n_tiles = (int)((n_cand + KBN - 1) / KBN);
   const __nv_bfloat16* bhi = (const __nv_bfloat16*)cand_planes;
   const __nv_bfloat16* blo = (const __nv_bfloat16*)((const char*)cand_planes + wplane_bytes((int)n_cand, d));

@@ -254,12 +254,13 @@ class LinkPredictor(nn.Module):
                              labels, p, seed, ctr)
 
     def rank_tails(self, node_embeddings: torch.Tensor, head_indices: torch.Tensor, relation_types: torch.Tensor,
-                   tail_indices: torch.Tensor):
+                   tail_indices: torch.Tensor, filter=None):
         """(rank, ties) of the true tails among all entities — the fused form of ``score_all_tails`` + the per-row
-        ``argsort`` loop of reference src/evaluate.py:260-276."""
+        ``argsort`` loop of reference src/evaluate.py:260-276.  ``filter`` (a ``KnownTriples``): filtered ranks, the
+        other known tails of each (head, relation) left out."""
         from .rank import rank_true_tails
         return rank_true_tails(node_embeddings, self.relation_embeddings.weight, head_indices, relation_types,
-                               tail_indices)
+                               tail_indices, filter=filter)
 
 
 class _ScoreAllTails(torch.autograd.Function):

@@ -12,6 +12,11 @@ fp32 mode of the encoder).  ``alpha`` / ``beta`` ride along as one extra K colum
 The ranking counts come from the score block itself (``rgcn_rank_count``), a block of queries at a time.
 ``method="simt"`` keeps the fp32 FMA tile kernels of ``csrc/rank.cu`` (every output accumulated in ascending k order with
 ``fmaf``; they never materialise the [queries, candidates] block when ranking).
+
+Filtered ranking (Bordes et al. 2013) and top-k of novel links take a ``KnownTriples`` index: per query a sorted list
+of candidate positions to leave out.  The tensor-core epilogues skip them as they sweep (``rgcn_scores_rank_excl_w``,
+``rgcn_scores_topk_excl_w``); ``tc_block`` and ``simt`` count unfiltered and then take the excluded positions back out
+with the counting pass's own score bits (``rgcn_rank_excl_correct``).
 """
 from __future__ import annotations
 
@@ -23,6 +28,130 @@ from . import _lib
 from .graph import _ptr, _stream
 
 _RANK_BLOCK = 2048       # queries ranked per score block of the tensor-core path (2048 x 30,926 fp32 = 253 MB)
+
+ExclLists = Tuple[torch.Tensor, torch.Tensor, torch.Tensor]     # (begin [n] int64, end [n] int64, positions int32)
+
+
+def _lex_order(major: torch.Tensor, minor: torch.Tensor) -> torch.Tensor:
+    """Permutation sorting by (major, minor): two stable sorts, no packed key that could overflow."""
+    o = torch.argsort(minor, stable=True)
+    return o[torch.argsort(major[o], stable=True)]
+
+
+def _check_candidates(cand: torch.Tensor, num_nodes: int) -> None:
+    """A candidate list that positions are mapped into must name distinct nodes of the graph."""
+    if cand.numel() and (int(cand.min()) < 0 or int(cand.max()) >= num_nodes):
+        raise ValueError("candidates hold node ids outside the filter's graph")
+    if torch.unique(cand).numel() != cand.numel():
+        raise ValueError("candidates must be distinct when a filter / exclusion is given")
+
+
+class KnownTriples:
+    """Known (head, relation, tail) triples on the device, indexed by (head, relation) with the tails of each key sorted
+    and distinct (multi-edges are deduplicated).  The filter of ``rank_true_tails(filter=...)`` (filtered MRR / Hits@K:
+    the other known true tails of a query's (head, relation) leave the candidate set) and the exclusion of
+    ``topk_all_pairs(exclude=...)`` (only links that are not known yet).
+
+    Head-side filtered ranking needs no second function: DistMult is symmetric, so
+    ``rank_true_tails(emb, table, tails, rels, heads, filter=known.reversed())`` ranks every true head among all heads.
+    """
+
+    def __init__(self, heads: torch.Tensor, rels: torch.Tensor, tails: torch.Tensor, num_nodes: int, num_relations: int):
+        for name, t in (("heads", heads), ("rels", rels), ("tails", tails)):
+            if not isinstance(t, torch.Tensor) or t.dim() != 1 or t.numel() != heads.numel():
+                raise ValueError("KnownTriples: heads, rels and tails must be 1-D tensors of one length")
+            if t.dtype.is_floating_point or t.dtype == torch.bool:
+                raise ValueError(f"KnownTriples: {name} must hold integer ids")
+        if not (0 < num_nodes < 2 ** 31 and num_relations > 0):
+            raise ValueError("KnownTriples: need 0 < num_nodes < 2^31 and num_relations > 0")
+        heads, rels, tails = heads.to(torch.int64), rels.to(torch.int64), tails.to(torch.int64)
+        if heads.numel():
+            lo = torch.stack([heads.min(), rels.min(), tails.min()])
+            hi = torch.stack([heads.max() - num_nodes, rels.max() - num_relations, tails.max() - num_nodes])
+            if bool((lo < 0).any()) or bool((hi >= 0).any()):
+                raise ValueError(f"KnownTriples: ids out of range (num_nodes={num_nodes}, num_relations={num_relations})")
+        if not (heads.is_cuda and rels.is_cuda and tails.is_cuda):
+            raise ValueError("KnownTriples: heads, rels and tails must be CUDA tensors (the index lives on the device)")
+        self.num_nodes, self.num_relations = int(num_nodes), int(num_relations)
+        self.device = heads.device
+        key = heads * num_relations + rels
+        o = _lex_order(key, tails)
+        key, tails = key[o], tails[o]
+        keep = torch.ones_like(key, dtype=torch.bool)
+        keep[1:] = (key[1:] != key[:-1]) | (tails[1:] != tails[:-1])
+        self.keys = key[keep].contiguous()                      # head * num_relations + rel, ascending
+        self.tails = tails[keep].to(torch.int32).contiguous()   # ascending within each key
+        self._reversed: Optional["KnownTriples"] = None
+        self._any: Optional["KnownTriples"] = None
+        self._cand = None                                       # (candidates tensor, its version, keys, positions)
+
+    @classmethod
+    def from_graphs(cls, *graphs, device=None) -> "KnownTriples":
+        """Every edge of the given graphs (the reference's dicts ``{'edge_index', 'edge_type', 'num_nodes',
+        'num_relations'}``, e.g. train + val + test) as known triples; ``device`` moves CPU-held graphs over."""
+        if not graphs:
+            raise ValueError("KnownTriples.from_graphs needs at least one graph")
+        ei = torch.cat([g["edge_index"].to(device) if device is not None else g["edge_index"] for g in graphs], 1)
+        et = torch.cat([g["edge_type"].to(device) if device is not None else g["edge_type"] for g in graphs])
+        return cls(ei[0], et, ei[1], max(int(g["num_nodes"]) for g in graphs),
+                   max(int(g["num_relations"]) for g in graphs))
+
+    def __len__(self) -> int:
+        return int(self.keys.numel())
+
+    def reversed(self) -> "KnownTriples":
+        """The (tail, relation) -> head view, for filtered head ranking."""
+        if self._reversed is None:
+            R = self.num_relations
+            self._reversed = KnownTriples(self.tails.to(torch.int64), self.keys % R, self.keys // R, self.num_nodes, R)
+            self._reversed._reversed = self
+        return self._reversed
+
+    def any_relation(self) -> "KnownTriples":
+        """The relation-agnostic view: head -> every tail it links to under any relation (query it with relation 0)."""
+        if self._any is None:
+            R = self.num_relations
+            self._any = KnownTriples(self.keys // R, torch.zeros_like(self.keys), self.tails.to(torch.int64),
+                                     self.num_nodes, 1)
+        return self._any
+
+    def _on_candidates(self, candidates: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+        """(keys, positions) with the tails mapped to positions in ``candidates`` (non-candidates dropped, positions
+        ascending per key); cached for the last candidates tensor."""
+        c = self._cand
+        if c is not None and c[0] is candidates and c[1] == candidates._version:
+            return c[2], c[3]
+        cand = candidates.to(self.device, torch.int64).reshape(-1)
+        n = cand.numel()
+        _check_candidates(cand, self.num_nodes)
+        inv = torch.full((self.num_nodes,), -1, dtype=torch.int64, device=self.device)
+        inv[cand] = torch.arange(n, dtype=torch.int64, device=self.device)
+        pos = inv[self.tails.to(torch.int64)]
+        keep = pos >= 0
+        keys, pos = self.keys[keep], pos[keep]
+        o = _lex_order(keys, pos)
+        keys, pos = keys[o].contiguous(), pos[o].to(torch.int32).contiguous()
+        self._cand = (candidates, candidates._version, keys, pos)
+        return keys, pos
+
+    def lists(self, heads: torch.Tensor, rels, candidates: Optional[torch.Tensor] = None) -> ExclLists:
+        """Per query (heads[i], rels[i]) its known tails as the kernels' exclusion lists: (begin, end, positions), the
+        positions being node ids (``candidates=None``: ranges straight into the index) or positions in ``candidates``.
+        ``rels`` may be one int for all queries."""
+        heads = heads.to(self.device, torch.int64).reshape(-1)
+        if isinstance(rels, int):
+            rels = torch.full_like(heads, rels)
+        rels = rels.to(self.device, torch.int64).reshape(-1)
+        keys, pos = (self.keys, self.tails) if candidates is None else self._on_candidates(candidates)
+        q = heads * self.num_relations + rels
+        begin = torch.searchsorted(keys, q)
+        end = torch.searchsorted(keys, q, right=True)
+        # an id outside the index must not alias another key: empty list
+        bad = (heads < 0) | (heads >= self.num_nodes) | (rels < 0) | (rels >= self.num_relations)
+        end = torch.where(bad, begin, end)
+        if pos.numel() == 0:                # every range is empty, but the kernels take a non-null list pointer
+            pos = torch.zeros(1, dtype=torch.int32, device=self.device)
+        return begin.contiguous(), end.contiguous(), pos
 
 
 def _prep(emb: torch.Tensor, idx: Optional[torch.Tensor], rel_table: Optional[torch.Tensor],
@@ -136,9 +265,11 @@ def _candidate_rows(B: torch.Tensor, idx: Optional[torch.Tensor]) -> torch.Tenso
     return out
 
 
-def _rank_fused(A: torch.Tensor, B: torch.Tensor, cand: Optional[torch.Tensor], tails: torch.Tensor):
-    """Tensor-core sweep whose epilogue counts instead of storing (``rgcn_scores_rank_w``); the threshold comes from the
-    diagonal tiles of queries x (their own true tails) with the same K order, so it carries the sweep's own bits."""
+def _rank_fused(A: torch.Tensor, B: torch.Tensor, cand: Optional[torch.Tensor], tails: torch.Tensor,
+                excl: Optional[ExclLists] = None):
+    """Tensor-core sweep whose epilogue counts instead of storing (``rgcn_scores_rank_excl_w``); the threshold comes
+    from the diagonal tiles of queries x (their own true tails) with the same K order, so it carries the sweep's own
+    bits.  ``excl``: per-query positions the epilogue leaves out."""
     from . import ops
     lib = _lib.load()
     nq, d = A.shape
@@ -156,16 +287,19 @@ def _rank_fused(A: torch.Tensor, B: torch.Tensor, cand: Optional[torch.Tensor], 
     st = _stream(A.device)
     _lib.check(lib.rgcn_scores_diag_w(_ptr(Q[0]), _ptr(Q[1]), Q[0].stride(0), d, _ptr(tail_planes), nq, _ptr(thr), st),
                "rgcn_scores_diag_w")
-    _lib.check(lib.rgcn_scores_rank_w(_ptr(Q[0]), _ptr(Q[1]), Q[0].stride(0), d, _ptr(cand_planes), nb, nq, _ptr(thr),
-                                      _ptr(tails), _ptr(greater), _ptr(equal), st), "rgcn_scores_rank_w")
+    xb, xe, xp = excl if excl is not None else (None, None, None)
+    _lib.check(lib.rgcn_scores_rank_excl_w(_ptr(Q[0]), _ptr(Q[1]), Q[0].stride(0), d, _ptr(cand_planes), nb, nq,
+                                           _ptr(thr), _ptr(tails), _ptr(greater), _ptr(equal), _ptr(xb), _ptr(xe),
+                                           _ptr(xp), st), "rgcn_scores_rank_excl_w")
     return greater, equal
 
 
 def topk_from_rows(A: torch.Tensor, B: torch.Tensor, k: int, b_idx: Optional[torch.Tensor] = None, alpha: float = 1.0,
-                   beta: float = 0.0) -> Tuple[torch.Tensor, torch.Tensor]:
+                   beta: float = 0.0, excl: Optional[ExclLists] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """(values [n_a, k], positions [n_a, k]): per row of ``A`` the k best rows of ``B[b_idx]`` by alpha * <a, b> + beta,
     sorted by value (ties: lower position first); positions index ``b_idx`` (or B).  Tensor cores, the score block is
-    consumed in the epilogue (``rgcn_scores_topk_w``), k <= 16."""
+    consumed in the epilogue (``rgcn_scores_topk_excl_w``), k <= 16.  ``excl`` (``KnownTriples.lists``): per row of A
+    the positions that are never returned; a row left with fewer than k candidates ends in -inf / -1."""
     from . import ops
     lib = _lib.load()
     if not (1 <= k <= 16):
@@ -188,42 +322,66 @@ def topk_from_rows(A: torch.Tensor, B: torch.Tensor, k: int, b_idx: Optional[tor
     ctr = torch.empty(na, dtype=torch.int32, device=dev)
     ov = torch.empty(na, k, dtype=torch.float32, device=dev)
     oi = torch.empty(na, k, dtype=torch.int64, device=dev)
-    _lib.check(lib.rgcn_scores_topk_w(_ptr(Q[0]), _ptr(Q[1]), Q[0].stride(0), d, _ptr(cand_planes), nb, na, int(k),
-                                      float(alpha), float(beta), _ptr(cv), _ptr(ci), _ptr(ctr), slots, _ptr(ov), _ptr(oi),
-                                      _stream(dev)), "rgcn_scores_topk_w")
+    xb, xe, xp = excl if excl is not None else (None, None, None)
+    _lib.check(lib.rgcn_scores_topk_excl_w(_ptr(Q[0]), _ptr(Q[1]), Q[0].stride(0), d, _ptr(cand_planes), nb, na, int(k),
+                                           float(alpha), float(beta), _ptr(cv), _ptr(ci), _ptr(ctr), slots, _ptr(ov),
+                                           _ptr(oi), _ptr(xb), _ptr(xe), _ptr(xp), _stream(dev)),
+               "rgcn_scores_topk_excl_w")
     return ov, oi
 
 
 def topk_all_pairs(emb: torch.Tensor, a_idx: torch.Tensor, b_idx: torch.Tensor, k: int = 10,
-                   rel_vec: Optional[torch.Tensor] = None, cosine: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+                   rel_vec: Optional[torch.Tensor] = None, cosine: bool = False,
+                   exclude: Optional[KnownTriples] = None, exclude_relation: Optional[int] = None
+                   ) -> Tuple[torch.Tensor, torch.Tensor]:
     """Per row of ``a_idx`` the k best of ``b_idx`` — DistMult ``(emb[a] * rel_vec) . emb[b]`` or cosine ``(cos + 1) / 2`` —
     without the [len(a), len(b)] matrix: (scores [len(a), k], node ids [len(a), k]).  The device form of the per-disease /
     per-drug sweeps + top-k filters of src/compare_methods.py:384-397, src/medical_validation.py:222-239 and
-    src/case_studies.py:260-274 (fused L2 normalisation, fused rescale)."""
+    src/case_studies.py:260-274 (fused L2 normalisation, fused rescale).
+
+    ``exclude``: return novel links only — ``b`` is left out for row ``a`` when (a, exclude_relation, b) is a known
+    triple, or, with ``exclude_relation=None``, when (a, r, b) is known for any relation r.  ``b_idx`` must then be
+    distinct; a row with fewer than k admissible candidates ends in -inf / -1."""
+    excl = None
+    if exclude is not None:
+        if exclude_relation is None:
+            view, rel = exclude.any_relation(), 0
+        else:
+            if not 0 <= int(exclude_relation) < exclude.num_relations:
+                raise ValueError(f"exclude_relation={exclude_relation} outside [0, {exclude.num_relations})")
+            view, rel = exclude, int(exclude_relation)
+        excl = view.lists(a_idx, rel, b_idx)
+    elif exclude_relation is not None:
+        raise ValueError("exclude_relation needs exclude=")
     b_idx = b_idx.to(torch.int64)
     if cosine:
         A = _prep(emb, a_idx, None, None, True)
         Bn = _prep(emb, b_idx, None, None, True)
-        val, pos = topk_from_rows(A, Bn, k, None, 0.5, 0.5)
+        val, pos = topk_from_rows(A, Bn, k, None, 0.5, 0.5, excl=excl)
     else:
         if rel_vec is not None:
             A = _prep(emb, a_idx, rel_vec.reshape(1, -1), torch.zeros(a_idx.numel(), dtype=torch.int64, device=emb.device), False)
         else:
             A = _prep(emb, a_idx, None, None, False)
-        val, pos = topk_from_rows(A, emb, k, b_idx)
+        val, pos = topk_from_rows(A, emb, k, b_idx, excl=excl)
     ids = torch.where(pos >= 0, b_idx[pos.clamp(min=0)], pos)
     return val, ids
 
 
 def rank_true_tails(emb: torch.Tensor, rel_table: torch.Tensor, heads: torch.Tensor, rels: torch.Tensor,
-                    tails: torch.Tensor, candidates: Optional[torch.Tensor] = None, method: str = "tc"
-                    ) -> Tuple[torch.Tensor, torch.Tensor]:
+                    tails: torch.Tensor, candidates: Optional[torch.Tensor] = None, method: str = "tc",
+                    filter: Optional[KnownTriples] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """(rank, ties): rank[i] = 1 + #{candidates scoring strictly above the true tail} (int64, 1-indexed like
     src/evaluate.py:274); ties[i] = #{other candidates with exactly the true tail's score}.  ``candidates`` = index list
     of admissible tails (default: all entities); ``tails`` then holds POSITIONS in that list.
     ``method``: "tc" = tensor cores, counts taken in the GEMM epilogue (no score block); "tc_block" = tensor cores through
-    materialised 2,048-query score blocks (round 1); "simt" = fp32 FMA tiles."""
+    materialised 2,048-query score blocks (round 1); "simt" = fp32 FMA tiles.
+    ``filter``: the filtered protocol (Bordes et al. 2013) — every known tail of (heads[i], rels[i]) other than the true
+    one leaves row i's candidate set, so it counts in neither rank nor ties (``candidates`` must then be distinct).
+    Filtered head ranks: ``rank_true_tails(emb, rel_table, tails, rels, heads, filter=known.reversed())`` (DistMult
+    is symmetric)."""
     lib = _lib.load()
+    excl = None if filter is None else filter.lists(heads, rels, candidates)
     A = _prep(emb, heads, rel_table, rels, False)
     B = emb.detach().to(torch.float32)
     if B.stride(1) != 1 or B.stride(0) % 4 or B.data_ptr() % 16:
@@ -235,24 +393,44 @@ def rank_true_tails(emb: torch.Tensor, rel_table: torch.Tensor, heads: torch.Ten
     greater = torch.empty(nq, dtype=torch.int32, device=A.device)
     equal = torch.empty(nq, dtype=torch.int32, device=A.device)
     if method == "tc" and nq > 0 and nb > 0 and A.size(1) % 4 == 0:
-        greater, equal = _rank_fused(A, B, cand, tails)
+        greater, equal = _rank_fused(A, B, cand, tails, excl)
         return greater.to(torch.int64) + 1, equal.to(torch.int64)
+    st = _stream(A.device)
+
+    def correct(q0, q1, thr, S=None):
+        # filtered counts: the excluded positions' own scores (block bits, or recomputed as the FMA tiles compute them)
+        # leave the unfiltered counts of rows q0 .. q1
+        if excl is None:
+            return
+        xb, xe, xp = excl
+        if S is not None:
+            ops = (_ptr(S), S.stride(0), None, 0, None, 0, None, A.size(1))
+        else:
+            ops = (None, 0, _ptr(A), A.stride(0), _ptr(B), B.stride(0), _ptr(cand), A.size(1))
+        _lib.check(lib.rgcn_rank_excl_correct(*ops, q1 - q0, nb, _ptr(tails[q0:q1]), _ptr(thr), _ptr(xb[q0:q1]),
+                                              _ptr(xe[q0:q1]), _ptr(xp), _ptr(greater[q0:q1]), _ptr(equal[q0:q1]), st),
+                   "rgcn_rank_excl_correct")
+
     if method in ("tc", "tc_block") and nq > 0 and nb > 0 and A.size(1) % 4 == 0:
         Bext = _tc_candidates(B, cand, 1.0, 0.0)
         # queries per score block: at most _RANK_BLOCK, and at most ~1 GiB of scores for very large candidate sets
         qb = max(128, min(_RANK_BLOCK, (1 << 28) // max(Bext.size(0), 1) // 128 * 128))
+        thr = None if excl is None else torch.empty(nq, dtype=torch.float32, device=A.device)
         for q0 in range(0, nq, qb):
             q1 = min(q0 + qb, nq)
             S = _tc_block(A[q0:q1], Bext, 1.0, 0.0)
-            _lib.check(lib.rgcn_rank_count(_ptr(S), S.stride(0), q1 - q0, nb, _ptr(tails[q0:q1]), None, _ptr(greater[q0:q1]),
-                                           _ptr(equal[q0:q1]), _stream(A.device)), "rgcn_rank_count")
+            _lib.check(lib.rgcn_rank_count(_ptr(S), S.stride(0), q1 - q0, nb, _ptr(tails[q0:q1]),
+                                           None if thr is None else _ptr(thr[q0:q1]), _ptr(greater[q0:q1]),
+                                           _ptr(equal[q0:q1]), st), "rgcn_rank_count")
+            correct(q0, q1, None if thr is None else thr[q0:q1], S)
         return greater.to(torch.int64) + 1, equal.to(torch.int64)
     if method not in ("tc", "tc_block", "simt"):
         raise ValueError("method must be 'tc' (tensor cores, fused count), 'tc_block' or 'simt' (fp32 FMA tiles)")
     thr = torch.empty(nq, dtype=torch.float32, device=A.device)
     _lib.check(lib.rgcn_allpairs_rank(_ptr(A), A.stride(0), nq, _ptr(B), B.stride(0), _ptr(cand), nb, A.size(1),
-                                      _ptr(tails), _ptr(thr), _ptr(greater), _ptr(equal), _stream(A.device)),
+                                      _ptr(tails), _ptr(thr), _ptr(greater), _ptr(equal), st),
                "rgcn_allpairs_rank")
+    correct(0, nq, thr)
     return greater.to(torch.int64) + 1, equal.to(torch.int64)
 
 
