@@ -4,10 +4,14 @@ Per step: positives in -> negatives drawn on the device -> full-graph 2-layer RG
 accuracy -> backward, all replayed as ONE CUDA graph (``GraphedTrainStep`` with a ``NegativeSampler``), then the
 reference's own clipping and Adam step (src/train.py:311-318).  ``--optimizer fused`` passes a ``FusedAdam(max_grad_norm=1.0)``
 into the graphed step instead: clipping and Adam become the last kernels of the same graph, one replay per iteration.
+``--negatives filtered`` redraws negatives that are edges of the graph; ``typed`` also keeps every replaced end to a node
+type the relation takes on that side (the graph's three type blocks) and picks head or tail with the Bernoulli
+probability of the relation; ``uniform`` (default) is the reference's sampler.
 Loss and accuracy stay on the device and are read once per logging interval instead of twice per step (src/train.py:322,
 :325).
 
     python examples/train_synthetic.py [--steps 300] [--hidden 128] [--batch 1024] [--optimizer torch|fused]
+                                        [--negatives uniform|filtered|typed]
 """
 import argparse
 import os
@@ -29,6 +33,7 @@ def main():
     ap.add_argument("--lr", type=float, default=0.01)
     ap.add_argument("--edges", type=int, default=849_456)
     ap.add_argument("--optimizer", choices=("torch", "fused"), default="torch")
+    ap.add_argument("--negatives", choices=("uniform", "filtered", "typed"), default="uniform")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     torch.manual_seed(42)
@@ -39,7 +44,17 @@ def main():
     fused = args.optimizer == "fused"
     opt = (pkg.FusedAdam(model.parameters(), lr=args.lr, max_grad_norm=1.0) if fused
            else torch.optim.Adam(model.parameters(), lr=args.lr))
-    sampler = pkg.NegativeSampler(kg.num_nodes, 1)
+    kw = {}
+    if args.negatives != "uniform":
+        known = pkg.KnownTriples.from_graphs(kg.as_dict(), device=dev)
+        kw["filter"] = known
+        if args.negatives == "typed":
+            node_type = torch.empty(kg.num_nodes, dtype=torch.int64)
+            for i, (lo, hi) in enumerate(kg.blocks.values()):
+                node_type[lo:hi] = i
+            kw["constraints"] = pkg.RelationConstraints.from_node_types(known, node_type)
+            kw["head_prob"] = known.bernoulli_head_prob()
+    sampler = pkg.NegativeSampler(kg.num_nodes, 1, **kw)
     step = pkg.GraphedTrainStep(model, ei, et, batch_size=2 * args.batch, sampler=sampler,
                                 optimizer=opt if fused else None)
     params = [p for p in model.parameters()]
@@ -66,6 +81,8 @@ def main():
     if first is not None and last is not None and args.steps >= 100:
         assert last < first, "the loss did not go down"
         print(f"loss {first:.4f} -> {last:.4f}")
+    if args.negatives != "uniform":
+        print(f"negatives that kept a rejected draw: {int(sampler.exhausted)}")
 
 
 if __name__ == "__main__":

@@ -611,6 +611,55 @@ int rgcn_bce_logits_bwd(const float* logits, const float* labels, int64_t n, con
 int rgcn_link_batch(const int64_t* pos_head, const int64_t* pos_tail, const int64_t* pos_rel, int64_t n_pos,
                     int32_t num_neg, int64_t num_nodes, uint32_t seed, unsigned long long* counter,
                     int64_t* heads, int64_t* tails, int64_t* rels, float* labels, rgcn_stream_t stream);
+
+/* Generalised negative sampler: rgcn_link_batch plus filtered (Bordes et al. 2013), type-constrained (Krompaß et al.
+ * 2015) and Bernoulli head / tail (Wang et al. 2014) negatives.  Same layout as rgcn_link_batch; rgcn_link_batch is
+ * this call with no tables and one block.
+ *   side    : negative i of positive q replaces its head with probability head_prob[rel_q] (NULL: 1/2), else its tail;
+ *             chosen once, from attempt 0's draw.
+ *   entity  : attempt j draws uniformly from the side's admissible list of rel_q (the multiply-shift of a 32-bit
+ *             draw into the list length; an empty list = all num_nodes nodes) and is rejected when the corrupted
+ *             triple is in the filter.  After max_tries rejections the last draw is kept (label 0 all the same) and
+ *             *exhausted (nullable) is incremented.
+ *   draws   : a counter-based hash of (seed, *counter, i, j); attempt 0 is rgcn_link_batch's draw, so with no tables
+ *             and head_prob = NULL the output is rgcn_link_batch's, bit for bit.  A positive whose relation is outside
+ *             [0, num_rel) gets an unconstrained, unfiltered draw with head probability 1/2.
+ *   filter  : the forward index of known triples: filter_keys [n_filter] = head * num_rel + rel ascending, filter_tails
+ *             [n_filter] ascending within each key (KnownTriples.keys / .tails).  Both NULL: no filter.
+ *   types   : head_offsets / tail_offsets [num_rel + 1] (CSR) into head_nodes / tail_nodes: the admissible heads /
+ *             tails of each relation.  All four NULL: unconstrained.
+ *   counter : advanced by exactly one per call; every block draws with the value before the call.  ticket NULL: one
+ *             block of 1024 threads; otherwise one thread per output entry, and the last block to finish advances the
+ *             counter and resets *ticket (an unsigned int, ZEROED once before first use).
+ * The struct is read on the host and passed to the kernel by value.  Arguments are checked before any CUDA call. */
+typedef struct rgcn_link_batch_args {
+  const int64_t* pos_head;
+  const int64_t* pos_tail;
+  const int64_t* pos_rel;
+  int64_t n_pos;
+  int32_t num_neg;
+  int32_t num_rel;            /* rows of head_prob and of the type tables; may be 0 when none is given */
+  int64_t num_nodes;
+  uint32_t seed;
+  int32_t max_tries;          /* >= 1 */
+  unsigned long long* counter;
+  int64_t* heads;
+  int64_t* tails;
+  int64_t* rels;
+  float* labels;
+  const float* head_prob;     /* [num_rel] in [0, 1], nullable */
+  const int64_t* filter_keys;
+  const int32_t* filter_tails;
+  int64_t n_filter;
+  const int64_t* head_offsets;
+  const int32_t* head_nodes;
+  const int64_t* tail_offsets;
+  const int32_t* tail_nodes;
+  unsigned long long* exhausted;
+  unsigned int* ticket;
+} rgcn_link_batch_args;
+
+int rgcn_link_batch_ex(const rgcn_link_batch_args* args_host, rgcn_stream_t stream);
 size_t rgcn_link_loss_workspace_bytes(int64_t n_pairs);
 int rgcn_link_loss_fwd(const float* emb, int64_t ld, const int64_t* head, const int64_t* tail, const int64_t* rel,
                        const float* rel_table, const float* labels, int64_t n_pairs, int32_t d, float dropout_p,

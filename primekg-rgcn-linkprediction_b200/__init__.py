@@ -10,10 +10,10 @@ from .graph import RelGraph, clear_graph_cache, get_graph, graph_from_state, gra
 from .graphed import GraphedTrainStep
 from .rank import KnownTriples, rank_true_tails, ranking_metrics, score_all_pairs, topk_all_pairs
 from .modules import DrugDiseaseModel, DrugDiseaseRGCN, LinkPredictor
-from .sampler import NegativeSampler
+from .sampler import NegativeSampler, RelationConstraints
 from .optim import FusedAdam, FusedAdamW
 
 __all__ = ["RGCNConv", "DrugDiseaseRGCN", "LinkPredictor", "DrugDiseaseModel", "RelGraph", "get_graph",
            "clear_graph_cache", "default_mode", "GraphedTrainStep", "graph_state", "graph_from_state", "register_graph", "KnownTriples", "rank_true_tails", "ranking_metrics", "score_all_pairs", "topk_all_pairs",
-           "NegativeSampler", "FusedAdam", "FusedAdamW"]
+           "NegativeSampler", "RelationConstraints", "FusedAdam", "FusedAdamW"]
 __version__ = "0.1.0"

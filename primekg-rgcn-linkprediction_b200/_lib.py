@@ -77,6 +77,16 @@ class AdamHparams(C.Structure):
     _fields_ = [("lr", C.c_double), ("beta1", C.c_double), ("beta2", C.c_double), ("eps", C.c_double),
                 ("weight_decay", C.c_double), ("decoupled_weight_decay", i32)]
 
+
+class LinkBatchArgs(C.Structure):
+    """Mirror of ``rgcn_link_batch_args`` (include/rgcn_b200.h)."""
+    _fields_ = [("pos_head", p), ("pos_tail", p), ("pos_rel", p), ("n_pos", i64), ("num_neg", i32), ("num_rel", i32),
+                ("num_nodes", i64), ("seed", u32), ("max_tries", i32), ("counter", p),
+                ("heads", p), ("tails", p), ("rels", p), ("labels", p), ("head_prob", p),
+                ("filter_keys", p), ("filter_tails", p), ("n_filter", i64),
+                ("head_offsets", p), ("head_nodes", p), ("tail_offsets", p), ("tail_nodes", p),
+                ("exhausted", p), ("ticket", p)]
+
 # name -> (restype, argtypes); must list every symbol of include/rgcn_b200.h
 PROTOTYPES = {
     "rgcn_abi_version": (C.c_int, []),
@@ -145,6 +155,7 @@ PROTOTYPES = {
     "rgcn_bce_logits_fwd": (C.c_int, [p, p, i64, p, p, p]),
     "rgcn_bce_logits_bwd": (C.c_int, [p, p, i64, p, p, p]),
     "rgcn_link_batch": (C.c_int, [p, p, p, i64, i32, i64, u32, p, p, p, p, p, p]),
+    "rgcn_link_batch_ex": (C.c_int, [C.POINTER(LinkBatchArgs), p]),
     "rgcn_link_loss_workspace_bytes": (sz, [i64]),
     "rgcn_link_loss_fwd": (C.c_int, [p, i64, p, p, p, p, p, i64, i32, C.c_float, u32, p, p, p, p, p, i64, i32, p, p, sz, p]),
     "rgcn_link_loss_bwd": (C.c_int, [p, i64, p, p, p, p, p, p, p, p, i64, i32, C.c_float, u32, p, p, i64, p, i32, i64, p]),

@@ -145,32 +145,90 @@ __device__ __forceinline__ uint2 draw2(uint32_t seed, unsigned long long ctr, ui
   return make_uint2(a, pcg32(a + 0x85EBCA6Bu + i));
 }
 
+// entity draw of attempt j >= 1 of negative i: a re-hash of attempt 0's side word x (itself a hash of seed, counter
+// value and i) with j — a pure function of (seed, counter value, i, j)
+__device__ __forceinline__ uint32_t redraw(uint32_t x, uint32_t i, uint32_t j) {
+  return pcg32(pcg32(x ^ (j * 0x9E3779B9u)) + i);
+}
+
+// (key, t) in the lexicographically sorted pairs (keys[k], tails[k]), k < n: one binary search over both columns,
+// the two loads of a step issued together
+__device__ __forceinline__ bool known_triple(const int64_t* __restrict__ keys, const int32_t* __restrict__ tails,
+                                             int64_t n, int64_t key, int32_t t) {
+  int64_t lo = 0, len = n;
+  while (len > 0) {
+    const int64_t half = len >> 1, m = lo + half;
+    const int64_t km = __ldg(keys + m);
+    const int32_t tm = __ldg(tails + m);
+    if (km < key || (km == key && tm < t)) { lo = m + 1; len -= half + 1; }
+    else len = half;
+  }
+  return lo < n && __ldg(keys + lo) == key && __ldg(tails + lo) == t;
+}
+
 // Negative sampling of reference src/train.py:59-97 + the concatenation / labels of :281-288 on device: out[0 .. n_pos)
-// = the positives (label 1); out[n_pos + i * num_neg + k] = positive i with its head (probability 1/2) or else its
-// tail replaced by a uniform node (label 0).  One block: every thread reads the step counter, then thread 0 advances
-// it — a captured graph draws fresh negatives on every replay.
-__global__ void __launch_bounds__(1024) link_batch_kernel(const int64_t* __restrict__ ph, const int64_t* __restrict__ pt,
-                                                          const int64_t* __restrict__ pr, int64_t n_pos, int32_t num_neg,
-                                                          int64_t num_nodes, uint32_t seed, unsigned long long* ctr,
-                                                          int64_t* __restrict__ heads, int64_t* __restrict__ tails,
-                                                          int64_t* __restrict__ rels, float* __restrict__ labels) {
+// = the positives (label 1); out[n_pos + i * num_neg + k] = positive i with its head (probability head_prob[r], default
+// 1/2) or else its tail replaced (label 0) by a node drawn uniformly from the relation's admissible list for that side
+// (default: all nodes), redrawn while the corrupted triple is a known one (rgcn_link_batch_ex).  Every thread reads the
+// step counter first; one block: thread 0 then advances it, several blocks: the last block to finish does — a captured
+// graph draws fresh negatives on every replay.
+__global__ void __launch_bounds__(1024) link_batch_kernel(const rgcn_link_batch_args a) {
   pdl_enter();
-  const unsigned long long c = *ctr;
+  const unsigned long long c = *a.counter;
   __syncthreads();
-  if (threadIdx.x == 0) *ctr = c + 1ull;
-  const int64_t n_neg = n_pos * num_neg;
-  for (int64_t i = threadIdx.x; i < n_pos + n_neg; i += 1024) {
-    if (i < n_pos) {
-      heads[i] = ph[i]; tails[i] = pt[i]; rels[i] = pr[i]; labels[i] = 1.f;
-    } else {
-      const int64_t q = (i - n_pos) / num_neg;
-      const uint2 r = draw2(seed, c, (uint32_t)(i - n_pos));
-      const bool corrupt_head = (r.x >> 31) != 0u;
-      // uniform in [0, num_nodes): multiply-shift of a 32-bit draw (bias < num_nodes / 2^32)
-      const int64_t ent = (int64_t)(((unsigned long long)r.y * (unsigned long long)num_nodes) >> 32);
-      heads[i] = corrupt_head ? ent : ph[q];
-      tails[i] = corrupt_head ? pt[q] : ent;
-      rels[i] = pr[q]; labels[i] = 0.f;
+  const bool one_block = gridDim.x == 1;
+  if (one_block && threadIdx.x == 0) *a.counter = c + 1ull;
+  const int64_t n_neg = a.n_pos * a.num_neg, n_out = a.n_pos + n_neg;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_out; i += stride) {
+    if (i < a.n_pos) {
+      a.heads[i] = a.pos_head[i]; a.tails[i] = a.pos_tail[i]; a.rels[i] = a.pos_rel[i]; a.labels[i] = 1.f;
+      continue;
+    }
+    const int64_t q = (i - a.n_pos) / a.num_neg;
+    const uint32_t ni = (uint32_t)(i - a.n_pos);
+    const uint2 r = draw2(a.seed, c, ni);
+    const int64_t hq = a.pos_head[q], tq = a.pos_tail[q], rq = a.pos_rel[q];
+    const bool rel_ok = rq >= 0 && rq < (int64_t)a.num_rel;      // else: no table is read
+    // head with probability p: x >= (1 - p) 2^32, which for p = 1/2 is the top bit and is exact for p = 0 and 1
+    unsigned long long thr = 1ull << 31;
+    if (a.head_prob && rel_ok) thr = (unsigned long long)((1.0 - (double)a.head_prob[rq]) * 4294967296.0);
+    const bool corrupt_head = (unsigned long long)r.x >= thr;
+    const int64_t* offs = corrupt_head ? a.head_offsets : a.tail_offsets;
+    const int32_t* nodes = corrupt_head ? a.head_nodes : a.tail_nodes;
+    int64_t base = 0, len = 0;                                    // len 0: all nodes
+    if (offs && rel_ok) { base = offs[rq]; len = offs[rq + 1] - base; }
+    const int64_t kept = corrupt_head ? tq : hq;
+    const bool filtered = a.filter_keys && rel_ok && kept >= 0 && kept < a.num_nodes;
+    uint32_t y = r.y;
+    int64_t ent;
+    for (int32_t j = 0;;) {
+      // uniform in [0, len): multiply-shift of a 32-bit draw (bias < len / 2^32)
+      ent = len > 0 ? (int64_t)__ldg(nodes + base + (int64_t)(((unsigned long long)y * (unsigned long long)len) >> 32))
+                    : (int64_t)(((unsigned long long)y * (unsigned long long)a.num_nodes) >> 32);
+      if (!filtered ||
+          !known_triple(a.filter_keys, a.filter_tails, a.n_filter, (corrupt_head ? ent : hq) * a.num_rel + rq,
+                        (int32_t)(corrupt_head ? tq : ent)))
+        break;
+      if (++j == a.max_tries) {                                   // keep the last draw
+        if (a.exhausted) atomicAdd(a.exhausted, 1ull);
+        break;
+      }
+      y = redraw(r.x, ni, (uint32_t)j);
+    }
+    a.heads[i] = corrupt_head ? ent : hq;
+    a.tails[i] = corrupt_head ? tq : ent;
+    a.rels[i] = rq; a.labels[i] = 0.f;
+  }
+  if (!one_block) {
+    // every thread of this block has read the counter; the last block to arrive advances it
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      __threadfence();
+      if (atomicAdd(a.ticket, 1u) == gridDim.x - 1) {
+        *a.ticket = 0u;                               // ready for the next launch (graph replay)
+        *a.counter = c + 1ull;
+      }
     }
   }
 }
@@ -646,17 +704,42 @@ extern "C" int rgcn_bce_logits_bwd(const float* logits, const float* labels, int
   return RGCN_OK;
 }
 
+extern "C" int rgcn_link_batch_ex(const rgcn_link_batch_args* args_host, rgcn_stream_t stream) {
+  RGCN_CHECK_ARG(args_host, "link_batch: null args");
+  const rgcn_link_batch_args& a = *args_host;
+  RGCN_CHECK_ARG(a.n_pos >= 0 && a.num_neg >= 0 && a.num_nodes > 0 && a.num_nodes < (1ll << 32) && a.num_rel >= 0 &&
+                 a.n_filter >= 0, "link_batch: bad sizes");
+  RGCN_CHECK_ARG(a.num_neg == 0 || a.n_pos <= (int64_t)0xffffffffll / a.num_neg,
+                 "link_batch: bad sizes (more than 2^32 - 1 negatives)");
+  RGCN_CHECK_ARG(a.max_tries >= 1, "link_batch: max_tries must be >= 1");
+  RGCN_CHECK_ARG(!a.filter_keys == !a.filter_tails && (a.n_filter == 0 || a.filter_keys),
+                 "link_batch: filter_keys and filter_tails must both be null or both be set");
+  const int n_type_tables = !!a.head_offsets + !!a.head_nodes + !!a.tail_offsets + !!a.tail_nodes;
+  RGCN_CHECK_ARG(n_type_tables == 0 || n_type_tables == 4,
+                 "link_batch: the four type-constraint tables must all be null or all be set");
+  const bool tables = a.head_prob || a.filter_keys || n_type_tables;
+  RGCN_CHECK_ARG(!tables || a.num_rel > 0, "link_batch: head_prob / filter / type tables need num_rel > 0");
+  RGCN_CHECK_ARG(!(a.filter_keys || n_type_tables) || a.num_nodes < (1ll << 31),
+                 "link_batch: filter / type tables hold int32 node ids: num_nodes must be < 2^31");
+  RGCN_CHECK_ARG(a.n_pos == 0 || (a.pos_head && a.pos_tail && a.pos_rel && a.heads && a.tails && a.rels && a.labels &&
+                                  a.counter), "link_batch: null argument");
+  if (a.n_pos == 0) return RGCN_OK;
+  // with a ticket: one thread per output entry, so that num_neg = 16 batches do not queue behind one block
+  const int64_t n_out = a.n_pos * (1 + (int64_t)a.num_neg);
+  const unsigned grid = a.ticket ? (unsigned)((n_out + 255) / 256) : 1u;
+  RGCN_CUDA(launch_pdl(link_batch_kernel, dim3(grid), dim3(a.ticket ? 256 : 1024), 0, (cudaStream_t)stream, a));
+  RGCN_LAUNCH_CHECK();
+  return RGCN_OK;
+}
+
 extern "C" int rgcn_link_batch(const int64_t* pos_head, const int64_t* pos_tail, const int64_t* pos_rel, int64_t n_pos,
                                int32_t num_neg, int64_t num_nodes, uint32_t seed, unsigned long long* counter,
                                int64_t* heads, int64_t* tails, int64_t* rels, float* labels, rgcn_stream_t stream) {
-  RGCN_CHECK_ARG(n_pos >= 0 && num_neg >= 0 && num_nodes > 0 && num_nodes < (1ll << 32), "link_batch: bad sizes");
-  RGCN_CHECK_ARG(n_pos == 0 || (pos_head && pos_tail && pos_rel && heads && tails && rels && labels && counter),
-                 "link_batch: null argument");
-  if (n_pos == 0) return RGCN_OK;
-  RGCN_CUDA(launch_pdl(link_batch_kernel, dim3(1), dim3(1024), 0, (cudaStream_t)stream, pos_head, pos_tail, pos_rel, n_pos,
-                       num_neg, num_nodes, seed, counter, heads, tails, rels, labels));
-  RGCN_LAUNCH_CHECK();
-  return RGCN_OK;
+  rgcn_link_batch_args a{};
+  a.pos_head = pos_head; a.pos_tail = pos_tail; a.pos_rel = pos_rel; a.n_pos = n_pos; a.num_neg = num_neg;
+  a.num_nodes = num_nodes; a.seed = seed; a.max_tries = 1; a.counter = counter;
+  a.heads = heads; a.tails = tails; a.rels = rels; a.labels = labels;
+  return rgcn_link_batch_ex(&a, stream);
 }
 
 static int fill_link_params(LinkLossParams& q, const float* emb, int64_t ld, const int64_t* head, const int64_t* tail,

@@ -792,8 +792,15 @@ def link_batch(pos_head: torch.Tensor, pos_tail: torch.Tensor, pos_rel: torch.Te
     ``out``: four preallocated tensors (e.g. the static buffers of a captured step)."""
     lib = _lib.load()
     ph, pt, pr = _idx(pos_head, "pos_head"), _idx(pos_tail, "pos_tail"), _idx(pos_rel, "pos_rel")
-    n = ph.numel()
-    tot = n * (1 + num_neg)
+    h, t, r, y = out = _link_batch_out(ph, num_neg, out)
+    _lib.check(lib.rgcn_link_batch(_ptr(ph), _ptr(pt), _ptr(pr), ph.numel(), int(num_neg), int(num_nodes),
+                                   int(seed) & 0xFFFFFFFF, _ptr(counter), _ptr(h), _ptr(t), _ptr(r), _ptr(y),
+                                   _stream(ph.device)), "rgcn_link_batch")
+    return out
+
+
+def _link_batch_out(ph: torch.Tensor, num_neg: int, out):
+    tot = ph.numel() * (1 + num_neg)
     dev = ph.device
     if out is None:
         out = (torch.empty(tot, dtype=torch.int64, device=dev), torch.empty(tot, dtype=torch.int64, device=dev),
@@ -802,8 +809,31 @@ def link_batch(pos_head: torch.Tensor, pos_tail: torch.Tensor, pos_rel: torch.Te
     if not (h.numel() == t.numel() == r.numel() == y.numel() == tot and h.dtype == t.dtype == r.dtype == torch.int64
             and y.dtype == torch.float32 and all(x.is_contiguous() for x in out)):
         raise ValueError("out must be (int64, int64, int64, float32) contiguous tensors of n_pos * (1 + num_neg) entries")
-    _lib.check(lib.rgcn_link_batch(_ptr(ph), _ptr(pt), _ptr(pr), n, int(num_neg), int(num_nodes), int(seed) & 0xFFFFFFFF,
-                                   _ptr(counter), _ptr(h), _ptr(t), _ptr(r), _ptr(y), _stream(dev)), "rgcn_link_batch")
+    return out
+
+
+def link_batch_ex(pos_head: torch.Tensor, pos_tail: torch.Tensor, pos_rel: torch.Tensor, num_nodes: int, num_neg: int,
+                  seed: int, counter: torch.Tensor, out=None, *, num_rel: int = 0,
+                  head_prob: Optional[torch.Tensor] = None, filter=None, constraints=None, max_tries: int = 1,
+                  exhausted: Optional[torch.Tensor] = None, ticket: Optional[torch.Tensor] = None):
+    """``link_batch`` with the tables of ``rgcn_link_batch_ex``, all device tensors: ``head_prob`` float32 [num_rel];
+    ``filter`` = (keys int64, tails int32) of a ``KnownTriples``; ``constraints`` = (head_offsets int64 [num_rel + 1],
+    head_nodes int32, tail_offsets, tail_nodes); ``exhausted`` int64 [1], incremented per negative that kept a rejected
+    draw; ``ticket`` int32 [1], zero before the first call: one thread per output entry instead of one block.  The
+    tables' contents are not checked here (``NegativeSampler`` checks them once at construction)."""
+    lib = _lib.load()
+    ph, pt, pr = _idx(pos_head, "pos_head"), _idx(pos_tail, "pos_tail"), _idx(pos_rel, "pos_rel")
+    h, t, r, y = out = _link_batch_out(ph, num_neg, out)
+    fk, ft = filter if filter is not None else (None, None)
+    ho, hn, to, tn = constraints if constraints is not None else (None, None, None, None)
+    a = _lib.LinkBatchArgs(
+        pos_head=_ptr(ph), pos_tail=_ptr(pt), pos_rel=_ptr(pr), n_pos=ph.numel(), num_neg=int(num_neg),
+        num_rel=int(num_rel), num_nodes=int(num_nodes), seed=int(seed) & 0xFFFFFFFF, max_tries=int(max_tries),
+        counter=_ptr(counter), heads=_ptr(h), tails=_ptr(t), rels=_ptr(r), labels=_ptr(y), head_prob=_ptr(head_prob),
+        filter_keys=_ptr(fk), filter_tails=_ptr(ft), n_filter=0 if fk is None else fk.numel(),
+        head_offsets=_ptr(ho), head_nodes=_ptr(hn), tail_offsets=_ptr(to), tail_nodes=_ptr(tn),
+        exhausted=_ptr(exhausted), ticket=_ptr(ticket))
+    _lib.check(lib.rgcn_link_batch_ex(C.byref(a), _stream(ph.device)), "rgcn_link_batch_ex")
     return out
 
 

@@ -115,6 +115,19 @@ class KnownTriples:
                                      self.num_nodes, 1)
         return self._any
 
+    def bernoulli_head_prob(self) -> torch.Tensor:
+        """float32 [num_relations]: tph / (tph + hpt) per relation, the head-replacement probability of Wang et al.
+        2014 (``NegativeSampler(head_prob=...)``).  tph = mean number of tails per (head, relation), hpt = mean number of
+        heads per (tail, relation); 1/2 for a relation without triples."""
+        R = self.num_relations
+        rel = self.keys % R
+        n = torch.bincount(rel, minlength=R).to(torch.float64)
+        n_heads = torch.bincount(torch.unique_consecutive(self.keys) % R, minlength=R).to(torch.float64)
+        n_tails = torch.bincount(torch.unique(self.tails.to(torch.int64) * R + rel) % R, minlength=R).to(torch.float64)
+        tph, hpt = n / n_heads.clamp(min=1), n / n_tails.clamp(min=1)
+        p = torch.where(n > 0, tph / (tph + hpt).clamp(min=1e-300), torch.full_like(n, 0.5))
+        return p.to(torch.float32)
+
     def _on_candidates(self, candidates: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
         """(keys, positions) with the tails mapped to positions in ``candidates`` (non-candidates dropped, positions
         ascending per key); cached for the last candidates tensor."""
