@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define RGCN_B200_ABI_VERSION 7
+#define RGCN_B200_ABI_VERSION 8
 
 enum {
   RGCN_OK = 0,
@@ -342,6 +342,10 @@ typedef struct rgcn_layer_fwd_args {
    * untouched.  rows / slot as built by rgcn_rows_list_build; a row listed twice is computed once (later duplicate
    * positions of A are zero rows). */
   const int64_t* rows; int64_t n_list; const int32_t* slot;
+  /* Row of the LAYER'S output that local row 0 is, for the fused dropout's element index only (0 on one GPU).  A
+   * destination-range shard passes the global id of its first node, so node v draws the same keep mask on every shard
+   * count; without it every shard would repeat the mask of the first shard's rows.  Needs w_planes when dropout_p > 0. */
+  int64_t dropout_row0;
 } rgcn_layer_fwd_args;
 
 typedef struct rgcn_layer_bwd_args {

@@ -12,7 +12,7 @@ import threading
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "librgcn_b200.so")
 
-ABI_VERSION = 7          # RGCN_B200_ABI_VERSION of include/rgcn_b200.h
+ABI_VERSION = 8          # RGCN_B200_ABI_VERSION of include/rgcn_b200.h
 
 _lock = threading.Lock()
 _lib = None
@@ -43,7 +43,7 @@ class LayerFwdArgs(C.Structure):
                 ("agg_workspace", p), ("agg_workspace_bytes", sz), ("gemm_workspace", p), ("gemm_workspace_bytes", sz),
                 ("w_planes", p), ("w_planes_bytes", sz), ("pipeline", i32),
                 ("x_bf16", p), ("ld_x_bf16", i64), ("out_bf16", p), ("ld_out_bf16", i64),
-                ("rows", p), ("n_list", i64), ("slot", p)]
+                ("rows", p), ("n_list", i64), ("slot", p), ("dropout_row0", i64)]
 
 
 class MaskedPlanesOut(C.Structure):

@@ -45,9 +45,10 @@ class _RGCNLayerFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x_src, x_root, W, root, bias, graph: RelGraph, relu: bool, mode: str, drop=None, in_mask_scale=None,
-                listed=None):
+                listed=None, dropout_row0: int = 0):
         """x_src [n_src, d_in]: rows the edges gather from; x_root [n_dst, d_in]: the rows being updated (self-loop
-        term).  On one GPU they are the same tensor; on a destination-range shard x_src is the all-gathered matrix."""
+        term).  On one GPU they are the same tensor; on a destination-range shard x_src is the all-gathered matrix.
+        ``dropout_row0``: global node id of row 0 of x_root (a shard's first node), which keys the dropout mask."""
         R, d_in, d_out = W.shape
         shared = x_src.data_ptr() == x_root.data_ptr() and x_src.shape == x_root.shape
         x_src = x_src.contiguous()
@@ -69,8 +70,10 @@ class _RGCNLayerFn(torch.autograd.Function):
         # them alone; the planes come back compact, in list order — what the row-sparse backward wants
         ctx.listed = listed if (listed is not None and shared and p_drop == 0.0 and not want16) else None
         rows_l, slot_l = ctx.listed if ctx.listed is not None else (None, None)
+        # the row offset keys the dropout mask and nothing else: handed on only where it changes the result
+        row0 = {"dropout_row0": dropout_row0} if (p_drop > 0.0 and dropout_row0) else {}
         res = ops.layer_fwd(graph, x_src, x_root, W.reshape(R * d_in, d_out), root, bias, relu, mode, p_drop, seed, ctr,
-                            x_bf16=x16, want_out_bf16=want16, rows=rows_l, slot=slot_l)
+                            x_bf16=x16, want_out_bf16=want16, rows=rows_l, slot=slot_l, **row0)
         out, A, wp = res[:3]
         if ctx.listed is not None:
             rowsparse.mark_listed_output(out)
@@ -130,7 +133,7 @@ class _RGCNLayerFn(torch.autograd.Function):
                 gx_src = gx if need_src else None             # full-length partial, reduced by the caller
                 gx_root = gA[:, K1:]
         gW = gWf.view(R, d_in, d_out) if gWf is not None else None
-        return gx_src, gx_root, gW, groot, gb, None, None, None, None, None, None
+        return gx_src, gx_root, gW, groot, gb, None, None, None, None, None, None, None
 
 
 class _RGCNBasisLayerFn(torch.autograd.Function):

@@ -73,6 +73,7 @@ struct FusedParams {
   float* out; int64_t ldo;
   __nv_bfloat16* out16; int64_t ldo16;
   uint32_t drop_thresh; float drop_scale; uint32_t drop_seed; const unsigned long long* drop_ctr;
+  int64_t drop_row0;                          // layer-output row of local row 0 (a shard's first node): dropout index
   float* peer_out[FL_MAXPEERS]; int32_t n_peer; int64_t peer_row0; int64_t peer_ld;
 };
 
@@ -234,7 +235,7 @@ fused_layer_fwd_kernel(const __grid_constant__ CUtensorMap tm_b_hi, const __grid
           if (p.relu) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
           if (p.drop_thresh) {
             // the same hash of the GLOBAL element index as the unfused epilogue (transform.cu): identical masks
-            const uint64_t e0 = (uint64_t)row * (uint64_t)p.N + (uint64_t)col;
+            const uint64_t e0 = (uint64_t)(row + p.drop_row0) * (uint64_t)p.N + (uint64_t)col;
             const uint32_t bk = drop_block_key(drop_key, e0), e32 = (uint32_t)e0;
             const uint32_t h0 = pcg_hash(e32 ^ bk), h1 = pcg_hash((e32 + 2) ^ bk);
             v.x = (h0 & 0xffffu) >= p.drop_thresh ? v.x * p.drop_scale : 0.f;
@@ -613,7 +614,7 @@ int fused_layer_fwd_launch(const rgcn_layer_fwd_args* a, cudaStream_t st) {
     const double th = (double)a->dropout_p * 65536.0 + 0.5;
     p.drop_thresh = th >= 65535.0 ? 65535u : (th < 1.0 ? 1u : (uint32_t)th);
     p.drop_scale = 1.f / (1.f - a->dropout_p);
-    p.drop_seed = a->dropout_seed; p.drop_ctr = a->dropout_counter;
+    p.drop_seed = a->dropout_seed; p.drop_ctr = a->dropout_counter; p.drop_row0 = a->dropout_row0;
   }
   p.n_peer = a->n_peer; p.peer_row0 = a->peer_row0; p.peer_ld = a->peer_ld;
   for (int q = 0; q < a->n_peer; ++q) p.peer_out[q] = a->peer_out_host[q];

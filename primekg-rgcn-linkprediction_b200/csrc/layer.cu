@@ -136,6 +136,8 @@ extern "C" int rgcn_layer_fwd(const rgcn_layer_fwd_args* a, rgcn_stream_t stream
   const int out_mode = a->mode == 0 ? 2 : 1;
   RGCN_CHECK_ARG(a->mode == 0 || a->mode == 1, "layer_fwd: mode must be 0 (fp32) or 1 (bf16)");
   RGCN_CHECK_ARG(a->A_hi && (a->mode == 1 || a->A_lo) && a->lda >= K1 + K2, "layer_fwd: operand planes missing or too narrow");
+  RGCN_CHECK_ARG(a->dropout_row0 >= 0 && (a->dropout_row0 == 0 || a->dropout_p == 0.f || a->w_planes),
+                 "layer_fwd: dropout_row0 must be >= 0 and needs w_planes with dropout");
   if (!a->w_planes) {
     // the row walk also appends x_root[i] as the last block of row i: the operand [H | X] in one kernel
     int rc = rgcn_aggregate_fwd(a->csr, a->x_src, a->ld_x_src, a->d_in, nullptr, 0, a->A_hi, a->mode == 0 ? a->A_lo : nullptr,
@@ -185,7 +187,7 @@ extern "C" int rgcn_layer_fwd(const rgcn_layer_fwd_args* a, rgcn_stream_t stream
     const char* lo = A_lo ? (const char*)A_lo + (size_t)r0 * a->lda * 2 : nullptr;
     void* o16 = a->out_bf16 ? (void*)((char*)a->out_bf16 + (size_t)r0 * a->ld_out_bf16 * 2) : nullptr;
     return rgcn_transform_fwd_w(hi, lo, a->lda, K, a->w_planes, a->bias, a->relu, r1 - r0, a->d_out, a->out + r0 * a->ldo,
-                                a->ldo, a->mode, a->dropout_p, a->dropout_seed, a->dropout_counter, r0, a->peer_out_host,
+                                a->ldo, a->mode, a->dropout_p, a->dropout_seed, a->dropout_counter, a->dropout_row0 + r0, a->peer_out_host,
                                 a->n_peer, a->peer_row0 + r0, a->peer_ld, o16, a->ld_out_bf16, s);
   };
   // bf16-transform mode with a bf16 copy of the input: the walk gathers the copy

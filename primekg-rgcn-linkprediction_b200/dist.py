@@ -176,8 +176,11 @@ class PartitionedRGCN(nn.Module):
             W = AllReduceGrad.apply(conv.relation_weights())
             root, bias = AllReduceGrad.apply(conv.root), AllReduceGrad.apply(conv.bias)
             p = self.dropout.p if (self.training and li != last) else 0.0
-            drop = conv.dropout_state(p, x.device) if (0.0 < p < 1.0 and x.is_cuda) else None
-            x = _RGCNLayerFn.apply(x_full, x, W, root, bias, self.graph, li != last, conv.mode or default_mode(), drop)
+            drop = conv.dropout_state(p, x.device) if 0.0 < p < 1.0 else None
+            # the mask is keyed by global node id, as on one GPU (padding rows share ids with the next shard's first rows:
+            # harmless, no edge and no decoder reads a padding row)
+            x = _RGCNLayerFn.apply(x_full, x, W, root, bias, self.graph, li != last, conv.mode or default_mode(), drop,
+                                   None, None, self.plan.bounds[self.rank])
             if li != last and p > 0.0 and drop is None:
                 x = self.dropout(x)
         return x

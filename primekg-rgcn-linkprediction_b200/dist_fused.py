@@ -64,6 +64,7 @@ class _Exchange:
         self.n_total = plan.world * plan.max_n
         self.max_n = plan.max_n
         self.row0 = rank * plan.max_n
+        self.node0 = plan.bounds[rank]                      # global id of this shard's first node
         self.half = self.n_total * max(dims)               # floats per half
         self.half = (self.half + 63) // 64 * 64
         # features: two halves that alternate between the layers + a DEDICATED region for the encoder's output, so the
@@ -135,9 +136,11 @@ class _FusedEncoderFn(torch.autograd.Function):
             # aggregate -> planes -> transform whose epilogue also stores every tile into all ranks' next buffer
             rows_l, slot_l = listed[:2] if (last and listed is not None) else (None, None)
             push_after = rows_l is None and push_after_transform()
+            # the dropout mask is keyed by global node id (ex.node0), as on one GPU; padding rows share ids with the next
+            # shard's first rows, which is harmless: no edge and no decoder reads a padding row
             out, A, wp = ops.layer_fwd(graph, x_full, x_full[row0:row0 + n], W.reshape(K1, d_out), root, bias, not last, mode,
                                        p_drop, seed, ctr, peer_out=None if push_after else ex.x_ptrs(l + 1), peer_row0=row0,
-                                       peer_ld=d_out, rows=rows_l, slot=slot_l)
+                                       peer_ld=d_out, rows=rows_l, slot=slot_l, dropout_row0=ex.node0)
             if push_after:
                 # all-gather as a separate push of whole rows (512-byte bursts per warp) instead of the epilogue's 64-byte
                 # pieces: no overlap with the MMA main loop, but a far better NVLink packet mix

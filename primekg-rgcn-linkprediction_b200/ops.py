@@ -525,7 +525,7 @@ def layer_fwd(g: RelGraph, x_src: torch.Tensor, x_root: torch.Tensor, W2d: torch
               bias: torch.Tensor, relu: bool, mode: str, dropout_p: float = 0.0, dropout_seed: int = 0,
               dropout_ctr: Optional[torch.Tensor] = None, peer_out=None, peer_row0: int = 0, peer_ld: int = 0,
               pipeline: int = 0, x_bf16: Optional[torch.Tensor] = None, want_out_bf16: bool = False,
-              rows: Optional[torch.Tensor] = None, slot: Optional[torch.Tensor] = None):
+              rows: Optional[torch.Tensor] = None, slot: Optional[torch.Tensor] = None, dropout_row0: int = 0):
     """aggregate -> operand planes -> tensor-core transform of one layer in ONE C call (``rgcn_layer_fwd``).
     bf16 mode: ``x_bf16`` = a bf16 copy of x (the walk gathers it: half the bytes); ``want_out_bf16``: also return the
     layer output rounded to bf16 as a fourth result (the next layer's ``x_bf16``).
@@ -535,7 +535,9 @@ def layer_fwd(g: RelGraph, x_src: torch.Tensor, x_root: torch.Tensor, W2d: torch
     not: measured slower; RGCN_PIPELINE=1 opts in), 1 = never, 2 = always.
     ``rows`` (int64 device list from ``rows_list_build``, with its ``slot`` map): the LISTED-ROWS form — only these rows of
     the output are computed (``out`` is uninitialised elsewhere) and the returned planes are compact
-    [rows_compact_size(len(rows)), K] in list order; pass them to ``layer_bwd(..., rows=, slot=, a_compact=True)``."""
+    [rows_compact_size(len(rows)), K] in list order; pass them to ``layer_bwd(..., rows=, slot=, a_compact=True)``.
+    ``dropout_row0``: the layer-output row that row 0 of ``out`` is, for the dropout mask only — a destination-range
+    shard passes its first node's global id, so every node draws the mask it draws on one GPU."""
     lib = _lib.load()
     x_src = _f32c(x_src, "x")
     x_root = x_src if x_root is x_src else _f32c(x_root, "x_root")
@@ -580,7 +582,7 @@ def layer_fwd(g: RelGraph, x_src: torch.Tensor, x_root: torch.Tensor, W2d: torch
         int(peer_row0), int(peer_ld), _dp(aws), 0 if aws is None else aws.numel() * 4, gws.data_ptr(), gws.numel(),
         _dp(wp), 0 if wp is None else wp.numel(), int(pipeline),
         _dp(x_bf16), 0 if x_bf16 is None else x_bf16.stride(0), _dp(out16), 0 if out16 is None else out16.stride(0),
-        _dp(rows), rows.numel() if listed else 0, _dp(slot) if listed else None)
+        _dp(rows), rows.numel() if listed else 0, _dp(slot) if listed else None, int(dropout_row0))
     _lib.check(lib.rgcn_layer_fwd(C.byref(args), _stream(dev)), "rgcn_layer_fwd")
     if want_out_bf16:
         return out, A, wp, out16

@@ -64,7 +64,8 @@ def aggregate_bwd(g, gH, d, init=None):
 
 
 def layer_fwd(g, x_src, x_root, W2d, root, bias, relu, mode, dropout_p=0.0, dropout_seed=0, dropout_ctr=None,
-              peer_out=None, peer_row0=0, peer_ld=0, pipeline=0, x_bf16=None, want_out_bf16=False, rows=None, slot=None):
+              peer_out=None, peer_row0=0, peer_ld=0, pipeline=0, x_bf16=None, want_out_bf16=False, rows=None, slot=None,
+              dropout_row0=0):
     assert not peer_out and not want_out_bf16 and rows is None          # (the listed-rows forward needs CUDA index tensors)
     d_in = x_src.size(1)
     K1 = g.R * d_in
@@ -73,9 +74,14 @@ def layer_fwd(g, x_src, x_root, W2d, root, bias, relu, mode, dropout_p=0.0, drop
     split_planes(x_root.detach(), A, col0=K1)
     out = transform_fwd(A, K1, d_in, W2d, root, bias, relu, mode)
     if dropout_p > 0.0:
-        # the fused ReLU + dropout epilogue: zero with probability p, the rest times 1 / (1 - p); the backward needs no
-        # mask tensor (the output is zero exactly where ReLU or dropout killed the element)
-        out = out * torch.bernoulli(torch.full_like(out, 1.0 - dropout_p)) / (1.0 - dropout_p)
+        # the fused ReLU + dropout epilogue with the kernels' counter-based mask (the counter is advanced before the
+        # transform reads it), keyed by the global row dropout_row0 + i; the backward needs no mask tensor (the output is
+        # zero exactly where ReLU or dropout killed the element)
+        from test_gpu_gemm_conformance import drop_keep, drop_scale
+        dropout_ctr += 1
+        keep = drop_keep(out.size(0), int(dropout_row0), out.size(1), dropout_p, int(dropout_seed), int(dropout_ctr),
+                         device=out.device)
+        out = torch.where(keep, out * drop_scale(dropout_p), 0.0)
     return out, A, None
 
 

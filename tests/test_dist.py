@@ -2,6 +2,7 @@
 reduce-scatter / all-reduce with autograd, layer wiring.  The kernels are replaced by CPU stand-ins
 (tests/cpu_ops_emulation.py); the 2-rank result must equal the single-process oracle on the unpartitioned graph."""
 import os
+import socket
 import sys
 
 import pytest
@@ -12,7 +13,18 @@ import torch.multiprocessing as mp
 from conftest import ROOT
 
 
-def _worker(rank, world, port, ret):
+class _HashDropout(torch.nn.Module):
+    """The fused dropout's keep masks (one per ReLU layer, in call order) applied as the reference's nn.Dropout."""
+
+    def __init__(self, keeps, scale):
+        super().__init__()
+        self.keeps, self.scale = list(keeps), scale
+
+    def forward(self, x):
+        return torch.where(self.keeps.pop(0), x * self.scale, 0.0)
+
+
+def _worker(rank, world, port, ret, dropout):
     sys.path.insert(0, ROOT)
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     os.environ["MASTER_ADDR"] = "127.0.0.1"
@@ -33,9 +45,11 @@ def _worker(rank, world, port, ret):
         et = kg.edge_type
         plan = D.plan_partition(ei[1], N, world)
         assert plan.bounds[0] == 0 and plan.bounds[-1] == N and sorted(plan.bounds) == plan.bounds
-        enc = D.PartitionedRGCN(plan, rank, R, d_e, H, dropout=0.0, num_layers=3, seed=9)
+        assert plan.bounds[1] > 0
+        enc = D.PartitionedRGCN(plan, rank, R, d_e, H, dropout=dropout, num_layers=3, seed=9)
         src, dst, rel = D.local_edges(ei, et, plan, rank)
         enc.set_graph(emu.CpuGraph(src, dst, rel, plan.max_n, world * plan.max_n, R))
+        torch.manual_seed(7)                                   # the same dropout seeds on every rank, as in the models
         out = enc()                                            # [max_n, H], this rank's rows
         n_loc = plan.size(rank)
         g = torch.Generator().manual_seed(100)
@@ -47,6 +61,12 @@ def _worker(rank, world, port, ret):
         dist.all_gather(shards, enc.node_embeddings.detach())
         table = torch.cat([shards[p][: plan.size(p)] for p in range(world)], 0)
         ref = O.EncoderRef(N, R, d_e, H, 0.0, None, num_layers=3)
+        if dropout > 0.0:
+            # one mask per ReLU layer over ALL nodes, keyed by global node id: the shards must draw these very masks
+            from test_gpu_gemm_conformance import drop_keep, drop_scale
+            keeps = [drop_keep(N, 0, H, dropout, conv._drop_seed, int(conv._drop_ctr), device="cpu")
+                     for conv in enc.convs[:-1]]
+            ref.dropout = _HashDropout(keeps, drop_scale(dropout))
         with torch.no_grad():
             ref.node_embeddings.weight.copy_(table)
             for mine, theirs in zip(enc.convs, [ref.conv1, ref.conv2] + list(ref.extra)):
@@ -74,11 +94,23 @@ def _worker(rank, world, port, ret):
 
 
 def test_partitioned_encoder_two_ranks_equals_single_process():
+    _run_two_ranks(0.0)
+
+
+def test_partitioned_encoder_two_ranks_dropout_masks_equal_single_process():
+    """The fused dropout mask is keyed by global node id, so the 2-rank encoder draws the single-process masks."""
+    _run_two_ranks(0.5)
+
+
+def _run_two_ranks(dropout):
     world = 2
     mgr = mp.Manager()
     ret = mgr.dict()
-    port = 29500 + os.getpid() % 2000
-    mp.spawn(_worker, args=(world, port, ret), nprocs=world, join=True)
+    s = socket.socket()
+    s.bind(("127.0.0.1", 0))
+    port = s.getsockname()[1]
+    s.close()
+    mp.spawn(_worker, args=(world, port, ret, dropout), nprocs=world, join=True)
     for r in range(world):
         assert ret.get(r) == "ok", ret.get(r)
 

@@ -75,13 +75,15 @@ def test_fused_partition_matches_single_gpu(pg, monkeypatch, layers, dropout, li
     s = model(heads, tails, rels)
     F.binary_cross_entropy_with_logits(s, labels).backward()
     assert all(p.grad is not None and torch.isfinite(p.grad).all() for p in model.parameters())
-    if dropout > 0:
-        return                                   # masks differ from the reference model's; finiteness is the check
-    ref = pkg.DrugDiseaseModel(N, R, d_e, H, dropout=0.0, decoder_dropout=0.0, num_layers=layers).to(DEV)
+    ref = pkg.DrugDiseaseModel(N, R, d_e, H, dropout=dropout, decoder_dropout=0.0, num_layers=layers).to(DEV)
     with torch.no_grad():
         ref.encoder.node_embeddings.weight.copy_(model.encoder.node_embeddings[:N])
         for mine, theirs in zip(model.encoder.convs, ref.encoder._layers()):
             theirs.weight.copy_(mine.weight); theirs.root.copy_(mine.root); theirs.bias.copy_(mine.bias)
+            if mine._drop_ctr is not None:
+                # the same dropout stream, from the counter value before the forward above: the masks are keyed by
+                # global node id, so the shard draws the single-GPU model's masks
+                theirs._drop_seed, theirs._drop_ctr = mine._drop_seed, mine._drop_ctr - 1
         ref.decoder.relation_embeddings.weight.copy_(model.decoder.relation_embeddings.weight)
     ref.train()
     rs = ref(ei, et, heads, tails, rels)

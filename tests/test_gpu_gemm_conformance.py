@@ -234,11 +234,11 @@ def drop_scale(p):
     return float(np.float32(1.0) / (np.float32(1.0) - np.float32(p)))
 
 
-def drop_keep(rows, row_offset, N, p, seed, c):
+def drop_keep(rows, row_offset, N, p, seed, c, device=DEV):
     """bool [rows, N]: element (row, col) of the call that read counter value c survives the fused dropout."""
     key = (_pcg((seed & M32) ^ (c & M32)) + (c >> 32)) & M32
-    r = torch.arange(rows, device=DEV, dtype=torch.int64)[:, None] + row_offset
-    col = torch.arange(N, device=DEV, dtype=torch.int64)[None, :]
+    r = torch.arange(rows, device=device, dtype=torch.int64)[:, None] + row_offset
+    col = torch.arange(N, device=device, dtype=torch.int64)[None, :]
     e4 = r * N + (col & ~3)                              # first element of the aligned group of four
     bk = _pcg((key + (e4 >> 32) * 0x9E3779B9) & M32)
     lo = e4 & M32

@@ -26,7 +26,7 @@ def test_library_exports_every_header_symbol(lib_built):
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/rgcn_b200.h but not exported"
     assert set(names) == set(_lib.PROTOTYPES), "ctypes prototypes and header disagree"
-    assert _lib.load().rgcn_abi_version() == _lib.ABI_VERSION == 7
+    assert _lib.load().rgcn_abi_version() == _lib.ABI_VERSION == 8
 
 
 def test_library_argument_errors_without_gpu(lib_built):
@@ -60,16 +60,18 @@ def test_arg_structs_match_header_layout(tmp_path):
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     src = tmp_path / "sz.c"
     src.write_text('#include <stdio.h>\n#include <stddef.h>\n#include "rgcn_b200.h"\n'
-                   'int main(void){printf("%zu %zu %zu %zu %zu %zu %zu %zu %zu\\n", sizeof(rgcn_csr_t), sizeof(rgcn_layer_fwd_args),'
+                   'int main(void){printf("%zu %zu %zu %zu %zu %zu %zu %zu %zu %zu\\n", sizeof(rgcn_csr_t), sizeof(rgcn_layer_fwd_args),'
                    'sizeof(rgcn_layer_bwd_args), offsetof(rgcn_layer_bwd_args, rows), offsetof(rgcn_layer_bwd_args, ldac),'
                    'offsetof(rgcn_layer_fwd_args, gemm_workspace_bytes), offsetof(rgcn_layer_fwd_args, pipeline),'
-                   'offsetof(rgcn_layer_bwd_args, w_planes), offsetof(rgcn_csr_t, order_chunk_rows));return 0;}\n')
+                   'offsetof(rgcn_layer_bwd_args, w_planes), offsetof(rgcn_csr_t, order_chunk_rows),'
+                   'offsetof(rgcn_layer_fwd_args, dropout_row0));return 0;}\n')
     exe = tmp_path / "sz"
     subprocess.run(["gcc", "-I", os.path.join(root, "include"), str(src), "-o", str(exe)], check=True)
     got = [int(t) for t in subprocess.run([str(exe)], check=True, capture_output=True, text=True).stdout.split()]
     want = [ctypes.sizeof(_lib.CsrStruct), ctypes.sizeof(_lib.LayerFwdArgs), ctypes.sizeof(_lib.LayerBwdArgs),
             _lib.LayerBwdArgs.rows.offset, _lib.LayerBwdArgs.ldac.offset, _lib.LayerFwdArgs.gemm_workspace_bytes.offset,
-            _lib.LayerFwdArgs.pipeline.offset, _lib.LayerBwdArgs.w_planes.offset, _lib.CsrStruct.order_chunk_rows.offset]
+            _lib.LayerFwdArgs.pipeline.offset, _lib.LayerBwdArgs.w_planes.offset, _lib.CsrStruct.order_chunk_rows.offset,
+            _lib.LayerFwdArgs.dropout_row0.offset]
     assert got == want
 
 

@@ -13,7 +13,7 @@ def test_excluding_entry_points_are_exported(lib_built):
     lib = ctypes.CDLL(_lib.LIB_PATH)
     for n in NEW_SYMBOLS:
         assert hasattr(lib, n) and n in _lib.PROTOTYPES
-    assert _lib.load().rgcn_abi_version() == 7
+    assert _lib.load().rgcn_abi_version() == _lib.ABI_VERSION == 8
 
 
 def _fake(addr=4096):

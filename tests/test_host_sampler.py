@@ -16,7 +16,7 @@ def test_sampler_entry_point_is_exported(lib_built):
     from primekg_rgcn_linkprediction_b200 import _lib
     lib = ctypes.CDLL(_lib.LIB_PATH)
     assert hasattr(lib, "rgcn_link_batch_ex") and "rgcn_link_batch_ex" in _lib.PROTOTYPES
-    assert _lib.load().rgcn_abi_version() == 7
+    assert _lib.load().rgcn_abi_version() == _lib.ABI_VERSION == 8
 
 
 def test_link_batch_args_match_header_layout(tmp_path):
