@@ -299,6 +299,18 @@ int rgcn_basis_combine_bwd(const float* comp, const float* V, const float* gW, i
                            float* g_V, float* g_comp, rgcn_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Block-diagonal relation weights, RGCNConv(num_blocks = nb) (PyG's `weight [R, nb, in/nb, out/nb]`):
+ *   rgcn_block_diag_expand : W [R, nb*bi, nb*bo] = blockdiag(blocks[r, 0], .., blocks[r, nb-1]) per relation; every
+ *                            element is written (explicit zeros off the blocks)
+ *   rgcn_block_diag_gather : g_blocks[r, k, c, d] = gW[r, k*bi + c, k*bo + d]   (the compact gradient; copies only)
+ * blocks / g_blocks [R, nb, bi, bo], W / gW [R, nb*bi, nb*bo], row-major fp32, 16-byte aligned; allocate nothing.
+ * ------------------------------------------------------------------------------------------ */
+int rgcn_block_diag_expand(const float* blocks, int32_t R, int32_t nb, int32_t bi, int32_t bo, float* W,
+                           rgcn_stream_t stream);
+int rgcn_block_diag_gather(const float* gW, int32_t R, int32_t nb, int32_t bi, int32_t bo, float* g_blocks,
+                           rgcn_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * One layer per call.  rgcn_layer_fwd = rgcn_aggregate_fwd (H into the first R blocks of the operand planes, x_root
  * appended as the last block by the same kernel) + rgcn_transform_fwd: everything `RGCNConv.forward` does at
  * src/models/rgcn.py:123 / :128 (+ the ReLU / dropout of :124-125 when asked).  rgcn_layer_bwd = rgcn_split_planes

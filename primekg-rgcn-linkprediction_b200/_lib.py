@@ -129,6 +129,8 @@ PROTOTYPES = {
                                      p, i32, i64, i64, p, sz, p]),
     "rgcn_basis_combine": (C.c_int, [p, p, i32, i32, i64, p, p]),
     "rgcn_basis_combine_bwd": (C.c_int, [p, p, p, i32, i32, i64, p, p, p]),
+    "rgcn_block_diag_expand": (C.c_int, [p, i32, i32, i32, i32, p, p]),
+    "rgcn_block_diag_gather": (C.c_int, [p, i32, i32, i32, i32, p, p]),
     "rgcn_layer_fwd": (C.c_int, [C.POINTER(LayerFwdArgs), p]),
     "rgcn_layer_bwd": (C.c_int, [C.POINTER(LayerBwdArgs), p]),
     "rgcn_p2p_pull_rows": (C.c_int, [p, i32, i64, i64, p, i64, i64, i32, p, i64, p]),

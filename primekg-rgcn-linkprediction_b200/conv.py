@@ -83,6 +83,7 @@ class _RGCNLayerFn(torch.autograd.Function):
             rowsparse.announce_bf16(out, res[3])
         ctx.graph, ctx.relu, ctx.mode, ctx.shared, ctx.p_drop = graph, relu, mode, shared, p_drop
         ctx.w_planes = wp               # the weights as bf16 planes (converted once): the backward's dgrad reads them
+        ctx.scratch_w = ops.is_grad_scratch(W)     # block-diagonal W: its dense gradient is scratch, not a parameter's
         # in_mask_scale: x is the fused ReLU (+ dropout) output of the layer upstream, whose backward will want this
         # layer's input gradient masked by x > 0 and scaled — the backward walk can write that directly (rowsparse.py)
         ctx.in_mask_scale = in_mask_scale if (shared and in_mask_scale is not None) else None
@@ -102,6 +103,7 @@ class _RGCNLayerFn(torch.autograd.Function):
         # gO zero outside a short, announced row list (the decoder's backward, rowsparse.py): compact backward
         rows = slot = None
         a_compact = False
+        scratch = {"scratch_w": True} if ctx.scratch_w else {}     # handed on only where it changes the result
         if ctx.listed is not None:
             # the forward computed the listed rows only (the others were never defined, nothing may flow into them): the
             # compaction of gO runs over the forward's own list, and its compact planes are the weight gradient's operand
@@ -120,7 +122,7 @@ class _RGCNLayerFn(torch.autograd.Function):
         res = ops.layer_bwd(
             graph, gO.contiguous(), out, mask_scale, (A_hi, A_lo), W.reshape(K1, d_out), root, d_in, mode,
             need_x=need_x, add_root_term=ctx.shared, need_w=need_w_any, need_b=need_w_any, rows=rows, g_ready=g_ready,
-            next_mask=next_mask, slot=slot, w_planes=ctx.w_planes, a_compact=a_compact,
+            next_mask=next_mask, slot=slot, w_planes=ctx.w_planes, a_compact=a_compact, **scratch,
             gx_out=ops.param_grad(graph.n_src, d_in, device=gO.device) if (need_x and ctx.x_is_param) else None)
         gx, gA, gWf, groot, gb = res[:5]
         if next_mask is not None:
@@ -215,18 +217,31 @@ def _glorot_(t: Optional[torch.Tensor]) -> None:
 
 
 class RGCNConv(nn.Module):
+    """``num_bases`` = B: W_r = sum_b comp[r, b] weight[b].  ``num_blocks`` = nb: W_r = blockdiag(weight[r, 0], ..,
+    weight[r, nb - 1]) with ``weight`` [R, nb, in / nb, out / nb] and no ``comp`` (PyG's two regularisers; at most one).
+    Both are materialised as the dense [R, in, out] W_r that the layer kernels consume (``relation_weights``)."""
+
     def __init__(self, in_channels: int, out_channels: int, num_relations: int, num_bases: Optional[int] = None,
-                 mode: Optional[str] = None):
+                 mode: Optional[str] = None, num_blocks: Optional[int] = None):
         super().__init__()
+        if num_bases is not None and num_blocks is not None:
+            raise ValueError("can not apply both basis-decomposition and block-diagonal-decomposition at the same time")
+        if num_blocks is not None and (num_blocks < 1 or in_channels % num_blocks or out_channels % num_blocks):
+            raise ValueError(f"num_blocks={num_blocks} must divide in_channels={in_channels} and "
+                             f"out_channels={out_channels}")
         if in_channels % 4 or out_channels % 4:
             raise ValueError("the sm_100a kernels need channel counts that are multiples of 4")
         self.in_channels, self.out_channels = in_channels, out_channels
-        self.num_relations, self.num_bases = num_relations, num_bases
+        self.num_relations, self.num_bases, self.num_blocks = num_relations, num_bases, num_blocks
         self.mode = mode
         self._drop_ctr, self._drop_seed = None, 0
         if num_bases is not None:
             self.weight = nn.Parameter(torch.empty(num_bases, in_channels, out_channels))
             self.comp = nn.Parameter(torch.empty(num_relations, num_bases))
+        elif num_blocks is not None:
+            self.weight = nn.Parameter(torch.empty(num_relations, num_blocks, in_channels // num_blocks,
+                                                   out_channels // num_blocks))
+            self.register_parameter("comp", None)
         else:
             self.weight = nn.Parameter(torch.empty(num_relations, in_channels, out_channels))
             self.register_parameter("comp", None)
@@ -242,7 +257,11 @@ class RGCNConv(nn.Module):
             self.bias.zero_()
 
     def relation_weights(self) -> torch.Tensor:
-        """[R, d_in, d_out]; with bases W_r = sum_b comp[r, b] V_b (differentiable)."""
+        """[R, d_in, d_out]; with bases W_r = sum_b comp[r, b] V_b, with blocks the block-diagonal W_r (differentiable)."""
+        if self.num_blocks is not None:
+            if not self.weight.is_cuda:
+                raise RuntimeError("block-diagonal RGCNConv needs CUDA tensors: there is no CPU implementation of this path")
+            return ops.block_diag_weights(self.weight)               # our kernels (csrc/basis.cu), forward and backward
         if self.comp is None:
             return self.weight
         B = self.weight.size(0)
@@ -303,4 +322,4 @@ class RGCNConv(nn.Module):
 
     def extra_repr(self) -> str:
         return (f"{self.in_channels}, {self.out_channels}, num_relations={self.num_relations}, "
-                f"num_bases={self.num_bases}")
+                f"num_bases={self.num_bases}" + (f", num_blocks={self.num_blocks}" if self.num_blocks is not None else ""))

@@ -80,6 +80,50 @@ __global__ void __launch_bounds__(256) comp_grad_kernel(const float* __restrict_
   }
 }
 
+// Block-diagonal relation weights (RGCNConv(num_blocks = nb), PyG's second regulariser, Schlichtkrull et al. 2018):
+// W_r = blockdiag(blocks[r, 0], .., blocks[r, nb - 1]),  W[r, k*bi + c, k*bo + d] = blocks[r, k, c, d], zero off the blocks.
+// The expanded W_r feeds the unchanged layer kernels; the backward copies the diagonal blocks of the dense gradient
+// back.  Pure copies (no arithmetic): bit-exact and deterministic.  VEC: 4 consecutive columns per thread (bo % 4 == 0,
+// so they never straddle a block).  One thread per output vector, 32-bit index arithmetic (the host caps the sizes).
+template <bool VEC>
+__global__ void __launch_bounds__(256) block_diag_expand_kernel(const float* __restrict__ blocks, int nb, int bi, int bo,
+                                                                float* __restrict__ W, unsigned n_vec) {
+  pdl_enter();
+  constexpr unsigned V = VEC ? 4 : 1;
+  const unsigned t = blockIdx.x * 256u + threadIdx.x;
+  if (t >= n_vec) return;
+  const unsigned d_in = (unsigned)nb * bi, cols = (unsigned)nb * bo / V;
+  const unsigned ri = t / cols, j = (t - ri * cols) * V;       // row r * d_in + i of W, first column
+  const unsigned r = ri / d_in, i = ri - r * d_in;
+  const unsigned k = i / bi;
+  const bool on = j >= k * bo && j < (k + 1) * bo;
+  const size_t src = ((size_t)(r * nb + k) * bi + (i - k * bi)) * bo + (j - k * bo);
+  if (VEC) {
+    reinterpret_cast<float4*>(W)[t] = on ? __ldg(reinterpret_cast<const float4*>(blocks + src)) : make_float4(0.f, 0.f, 0.f, 0.f);
+  } else {
+    W[t] = on ? __ldg(blocks + src) : 0.f;
+  }
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(256) block_diag_gather_kernel(const float* __restrict__ gW, int nb, int bi, int bo,
+                                                                float* __restrict__ g_blocks, unsigned n_vec) {
+  pdl_enter();
+  constexpr unsigned V = VEC ? 4 : 1;
+  const unsigned t = blockIdx.x * 256u + threadIdx.x;
+  if (t >= n_vec) return;
+  const unsigned cols = (unsigned)bo / V;
+  const unsigned rkc = t / cols, d = (t - rkc * cols) * V;    // (r * nb + k) * bi + c, column in the block
+  const unsigned rk = rkc / bi, c = rkc - rk * bi;
+  const unsigned r = rk / nb, k = rk - r * nb;
+  const size_t src = ((size_t)r * nb * bi + k * bi + c) * ((size_t)nb * bo) + k * bo + d;
+  if (VEC) {
+    reinterpret_cast<float4*>(g_blocks)[t] = __ldg(reinterpret_cast<const float4*>(gW + src));
+  } else {
+    g_blocks[t] = __ldg(gW + src);
+  }
+}
+
 }  // namespace rgcn
 
 using namespace rgcn;
@@ -118,5 +162,46 @@ extern "C" int rgcn_basis_combine_bwd(const float* comp, const float* V, const f
     RGCN_CUDA(launch_pdl(comp_grad_kernel, dim3((unsigned)R), dim3(256), 0, (cudaStream_t)stream, gW, V, (int)B, cols4, g_comp, (int)B));
     RGCN_LAUNCH_CHECK();
   }
+  return RGCN_OK;
+}
+
+static int check_block_diag(const char* who, const float* a, const float* b, int32_t R, int32_t nb, int32_t bi, int32_t bo) {
+  RGCN_CHECK_ARG(a && b && R >= 1 && nb >= 1 && bi >= 1 && bo >= 1, "%s: need non-null matrices and R, nb, bi, bo >= 1", who);
+  RGCN_CHECK_ARG((int64_t)nb * bi <= (1 << 20) && (int64_t)nb * bo <= (1 << 20) && R <= (1 << 20),
+                 "%s: in, out = nb * bi, nb * bo and R must be at most 2^20", who);
+  RGCN_CHECK_ARG((int64_t)R * nb * bi * nb * bo < ((int64_t)1 << 31), "%s: the dense W must have fewer than 2^31 elements", who);
+  RGCN_CHECK_ARG((((uintptr_t)a | (uintptr_t)b) & 15) == 0, "%s: matrices must be 16-byte aligned", who);
+  return RGCN_OK;
+}
+
+extern "C" int rgcn_block_diag_expand(const float* blocks, int32_t R, int32_t nb, int32_t bi, int32_t bo, float* W,
+                                      rgcn_stream_t stream) {
+  int rc = check_block_diag("block_diag_expand", blocks, W, R, nb, bi, bo);
+  if (rc) return rc;
+  const int64_t n = (int64_t)R * nb * bi * nb * bo;
+  if (bo % 4 == 0) {
+    RGCN_CUDA(launch_pdl(block_diag_expand_kernel<true>, dim3((unsigned)((n / 4 + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                         blocks, (int)nb, (int)bi, (int)bo, W, (unsigned)(n / 4)));
+  } else {
+    RGCN_CUDA(launch_pdl(block_diag_expand_kernel<false>, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                         blocks, (int)nb, (int)bi, (int)bo, W, (unsigned)n));
+  }
+  RGCN_LAUNCH_CHECK();
+  return RGCN_OK;
+}
+
+extern "C" int rgcn_block_diag_gather(const float* gW, int32_t R, int32_t nb, int32_t bi, int32_t bo, float* g_blocks,
+                                      rgcn_stream_t stream) {
+  int rc = check_block_diag("block_diag_gather", gW, g_blocks, R, nb, bi, bo);
+  if (rc) return rc;
+  const int64_t n = (int64_t)R * nb * bi * bo;
+  if (bo % 4 == 0) {
+    RGCN_CUDA(launch_pdl(block_diag_gather_kernel<true>, dim3((unsigned)((n / 4 + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                         gW, (int)nb, (int)bi, (int)bo, g_blocks, (unsigned)(n / 4)));
+  } else {
+    RGCN_CUDA(launch_pdl(block_diag_gather_kernel<false>, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+                         gW, (int)nb, (int)bi, (int)bo, g_blocks, (unsigned)n));
+  }
+  RGCN_LAUNCH_CHECK();
   return RGCN_OK;
 }

@@ -24,6 +24,7 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from .conv import RGCNConv, _RGCNLayerFn, default_mode
+from . import ops
 from .graph import RelGraph
 
 
@@ -137,15 +138,15 @@ class PartitionedRGCN(nn.Module):
 
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, num_bases: Optional[int] = None, num_layers: int = 2,
-                 seed: int = 42):
+                 seed: int = 42, num_blocks: Optional[int] = None):
         super().__init__()
         self.plan, self.rank, self.num_relations = plan, rank, num_relations
         self.n_local = plan.size(rank)
         g = torch.Generator().manual_seed(seed)
         dims = [embedding_dim] + [hidden_dim] * num_layers
-        self.convs = nn.ModuleList(RGCNConv(dims[i], dims[i + 1], num_relations, num_bases=num_bases)
-                                   for i in range(num_layers))
-        for conv in self.convs:                       # identical replicated weights on every rank
+        self.convs = nn.ModuleList(RGCNConv(dims[i], dims[i + 1], num_relations, num_bases=num_bases,
+                                            num_blocks=num_blocks) for i in range(num_layers))
+        for conv in self.convs:                       # identical replicated weights on every rank (glorot on the last two dims)
             for prm in (conv.weight, conv.comp, conv.root):
                 if prm is not None:
                     a = (6.0 / (prm.size(-2) + prm.size(-1))) ** 0.5
@@ -173,7 +174,10 @@ class PartitionedRGCN(nn.Module):
         last = len(self.convs) - 1
         for li, conv in enumerate(self.convs):
             x_full = AllGatherRows.apply(x)                                  # NCCL all-gather over NVLink
-            W = AllReduceGrad.apply(conv.relation_weights())
+            Wr = conv.relation_weights()
+            W = AllReduceGrad.apply(Wr)
+            if ops.is_grad_scratch(Wr):
+                W._rgcn_grad_scratch = True                                  # block-diagonal: dense gradient is scratch
             root, bias = AllReduceGrad.apply(conv.root), AllReduceGrad.apply(conv.bias)
             p = self.dropout.p if (self.training and li != last) else 0.0
             drop = conv.dropout_state(p, x.device) if 0.0 < p < 1.0 else None
@@ -200,12 +204,13 @@ class PartitionedModel(nn.Module):
 
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, decoder_dropout: float = 0.0,
-                 num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42):
+                 num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42,
+                 num_blocks: Optional[int] = None):
         super().__init__()
         from .modules import LinkPredictor
         self.plan = plan
         self.encoder = PartitionedRGCN(plan, rank, num_relations, embedding_dim, hidden_dim, dropout, num_bases,
-                                       num_layers, seed)
+                                       num_layers, seed, num_blocks=num_blocks)
         state = torch.random.get_rng_state()
         torch.manual_seed(seed + 12345)                       # identical decoder on every rank
         self.decoder = LinkPredictor(num_relations, hidden_dim, decoder_dropout)

@@ -153,6 +153,7 @@ class _FusedEncoderFn(torch.autograd.Function):
         ctx.listed = listed
         ctx.generation = ex.generation
         ctx.w_planes = wps
+        ctx.scratch_w = ops.is_grad_scratch(params[3 * (L - 1)])     # block-diagonal last layer (conv.py)
         ctx.p_drops = [d[0] if d is not None else 0.0 for d in drops]
         ctx.d0 = x0.size(1)
         ctx.save_for_backward(*saved, *[o for o in outs if o is not None])
@@ -222,7 +223,8 @@ class _FusedEncoderFn(torch.autograd.Function):
                 _, gA_c, gWf, groot, gb, slot = ops.layer_bwd(
                     graph, g_local, None, 1.0, (A_hi, A_lo), Wf, root, d_in, mode, need_x=True, add_root_term=False,
                     need_w=True, need_b=True, gx_out=ex.g_view(l, d_in), rows=sparse_rows, w_planes=ctx.w_planes[l],
-                    return_compact=True, slot=slot_fwd, a_compact=slot_fwd is not None)
+                    return_compact=True, slot=slot_fwd, a_compact=slot_fwd is not None,
+                    **({"scratch_w": True} if ctx.scratch_w else {}))
                 # root-term gradient of this rank's rows: the compact rows scattered back (unlisted rows read the zero row)
                 extra = gA_c[:, K1:].index_select(0, slot.long())
                 grads[3 * l: 3 * l + 3] = [gWf.view(R, d_in, d_out), groot, gb]
@@ -290,12 +292,13 @@ class FusedPartitionedModel(nn.Module):
 
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, decoder_dropout: float = 0.0,
-                 num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42):
+                 num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42,
+                 num_blocks: Optional[int] = None):
         super().__init__()
         from .modules import LinkPredictor
         self.plan = plan
         self.encoder = FusedPartitionedRGCN(plan, rank, num_relations, embedding_dim, hidden_dim, dropout, num_bases,
-                                            num_layers, seed)
+                                            num_layers, seed, num_blocks=num_blocks)
         state = torch.random.get_rng_state()
         torch.manual_seed(seed + 12345)                       # identical decoder on every rank
         self.decoder = LinkPredictor(num_relations, hidden_dim, decoder_dropout)

@@ -42,7 +42,8 @@ class DrugDiseaseRGCN(nn.Module):
     pattern of reference guide/MODEL_ARCHITECTURE.md:245-249; used by the 3-layer 10 M-node config)."""
 
     def __init__(self, num_nodes: int, num_relations: int, embedding_dim: int = 64, hidden_dim: int = 128,
-                 dropout: float = 0.5, num_bases: Optional[int] = None, num_layers: int = 2):
+                 dropout: float = 0.5, num_bases: Optional[int] = None, num_layers: int = 2,
+                 num_blocks: Optional[int] = None):
         super().__init__()
         self.num_nodes = num_nodes
         self.num_relations = num_relations
@@ -50,11 +51,12 @@ class DrugDiseaseRGCN(nn.Module):
         self.hidden_dim = hidden_dim
         # construction order = the reference's, so a seeded init draws the same random stream
         self.node_embeddings = nn.Embedding(num_nodes, embedding_dim)
-        self.conv1 = RGCNConv(embedding_dim, hidden_dim, num_relations, num_bases=num_bases)
-        self.conv2 = RGCNConv(hidden_dim, hidden_dim, num_relations, num_bases=num_bases)
+        dec = dict(num_bases=num_bases, num_blocks=num_blocks)
+        self.conv1 = RGCNConv(embedding_dim, hidden_dim, num_relations, **dec)
+        self.conv2 = RGCNConv(hidden_dim, hidden_dim, num_relations, **dec)
         if num_layers > 2:
             self.extra_convs = nn.ModuleList(
-                RGCNConv(hidden_dim, hidden_dim, num_relations, num_bases=num_bases) for _ in range(num_layers - 2))
+                RGCNConv(hidden_dim, hidden_dim, num_relations, **dec) for _ in range(num_layers - 2))
         self.dropout = nn.Dropout(dropout)
         self._eval_cache = None
         self._register_load_state_dict_pre_hook(self._drop_cache_on_load)
@@ -291,14 +293,14 @@ class DrugDiseaseModel(nn.Module):
 
     def __init__(self, num_nodes: int, num_relations: int, embedding_dim: int = 64, hidden_dim: int = 128,
                  dropout: float = 0.5, decoder_dropout: float = 0.0, num_bases: Optional[int] = None,
-                 num_layers: int = 2):
+                 num_layers: int = 2, num_blocks: Optional[int] = None):
         super().__init__()
         self.num_nodes = num_nodes
         self.num_relations = num_relations
         self.hidden_dim = hidden_dim
         self.encoder = DrugDiseaseRGCN(num_nodes=num_nodes, num_relations=num_relations,
                                        embedding_dim=embedding_dim, hidden_dim=hidden_dim, dropout=dropout,
-                                       num_bases=num_bases, num_layers=num_layers)
+                                       num_bases=num_bases, num_layers=num_layers, num_blocks=num_blocks)
         self.decoder = LinkPredictor(num_relations=num_relations, embedding_dim=hidden_dim, dropout=decoder_dropout)
 
     def forward(self, edge_index, edge_type, head_indices, tail_indices, relation_types) -> torch.Tensor:

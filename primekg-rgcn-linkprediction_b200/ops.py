@@ -593,7 +593,7 @@ def layer_bwd(g: RelGraph, gO: torch.Tensor, relu_mask: Optional[torch.Tensor], 
               root: torch.Tensor, d_in: int, mode: str, need_x: bool, add_root_term: bool, need_w: bool, need_b: bool,
               gx_out: Optional[torch.Tensor] = None, rows: Optional[torch.Tensor] = None, g_ready=None, next_mask=None,
               slot: Optional[torch.Tensor] = None, w_planes: Optional[torch.Tensor] = None, return_compact: bool = False,
-              a_compact: bool = False):
+              a_compact: bool = False, scratch_w: bool = False):
     """split(gO, mask) -> dgrad -> transposed gather -> wgrad of one layer in ONE C call (``rgcn_layer_bwd``).
     Returns (g_x | None, gA | None, gW2d | None, g_root | None, g_bias | None); ``gA[:, R*d_in:]`` is the root-term
     gradient (already inside g_x when ``add_root_term``).
@@ -605,7 +605,8 @@ def layer_bwd(g: RelGraph, gO: torch.Tensor, relu_mask: Optional[torch.Tensor], 
     ``a_compact`` (row-sparse form): ``planes`` are the compact planes of the listed-rows forward over this very list.
     ``g_ready`` = ((G_hi, G_lo | None), colsum [n, d_out]): this layer's masked output gradient as planes, already written
     by the downstream layer (skips the split pass).  ``next_mask`` = (mask [n_src, d_in], scale): also produce g_x masked
-    for the upstream layer; the result gains a sixth entry ((hi, lo | None), colsum)."""
+    for the upstream layer; the result gains a sixth entry ((hi, lo | None), colsum).
+    ``scratch_w``: the weight is an intermediate (``is_grad_scratch``), its gradient a plain tensor outside the arena."""
     lib = _lib.load()
     gO = _f32c(gO, "gO")
     if relu_mask is not None:
@@ -643,7 +644,9 @@ def layer_bwd(g: RelGraph, gO: torch.Tensor, relu_mask: Optional[torch.Tensor], 
     gx = None
     if need_x:
         gx = gx_out if gx_out is not None else torch.empty(g.n_src, d_in, dtype=torch.float32, device=dev)
-    gW = param_grad(K1, d_out, device=dev) if need_w else None
+    gW = None
+    if need_w:
+        gW = torch.empty(K1, d_out, dtype=torch.float32, device=dev) if scratch_w else param_grad(K1, d_out, device=dev)
     groot = param_grad(d_in, d_out, device=dev) if need_w else None
     gb = param_grad(d_out, device=dev) if (need_w and need_b) else None
     slot_ready = bool(sparse and slot is not None)
@@ -996,6 +999,50 @@ def basis_combine(comp: torch.Tensor, V: torch.Tensor) -> torch.Tensor:
     if comp.size(0) > 64 or comp.size(1) > 16 or V[0].numel() % 4:
         raise ValueError("basis_combine handles up to 64 relations, 16 bases and in * out a multiple of 4")
     return _BasisCombine.apply(comp, V)
+
+
+# ---- block-diagonal relation weights (RGCNConv(num_blocks = nb)) -----------------------------------------------------
+class _BlockDiag(torch.autograd.Function):
+    """W [R, nb * bi, nb * bo] = blockdiag(blocks[r, 0], .., blocks[r, nb - 1]) from blocks [R, nb, bi, bo], and its
+    backward (the diagonal blocks of the dense gradient), on ``rgcn_block_diag_expand`` / ``_gather``."""
+
+    @staticmethod
+    def forward(ctx, blocks):
+        lib = _lib.load()
+        b = blocks.detach().contiguous()
+        R, nb, bi, bo = b.shape
+        W = torch.empty(R, nb * bi, nb * bo, dtype=torch.float32, device=b.device)
+        _lib.check(lib.rgcn_block_diag_expand(_ptr(b), R, nb, bi, bo, _ptr(W), _stream(b.device)), "rgcn_block_diag_expand")
+        ctx.shape = (R, nb, bi, bo)
+        return W
+
+    @staticmethod
+    def backward(ctx, gW):
+        lib = _lib.load()
+        R, nb, bi, bo = ctx.shape
+        gW = gW.to(torch.float32).contiguous()
+        g = param_grad(R, nb, bi, bo, device=gW.device)
+        _lib.check(lib.rgcn_block_diag_gather(_ptr(gW), R, nb, bi, bo, _ptr(g), _stream(gW.device)), "rgcn_block_diag_gather")
+        return g
+
+
+def block_diag_weights(blocks: torch.Tensor) -> torch.Tensor:
+    """The dense [R, in, out] relation weights of a block-diagonal layer (differentiable).  The layer's backward writes
+    the dense weight gradient into scratch, not into the gradient arena: only the compact block gradient is a parameter
+    gradient (``is_grad_scratch``)."""
+    if not blocks.is_cuda:
+        raise RuntimeError("block_diag_weights needs CUDA tensors: there is no CPU implementation of this path")
+    if blocks.dim() != 4 or blocks.dtype != torch.float32:
+        raise ValueError("blocks must be a float32 [R, num_blocks, in / num_blocks, out / num_blocks] tensor")
+    W = _BlockDiag.apply(blocks)
+    W._rgcn_grad_scratch = True
+    return W
+
+
+def is_grad_scratch(W: torch.Tensor) -> bool:
+    """True for weights whose gradient is an intermediate (e.g. ``block_diag_weights``): a backward kernel writes it
+    into a plain tensor instead of a slice of the gradient arena, which is sized for the parameters alone."""
+    return bool(getattr(W, "_rgcn_grad_scratch", False))
 
 
 class _PairScores(torch.autograd.Function):
