@@ -239,6 +239,28 @@ int rgcn_aggregate_bwd_rows_marked(const rgcn_csr_t* gt, const rgcn_csr_t* g_fwd
                                    void* workspace, size_t workspace_bytes, rgcn_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Max aggregation (RGCNConv(aggr='max'), csrc/aggregate_max.cu).  Forward over the forward-orientation CSR g:
+ *   Hmax[i, r*d + c] = max_{e in seg(i, r)} X[col[e], c]     (NaN propagates; 0 for an empty segment)
+ *   Hcnt[i, r*d + c] = |{e in seg(i, r) : X[col[e], c] == Hmax}| + [Hmax == 0]
+ * = torch's zeros(..).scatter_reduce_(0, idx, src, 'amax', include_self=False) and the divisor of its backward (the zero
+ * initial value counts as a tie when the maximum is exactly 0).  Hmax is also written as the transform's operand planes
+ * (out_mode 1: bf16 hi plane, 2: hi + lo) with x_root (optional) appended as block R, like rgcn_aggregate_fwd.
+ * Backward over the TRANSPOSED CSR gt (no weights used), deterministic, no atomics:
+ *   gX[j] = init[j] + sum_r sum_{e: j -> i in seg_t(j, r)} [X[j] == Hmax[i, r]] * gH[i, r] / Hcnt[i, r]
+ * (and NaN where Hmax is NaN, as torch's backward gives).  init (optional): e.g. the root-term gradient.
+ * Segments longer than the hub threshold go through the orientation's hub plan (chunk partials reduced by whole blocks
+ * first: (max, ties) pairs forward, sums backward), into `workspace` of rgcn_aggregate_max_workspace_bytes(g, d,
+ * backward) bytes.  Deterministic; neither call allocates; both check their arguments before any CUDA call.
+ * ------------------------------------------------------------------------------------------ */
+size_t rgcn_aggregate_max_workspace_bytes(const rgcn_csr_t* g, int32_t d, int32_t backward);
+int rgcn_aggregate_max_fwd(const rgcn_csr_t* g, const float* X, int64_t ldx, int32_t d, void* H, void* H_lo, int64_t ldh,
+                           int32_t out_mode, const float* x_root, int64_t ld_x_root, float* Hmax, float* Hcnt, int64_t ldm,
+                           void* workspace, size_t workspace_bytes, rgcn_stream_t stream);
+int rgcn_aggregate_max_bwd(const rgcn_csr_t* gt, const float* gH, int64_t ldg, const float* Hmax, const float* Hcnt,
+                           int64_t ldm, const float* X, int64_t ldx, int32_t d, const float* init, int64_t ld_init,
+                           float* gX, int64_t ldgx, void* workspace, size_t workspace_bytes, rgcn_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Relational transform on the tensor cores (tcgen05.mma, fp32 accumulators in TMEM, every operand tile
  * streamed by TMA).  Replaces the R+1 matmuls `h_r @ W_r`, `x @ root` per layer of RGCNConv's loop path
  * (src/models/rgcn.py:123, :128) and their autograd transposes (src/train.py:306), concatenated

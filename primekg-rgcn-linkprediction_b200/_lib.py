@@ -105,6 +105,9 @@ PROTOTYPES = {
     "rgcn_aggregate_fwd": (C.c_int, [PCSR, p, i64, i32, p, i32, p, p, i64, i32, p, i64, p, p, i64, p, sz, p]),
     "rgcn_reduce_partials": (C.c_int, [p, i64, i32, p, p]),
     "rgcn_aggregate_bwd": (C.c_int, [PCSR, p, i64, i32, p, i64, p, i64, C.POINTER(MaskedPlanesOut), p, sz, p]),
+    "rgcn_aggregate_max_workspace_bytes": (sz, [PCSR, i32, i32]),
+    "rgcn_aggregate_max_fwd": (C.c_int, [PCSR, p, i64, i32, p, p, i64, i32, p, i64, p, p, i64, p, sz, p]),
+    "rgcn_aggregate_max_bwd": (C.c_int, [PCSR, p, i64, p, p, i64, p, i64, i32, p, i64, p, i64, p, sz, p]),
     "rgcn_aggregate_row_blocks": (i64, [PCSR, i32]),
     "rgcn_aggregate_fwd_rows": (C.c_int, [PCSR, p, i64, i32, p, p, i64, i32, p, i64, i64, i64, i32, p, sz, p]),
     "rgcn_weight_planes_bytes": (sz, [i32, i32]),

@@ -16,7 +16,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "librgcn_b200.so")
-SOURCES = ["lib.cu", "csr_build.cu", "aggregate.cu", "decoder.cu", "transform.cu", "rank.cu", "p2p.cu", "rowsparse.cu", "basis.cu", "layer.cu", "fused_layer.cu", "probe.cu", "optim.cu"]
+SOURCES = ["lib.cu", "csr_build.cu", "aggregate.cu", "aggregate_max.cu", "decoder.cu", "transform.cu", "rank.cu", "p2p.cu", "rowsparse.cu", "basis.cu", "layer.cu", "fused_layer.cu", "probe.cu", "optim.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xptxas=-v",

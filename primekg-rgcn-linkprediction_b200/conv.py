@@ -24,6 +24,15 @@ from .graph import RelGraph, get_graph
 
 
 MODES = ("fp32", "bf16")
+AGGRS = {"mean": "mean", "add": "sum", "sum": "sum", "max": "max"}     # PyG's names -> the walk that computes them
+
+
+def canonical_aggr(aggr) -> str:
+    """'mean', 'sum' (PyG's 'add' and 'sum' are aliases) or 'max'; anything else is a ValueError."""
+    if not isinstance(aggr, str) or aggr not in AGGRS:
+        raise ValueError(f"aggr must be one of {sorted(AGGRS)} (RGCNConv on sm_100a supports mean, sum and max "
+                         f"aggregation), got {aggr!r}")
+    return AGGRS[aggr]
 
 
 def default_mode() -> str:
@@ -138,6 +147,63 @@ class _RGCNLayerFn(torch.autograd.Function):
         return gx_src, gx_root, gW, groot, gb, None, None, None, None, None, None, None
 
 
+class _RGCNAggrLayerFn(torch.autograd.Function):
+    """The two-kernel layer for what the one-call layer (``_RGCNLayerFn``, K = (R+1) d_in, bias always) does not take:
+    ``aggr='max'`` with or without root / bias, and mean / sum layers without root or without bias.
+
+      forward : the walk writes H as planes into A[:, :R*d_in] (mean / sum: rgcn_aggregate_fwd over ``graph``, whose edge
+                weights select the sum; max: rgcn_aggregate_max_fwd, which also keeps the fp32 maxima and tie counts), x as
+                block R only when ``root`` exists; transform_fwd over K = R*d_in (+ d_in), bias in the epilogue if it exists.
+      backward: split_planes(gO, ReLU / dropout mask) -> G (+ bias column sums if there is a bias); dgrad -> gA; the
+                transposed walk (mean / sum: rgcn_aggregate_bwd; max: rgcn_aggregate_max_bwd) adds the root term
+                gA[:, R*d_in:] only when ``root`` exists; split-K wgrad -> grad W (, root) (, bias).
+    Unpartitioned graphs only (n_src == n_dst, x gathered and updated)."""
+
+    @staticmethod
+    def forward(ctx, x, W, root, bias, graph: RelGraph, relu: bool, mode: str, drop, aggr: str):
+        R, d_in, d_out = W.shape
+        x = x.contiguous()
+        if graph.n_src != graph.n_dst or x.size(0) != graph.n_dst:
+            raise ValueError("this layer form works on an unpartitioned graph")
+        K1, K2 = R * d_in, (d_in if root is not None else 0)
+        A = ops.alloc_planes(graph.n_dst, K1 + K2, mode, x.device)
+        x_root = x if root is not None else None
+        Hmax = Hcnt = None
+        if aggr == "max":
+            Hmax, Hcnt = ops.aggregate_max_fwd(graph, x, A, x_root=x_root)
+        else:
+            ops.aggregate_fwd(graph, x, planes=A, x_root=x_root)
+        p_drop, seed, ctr = drop if drop is not None else (0.0, 0, None)
+        out = ops.transform_fwd(A, K1, K2, W.reshape(K1, d_out), root, bias, relu, mode, p_drop, seed, ctr)
+        rowsparse.unmark_listed_output()
+        ctx.graph, ctx.relu, ctx.mode, ctx.p_drop, ctx.aggr = graph, relu, mode, p_drop, aggr
+        ctx.save_for_backward(A[0], A[1], W, root, out if relu else None, x if aggr == "max" else None, Hmax, Hcnt)
+        return out
+
+    @staticmethod
+    def backward(ctx, gO):
+        A_hi, A_lo, W, root, out, x, Hmax, Hcnt = ctx.saved_tensors
+        graph, mode = ctx.graph, ctx.mode
+        R, d_in, d_out = W.shape
+        K1, K2 = R * d_in, (d_in if root is not None else 0)
+        need_x, need_W, need_root, need_b = ctx.needs_input_grad[:4]
+        G = ops.alloc_planes(graph.n_dst, d_out, mode, gO.device)
+        colsum = ops.split_planes(gO.contiguous(), G, relu_mask=out, colsum=need_b, mask_scale=1.0 / (1.0 - ctx.p_drop))
+        gx = gW = groot = gb = None
+        if need_x:
+            Wd = W.detach()
+            gA = ops.transform_dgrad(G, d_out, Wd.reshape(K1, d_out), None if root is None else root.detach(), mode)
+            init = gA[:, K1:] if root is not None else None
+            if ctx.aggr == "max":
+                gx = ops.aggregate_max_bwd(graph, gA, Hmax, Hcnt, x, init=init)
+            else:
+                gx = ops.aggregate_bwd(graph, gA, d_in, init=init)
+        if need_W or need_root or need_b:
+            gWf, groot, gb = ops.transform_wgrad((A_hi, A_lo), K1, K2, G, d_out, colsum, mode)
+            gW = gWf.view(R, d_in, d_out)
+        return gx, gW, groot, gb, None, None, None, None, None
+
+
 class _RGCNBasisLayerFn(torch.autograd.Function):
     """Basis-decomposed layer in the B-accumulator ("Z") form:  out = [relu]( [Z | x] @ [V_1; ..; V_B; root] + bias ),
     Z_b = sum_r comp[r, b] * H_r(x)  — the same function as ``_RGCNLayerFn`` with W_r = sum_b comp[r, b] V_b, but the
@@ -219,11 +285,19 @@ def _glorot_(t: Optional[torch.Tensor]) -> None:
 class RGCNConv(nn.Module):
     """``num_bases`` = B: W_r = sum_b comp[r, b] weight[b].  ``num_blocks`` = nb: W_r = blockdiag(weight[r, 0], ..,
     weight[r, nb - 1]) with ``weight`` [R, nb, in / nb, out / nb] and no ``comp`` (PyG's two regularisers; at most one).
-    Both are materialised as the dense [R, in, out] W_r that the layer kernels consume (``relation_weights``)."""
+    Both are materialised as the dense [R, in, out] W_r that the layer kernels consume (``relation_weights``).
+
+    ``aggr``: 'mean' (default), 'add' / 'sum' (aliases) or 'max' — PyG's per-relation loop, h_r = aggr_{j in N_r(i)} x_j,
+    an empty segment giving 0; 'max' has torch's scatter_reduce('amax', include_self=False) semantics and gradient.
+    ``root_weight=False`` / ``bias=False``: no ``root`` / ``bias`` parameter (registered as None, as PyG does) and no such
+    term.  ``is_sorted`` is accepted and ignored (it only steers PyG's segment-matmul path)."""
 
     def __init__(self, in_channels: int, out_channels: int, num_relations: int, num_bases: Optional[int] = None,
-                 mode: Optional[str] = None, num_blocks: Optional[int] = None):
+                 mode: Optional[str] = None, num_blocks: Optional[int] = None, aggr: str = "mean",
+                 root_weight: bool = True, is_sorted: bool = False, bias: bool = True):
         super().__init__()
+        self._aggr = canonical_aggr(aggr)
+        self.aggr, self.root_weight, self.is_sorted = aggr, bool(root_weight), bool(is_sorted)
         if num_bases is not None and num_blocks is not None:
             raise ValueError("can not apply both basis-decomposition and block-diagonal-decomposition at the same time")
         if num_blocks is not None and (num_blocks < 1 or in_channels % num_blocks or out_channels % num_blocks):
@@ -245,16 +319,23 @@ class RGCNConv(nn.Module):
         else:
             self.weight = nn.Parameter(torch.empty(num_relations, in_channels, out_channels))
             self.register_parameter("comp", None)
-        self.root = nn.Parameter(torch.empty(in_channels, out_channels))
-        self.bias = nn.Parameter(torch.empty(out_channels))
+        if root_weight:
+            self.root = nn.Parameter(torch.empty(in_channels, out_channels))
+        else:
+            self.register_parameter("root", None)
+        if bias:
+            self.bias = nn.Parameter(torch.empty(out_channels))
+        else:
+            self.register_parameter("bias", None)
         self.reset_parameters()
 
     def reset_parameters(self) -> None:
         _glorot_(self.weight)
         _glorot_(self.comp)
         _glorot_(self.root)
-        with torch.no_grad():
-            self.bias.zero_()
+        if self.bias is not None:
+            with torch.no_grad():
+                self.bias.zero_()
 
     def relation_weights(self) -> torch.Tensor:
         """[R, d_in, d_out]; with bases W_r = sum_b comp[r, b] V_b, with blocks the block-diagonal W_r (differentiable)."""
@@ -294,6 +375,13 @@ class RGCNConv(nn.Module):
         if dropout_p > 0.0 and not relu:
             raise ValueError("the fused dropout follows the fused ReLU; use nn.Dropout for other placements")
         drop = self.dropout_state(dropout_p, x.device) if dropout_p > 0.0 else None
+        mode = self.mode or default_mode()
+        if self._aggr == "max" or self.root is None or self.bias is None:
+            # max, or a missing root / bias term: the two-kernel layer (no Z form, no listed rows, no bf16 gather)
+            return _RGCNAggrLayerFn.apply(x, self.relation_weights(), self.root, self.bias, graph.for_aggr(self._aggr),
+                                          relu, mode, drop, self._aggr)
+        if self._aggr != "mean":
+            graph = graph.for_aggr(self._aggr)
         if self._use_z_form(graph):
             return _RGCNBasisLayerFn.apply(x, self.weight, self.comp, self.root, self.bias, graph, relu,
                                            self.mode or default_mode(), drop)
@@ -321,5 +409,12 @@ class RGCNConv(nn.Module):
         return self.forward_graph(x, graph)
 
     def extra_repr(self) -> str:
-        return (f"{self.in_channels}, {self.out_channels}, num_relations={self.num_relations}, "
-                f"num_bases={self.num_bases}" + (f", num_blocks={self.num_blocks}" if self.num_blocks is not None else ""))
+        s = (f"{self.in_channels}, {self.out_channels}, num_relations={self.num_relations}, "
+             f"num_bases={self.num_bases}" + (f", num_blocks={self.num_blocks}" if self.num_blocks is not None else ""))
+        if self._aggr != "mean":
+            s += f", aggr={self.aggr!r}"
+        if not self.root_weight:
+            s += ", root_weight=False"
+        if self.bias is None:
+            s += ", bias=False"
+        return s

@@ -245,10 +245,10 @@ constexpr int agg_min_blocks(int G, int vpl, int mix, bool w) {
 // MARK (row-sparse backward only): rows whose row_flag byte is zero leave at once — a separate instantiation, so that the
 // unmarked walk keeps its register allocation (with the test compiled in, the d = 256 row-sparse walk spilled: 33 -> 66 us)
 template <int G, int VPL, int MIX, bool W, bool SLOT = false, bool MP = false, bool LIST = false, bool MARK = false>
-__global__ void __launch_bounds__(256, LIST ? (VPL > 2 ? 1 : 3) : agg_min_blocks(G, VPL, MIX, W) - (((MP || MARK) && agg_min_blocks(G, VPL, MIX, W) > 1) ? 1 : 0))
+__global__ void __launch_bounds__(256, LIST ? (VPL > 2 ? 1 : (W ? 2 : 3)) : agg_min_blocks(G, VPL, MIX, W) - (((MP || MARK) && agg_min_blocks(G, VPL, MIX, W) > 1) ? 1 : 0))
 aggregate_rows_kernel(const AggParams p) {
   static_assert(!MARK || (SLOT && !MP && MIX == MIX_SUM), "marked sources serve the row-sparse backward walk");
-  static_assert(!LIST || (MIX == MIX_NONE && !W && !SLOT && !MP), "the listed-rows walk is the unmixed forward form");
+  static_assert(!LIST || (MIX == MIX_NONE && !SLOT && !MP), "the listed-rows walk is the unmixed forward form");
   pdl_enter();
   constexpr int GROUPS = 256 / G;
   constexpr int NB = (MIX == MIX_BASIS) ? kMaxBasis : 1;
@@ -827,7 +827,17 @@ __device__ __forceinline__ uint4 pack_bf8(const f8& a) {
   return o;
 }
 
-template <int G, int VPL>
+// fma of 8 bf16 features by an edge weight (the weighted form: unit weights of a sum layer give the sum's bits)
+__device__ __forceinline__ void fma_bf8(f8& a, float w, const uint4& r) {
+  const uint32_t x[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    a.v[2 * i] = fmaf(w, __uint_as_float(x[i] << 16), a.v[2 * i]);
+    a.v[2 * i + 1] = fmaf(w, __uint_as_float(x[i] & 0xffff0000u), a.v[2 * i + 1]);
+  }
+}
+
+template <int G, int VPL, bool W = false>
 __global__ void __launch_bounds__(256) hub_partial_bf16_kernel(const AggParams p) {
   pdl_enter();
   constexpr int GROUPS = 256 / G;
@@ -858,24 +868,33 @@ __global__ void __launch_bounds__(256) hub_partial_bf16_kernel(const AggParams p
   static_assert(PER <= G, "a group's slice of a hub chunk must fit its lanes");
   const unsigned gmask = (G == 32) ? 0xffffffffu : (((1u << G) - 1u) << ((threadIdx.x & 31) / G * G));
   const int my_j = (lane < PER && g_beg + lane < g_end) ? __ldg(p.idx + g_beg + lane) : 0;     // one coalesced index load
+  const float my_w = (W && lane < PER && g_beg + lane < g_end) ? __ldg(p.edge_w + g_beg + lane) : 0.f;
   int e = g_beg;
   for (; e + U <= g_end; e += U) {
     uint4 v[U][VPL];
+    float w[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int j = __shfl_sync(gmask, my_j, e + u - g_beg, G);
+      if (W) w[u] = __shfl_sync(gmask, my_w, e + u - g_beg, G);
 #pragma unroll
       for (int k = 0; k < VPL; ++k) ld_bf8(F + (size_t)j * p.ldf + vcol[k], v[u][k]);
     }
 #pragma unroll
     for (int u = 0; u < U; ++u)
 #pragma unroll
-      for (int k = 0; k < VPL; ++k) acc_bf8(acc[k], v[u][k]);
+      for (int k = 0; k < VPL; ++k) {
+        if (W) fma_bf8(acc[k], w[u], v[u][k]); else acc_bf8(acc[k], v[u][k]);
+      }
   }
   for (; e < g_end; ++e) {
     const int j = __shfl_sync(gmask, my_j, e - g_beg, G);
+    const float wv = W ? __shfl_sync(gmask, my_w, e - g_beg, G) : 1.f;
 #pragma unroll
-    for (int k = 0; k < VPL; ++k) { uint4 r; ld_bf8(F + (size_t)j * p.ldf + vcol[k], r); acc_bf8(acc[k], r); }
+    for (int k = 0; k < VPL; ++k) {
+      uint4 r; ld_bf8(F + (size_t)j * p.ldf + vcol[k], r);
+      if (W) fma_bf8(acc[k], wv, r); else acc_bf8(acc[k], r);
+    }
   }
 #pragma unroll
   for (int k = 0; k < VPL; ++k)
@@ -889,8 +908,8 @@ __global__ void __launch_bounds__(256) hub_partial_bf16_kernel(const AggParams p
   }
 }
 
-template <int G, int VPL, bool LIST = false>
-__global__ void __launch_bounds__(256, (VPL == 1 ? 4 : 3)) aggregate_rows_bf16_kernel(const AggParams p) {
+template <int G, int VPL, bool LIST = false, bool W = false>
+__global__ void __launch_bounds__(256, (VPL == 1 ? 4 : 3) - (W ? 1 : 0)) aggregate_rows_bf16_kernel(const AggParams p) {
   pdl_enter();
   constexpr int GROUPS = 256 / G;
   constexpr int U0 = VPL >= 2 ? 4 : 8;
@@ -955,10 +974,15 @@ __global__ void __launch_bounds__(256, (VPL == 1 ? 4 : 3)) aggregate_rows_bf16_k
   }
   const int row_end = __ldg(rowptr + R);
   int wbase = -(1 << 30), wi0 = 0, wi1 = 0;
+  float ww0 = 1.f, ww1 = 1.f;
   auto refill = [&](int e) {
     wbase = e;
     wi0 = (e + lane < row_end) ? __ldg(idx + e + lane) : 0;
     wi1 = (e + G + lane < row_end) ? __ldg(idx + e + G + lane) : 0;
+    if (W) {
+      ww0 = (e + lane < row_end) ? __ldg(p.edge_w + e + lane) : 0.f;
+      ww1 = (e + G + lane < row_end) ? __ldg(p.edge_w + e + G + lane) : 0.f;
+    }
   };
   for (int rbase = r_lo; rbase < r_hi; rbase += G) {
     const int rl = rbase + lane;
@@ -998,17 +1022,21 @@ __global__ void __launch_bounds__(256, (VPL == 1 ? 4 : 3)) aggregate_rows_bf16_k
           constexpr int UB = decltype(ub)::value;
           if (e + UB > wbase + 2 * G) refill(e);
           uint4 v[UB][VPL];
+          float w[UB];
 #pragma unroll
           for (int u = 0; u < UB; ++u) {
             const int off = e + u - wbase;
             const int j = __shfl_sync(gmask, (off & G) ? wi1 : wi0, off & (G - 1), G);
+            if (W) w[u] = __shfl_sync(gmask, (off & G) ? ww1 : ww0, off & (G - 1), G);
 #pragma unroll
             for (int k = 0; k < VPL; ++k) ld_bf8(F + (size_t)j * ldf + vcol[k], v[u][k]);
           }
 #pragma unroll
           for (int u = 0; u < UB; ++u)
 #pragma unroll
-            for (int k = 0; k < VPL; ++k) acc_bf8(acc[k], v[u][k]);
+            for (int k = 0; k < VPL; ++k) {
+              if (W) fma_bf8(acc[k], w[u], v[u][k]); else acc_bf8(acc[k], v[u][k]);
+            }
           e += UB;
         };
         while (e + U <= end) batch(std::integral_constant<int, U>{});
@@ -1016,7 +1044,7 @@ __global__ void __launch_bounds__(256, (VPL == 1 ? 4 : 3)) aggregate_rows_bf16_k
         if (U > 2 && e + 2 <= end) batch(std::integral_constant<int, (U > 2 ? 2 : 1)>{});
         if (e < end) batch(std::integral_constant<int, 1>{});
       }
-      if (len > 1) {
+      if (!W && len > 1) {
         const float c = (float)len;                   // s / clamp(cnt, 1): a true division, like the reference
         const float rc = __frcp_rn(c);
 #pragma unroll
@@ -1036,14 +1064,20 @@ static int launch_agg_bf16(AggParams p, int n_chunks, cudaStream_t st) {
   constexpr int GROUPS = 256 / G;
   if (!p.range_mode) { p.row_begin = 0; p.row_end = p.n_rows; }
   if (n_chunks > 0 && !p.no_hub_pass) {
-    RGCN_CUDA(launch_pdl(hub_partial_bf16_kernel<G, VPL>, dim3(n_chunks), dim3(256), 0, st, p));
+    if (p.edge_w) RGCN_CUDA(launch_pdl(hub_partial_bf16_kernel<G, VPL, true>, dim3(n_chunks), dim3(256), 0, st, p));
+    else RGCN_CUDA(launch_pdl(hub_partial_bf16_kernel<G, VPL>, dim3(n_chunks), dim3(256), 0, st, p));
     RGCN_LAUNCH_CHECK();
   }
   const int64_t n_walk = p.row_end - p.row_begin;
   if (n_walk <= 0) return RGCN_OK;
-  if (p.list) RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL, true>, dim3((unsigned)((n_walk + GROUPS - 1) / GROUPS), (unsigned)(p.list_slices > 0 ? p.list_slices : 1),
-                                   (unsigned)(p.list_rsplit > 0 ? p.list_rsplit : 1)), dim3(256), 0, st, p));
-  else RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL>, dim3((unsigned)((n_walk + GROUPS - 1) / GROUPS)), dim3(256), 0, st, p));
+  const dim3 lgrid((unsigned)((n_walk + GROUPS - 1) / GROUPS), (unsigned)(p.list_slices > 0 ? p.list_slices : 1),
+                   (unsigned)(p.list_rsplit > 0 ? p.list_rsplit : 1));
+  const dim3 grid((unsigned)((n_walk + GROUPS - 1) / GROUPS));
+  // a weighted CSR (RGCNConv(aggr='sum'): unit weights) takes the weighted instantiations, the mean's are unchanged
+  if (p.list && p.edge_w) RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL, true, true>, lgrid, dim3(256), 0, st, p));
+  else if (p.list) RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL, true>, lgrid, dim3(256), 0, st, p));
+  else if (p.edge_w) RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL, false, true>, grid, dim3(256), 0, st, p));
+  else RGCN_CUDA(launch_pdl(aggregate_rows_bf16_kernel<G, VPL>, grid, dim3(256), 0, st, p));
   RGCN_LAUNCH_CHECK();
   return RGCN_OK;
 }
@@ -1121,11 +1155,12 @@ static int launch_agg(const AggParams& p_in, int mix, int n_chunks, cudaStream_t
     return w ? launch_agg_overlapped<G, VPL, MIX_SUM, true>(p, n_chunks, st) : launch_agg_overlapped<G, VPL, MIX_SUM, false>(p, n_chunks, st);
   }
   if (p.list) {
-    // listed-rows walk: forward, unmixed, unweighted (the last layer of a link-prediction step)
-    if (mix != MIX_NONE || p.edge_w || p.slot || p.mp_hi) { set_error("aggregate: the listed-rows walk serves the unmixed forward only"); return RGCN_EINVAL; }
+    // listed-rows walk: forward, unmixed (the last layer of a link-prediction step); a weighted CSR (RGCNConv(aggr='sum'):
+    // unit weights) takes the weighted instantiations, the mean's are unchanged
+    if (mix != MIX_NONE || p.slot || p.mp_hi) { set_error("aggregate: the listed-rows walk serves the unmixed forward only"); return RGCN_EINVAL; }
     const dim3 lgrid((unsigned)((n_walk + GROUPS - 1) / GROUPS), (unsigned)(p.list_slices > 0 ? p.list_slices : 1),
                      (unsigned)(p.list_rsplit > 0 ? p.list_rsplit : 1));
-    ForkJoin* fj = (p.list_overlap_hubs && n_chunks > 0 && n_walk > 0 && p.list_slices <= 1) ? fork_join_existing(st) : nullptr;
+    ForkJoin* fj = (p.list_overlap_hubs && !p.edge_w && n_chunks > 0 && n_walk > 0 && p.list_slices <= 1) ? fork_join_existing(st) : nullptr;
     if (fj) {
       // hub chunks on the side stream, the walk (without the hub segments) on this one, then the finish kernel
       RGCN_CUDA(cudaEventRecord(fj->fork, st));
@@ -1142,11 +1177,13 @@ static int launch_agg(const AggParams& p_in, int mix, int n_chunks, cudaStream_t
       return RGCN_OK;
     }
     if (n_chunks > 0) {
-      RGCN_CUDA(launch_pdl(hub_partial_kernel<G, VPL, false>, dim3(n_chunks), dim3(256), 0, st, p));
+      if (p.edge_w) RGCN_CUDA(launch_pdl(hub_partial_kernel<G, VPL, true>, dim3(n_chunks), dim3(256), 0, st, p));
+      else RGCN_CUDA(launch_pdl(hub_partial_kernel<G, VPL, false>, dim3(n_chunks), dim3(256), 0, st, p));
       RGCN_LAUNCH_CHECK();
     }
     if (n_walk <= 0) return RGCN_OK;
-    RGCN_CUDA(launch_pdl(aggregate_rows_kernel<G, VPL, MIX_NONE, false, false, false, true>, lgrid, dim3(256), 0, st, p));
+    if (p.edge_w) RGCN_CUDA(launch_pdl(aggregate_rows_kernel<G, VPL, MIX_NONE, true, false, false, true>, lgrid, dim3(256), 0, st, p));
+    else RGCN_CUDA(launch_pdl(aggregate_rows_kernel<G, VPL, MIX_NONE, false, false, false, true>, lgrid, dim3(256), 0, st, p));
     RGCN_LAUNCH_CHECK();
     return RGCN_OK;
   }
@@ -1355,7 +1392,7 @@ extern "C" int rgcn_aggregate_fwd_bf16(const rgcn_csr_t* g, const void* X16, int
                                             (row_end % g->order_chunk_rows == 0 || row_end == g->n_rows)),
                  "aggregate_fwd_bf16: with a row order the range must consist of whole order chunks");
   AggParams p{};
-  p.rowptr = g->rowptr; p.idx = g->idx;
+  p.rowptr = g->rowptr; p.idx = g->idx; p.edge_w = g->w;
   p.hub_keys = g->hub_keys; p.hub_chunk_ptr = g->hub_chunk_ptr; p.n_hubs = g->n_hubs; p.chunk_table = g->chunk_table;
   p.row_order = g->row_order; p.hub_threshold = g->hub_threshold;
   p.n_rows = g->n_rows; p.R = g->R;
@@ -1497,6 +1534,7 @@ static int aggregate_fwd_list_impl(const rgcn_csr_t* g, const void* X, int64_t l
   p.F = (const float*)X; p.ldf = ldx; p.src_rel_stride = 0; p.d = d; p.block_stride = d;
   p.O = H; p.O_lo = H_lo; p.ldo = ldh; p.out_mode = out_mode; p.partials = (float*)workspace;
   p.root_rows = (const float*)x_root; p.ld_root = ld_x_root;
+  p.edge_w = g->w;                                   // unit weights of a sum layer: the weighted instantiations
   p.list = rows; p.n_list = n_list; p.hub_filter = slot; p.hub_unlisted = (int32_t)m_c;
   // by rows (degree order, unlisted rows leave at once) while the row count is moderate; by list positions beyond
   static int env_by_rows = -1;
@@ -1525,7 +1563,7 @@ static int aggregate_fwd_list_impl(const rgcn_csr_t* g, const void* X, int64_t l
   if (env_overlap < 0) { const char* e = getenv("RGCN_LIST_OVERLAP_HUBS"); env_overlap = e ? atoi(e) : 0; }
   static int env_slice0 = -1;
   if (env_slice0 < 0) { const char* e = getenv("RGCN_LIST_SLICE"); env_slice0 = e ? atoi(e) : 0; }
-  if (!x_bf16 && env_overlap && env_slice0 == 0 && g->n_chunks > 0) {
+  if (!x_bf16 && !g->w && env_overlap && env_slice0 == 0 && g->n_chunks > 0) {
     cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
     const bool capturing = cudaStreamIsCapturing(st, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusActive;
     if (!capturing) (void)fork_join_existing(st);   // (the side stream is made by the first eager call: GraphedTrainStep and

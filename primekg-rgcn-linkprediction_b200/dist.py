@@ -23,7 +23,7 @@ import torch
 import torch.distributed as dist
 import torch.nn as nn
 
-from .conv import RGCNConv, _RGCNLayerFn, default_mode
+from .conv import RGCNConv, _RGCNLayerFn, canonical_aggr, default_mode
 from . import ops
 from .graph import RelGraph
 
@@ -138,14 +138,16 @@ class PartitionedRGCN(nn.Module):
 
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, num_bases: Optional[int] = None, num_layers: int = 2,
-                 seed: int = 42, num_blocks: Optional[int] = None):
+                 seed: int = 42, num_blocks: Optional[int] = None, aggr: str = "mean"):
         super().__init__()
+        if canonical_aggr(aggr) == "max":
+            raise ValueError("the partitioned encoder supports aggr='mean' and 'sum' (no max backward across shards)")
         self.plan, self.rank, self.num_relations = plan, rank, num_relations
         self.n_local = plan.size(rank)
         g = torch.Generator().manual_seed(seed)
         dims = [embedding_dim] + [hidden_dim] * num_layers
         self.convs = nn.ModuleList(RGCNConv(dims[i], dims[i + 1], num_relations, num_bases=num_bases,
-                                            num_blocks=num_blocks) for i in range(num_layers))
+                                            num_blocks=num_blocks, aggr=aggr) for i in range(num_layers))
         for conv in self.convs:                       # identical replicated weights on every rank (glorot on the last two dims)
             for prm in (conv.weight, conv.comp, conv.root):
                 if prm is not None:
@@ -183,7 +185,8 @@ class PartitionedRGCN(nn.Module):
             drop = conv.dropout_state(p, x.device) if 0.0 < p < 1.0 else None
             # the mask is keyed by global node id, as on one GPU (padding rows share ids with the next shard's first rows:
             # harmless, no edge and no decoder reads a padding row)
-            x = _RGCNLayerFn.apply(x_full, x, W, root, bias, self.graph, li != last, conv.mode or default_mode(), drop,
+            x = _RGCNLayerFn.apply(x_full, x, W, root, bias, self.graph if conv._aggr == "mean" else self.graph.for_aggr(conv._aggr),
+                                   li != last, conv.mode or default_mode(), drop,
                                    None, None, self.plan.bounds[self.rank])
             if li != last and p > 0.0 and drop is None:
                 x = self.dropout(x)
@@ -205,12 +208,12 @@ class PartitionedModel(nn.Module):
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, decoder_dropout: float = 0.0,
                  num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42,
-                 num_blocks: Optional[int] = None):
+                 num_blocks: Optional[int] = None, aggr: str = "mean"):
         super().__init__()
         from .modules import LinkPredictor
         self.plan = plan
         self.encoder = PartitionedRGCN(plan, rank, num_relations, embedding_dim, hidden_dim, dropout, num_bases,
-                                       num_layers, seed, num_blocks=num_blocks)
+                                       num_layers, seed, num_blocks=num_blocks, aggr=aggr)
         state = torch.random.get_rng_state()
         torch.manual_seed(seed + 12345)                       # identical decoder on every rank
         self.decoder = LinkPredictor(num_relations, hidden_dim, decoder_dropout)

@@ -282,9 +282,10 @@ class FusedPartitionedRGCN(PartitionedRGCN):
                 raise ValueError("fused dropout needs p < 1")
             drops.append(conv.dropout_state(p, self.node_embeddings.device) if p > 0.0 else None)
         mode = self.convs[0].mode or default_mode()
+        aggr = self.convs[0]._aggr
         if read_ids is not None and not (torch.is_grad_enabled() and listed_last_layer()):
             read_ids = None
-        return _FusedEncoderFn.apply(self._exchange(), self.graph, mode, drops, read_ids, self.node_embeddings, *params)
+        return _FusedEncoderFn.apply(self._exchange(), self.graph if aggr == "mean" else self.graph.for_aggr(aggr), mode, drops, read_ids, self.node_embeddings, *params)
 
 
 class FusedPartitionedModel(nn.Module):
@@ -293,12 +294,12 @@ class FusedPartitionedModel(nn.Module):
     def __init__(self, plan: PartitionPlan, rank: int, num_relations: int, embedding_dim: int = 64,
                  hidden_dim: int = 128, dropout: float = 0.5, decoder_dropout: float = 0.0,
                  num_bases: Optional[int] = None, num_layers: int = 2, seed: int = 42,
-                 num_blocks: Optional[int] = None):
+                 num_blocks: Optional[int] = None, aggr: str = "mean"):
         super().__init__()
         from .modules import LinkPredictor
         self.plan = plan
         self.encoder = FusedPartitionedRGCN(plan, rank, num_relations, embedding_dim, hidden_dim, dropout, num_bases,
-                                            num_layers, seed, num_blocks=num_blocks)
+                                            num_layers, seed, num_blocks=num_blocks, aggr=aggr)
         state = torch.random.get_rng_state()
         torch.manual_seed(seed + 12345)                       # identical decoder on every rank
         self.decoder = LinkPredictor(num_relations, hidden_dim, decoder_dropout)

@@ -171,6 +171,26 @@ class RelGraph:
             self.bwd = _Orientation(self.rowptr_t, self.row_t, self.w_t, n_src, R, E)
         del ws
 
+    def for_aggr(self, aggr: str) -> "RelGraph":
+        """The graph as the layer kernels see it for aggregation ``aggr``: itself for 'mean' and 'max'; for 'sum' a view
+        (made once, kept) whose two orientations carry unit edge weights.  The weighted walks then compute the plain
+        segment sum: fma(1, v, s) rounds exactly like s + v, so the forward equals index_add_ in edge order, and the
+        transposed walk is the sum's backward."""
+        if aggr != "sum":
+            return self
+        views = self.__dict__.setdefault("_views", {})
+        v = views.get(aggr)
+        if v is None:
+            v = RelGraph.__new__(RelGraph)
+            v.__dict__.update({k: val for k, val in self.__dict__.items() if k != "_views"})
+            ones = torch.ones(max(self.E, 1), dtype=torch.float32, device=self.device)
+            with torch.cuda.device(self.device):
+                v.fwd = _Orientation(self.rowptr, self.col, ones, self.n_dst, self.R, self.E)
+                v.bwd = _Orientation(self.rowptr_t, self.row_t, ones, self.n_src, self.R, self.E)
+            v.unit_w = ones
+            views[aggr] = v
+        return v
+
     @classmethod
     def from_edges(cls, edge_index: torch.Tensor, edge_type: torch.Tensor, num_nodes: int, num_relations: int):
         if edge_index.dim() != 2 or edge_index.size(0) != 2:

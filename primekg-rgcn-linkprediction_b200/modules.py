@@ -43,7 +43,7 @@ class DrugDiseaseRGCN(nn.Module):
 
     def __init__(self, num_nodes: int, num_relations: int, embedding_dim: int = 64, hidden_dim: int = 128,
                  dropout: float = 0.5, num_bases: Optional[int] = None, num_layers: int = 2,
-                 num_blocks: Optional[int] = None):
+                 num_blocks: Optional[int] = None, aggr: str = "mean"):
         super().__init__()
         self.num_nodes = num_nodes
         self.num_relations = num_relations
@@ -51,7 +51,7 @@ class DrugDiseaseRGCN(nn.Module):
         self.hidden_dim = hidden_dim
         # construction order = the reference's, so a seeded init draws the same random stream
         self.node_embeddings = nn.Embedding(num_nodes, embedding_dim)
-        dec = dict(num_bases=num_bases, num_blocks=num_blocks)
+        dec = dict(num_bases=num_bases, num_blocks=num_blocks, aggr=aggr)       # aggr: every layer's aggregation
         self.conv1 = RGCNConv(embedding_dim, hidden_dim, num_relations, **dec)
         self.conv2 = RGCNConv(hidden_dim, hidden_dim, num_relations, **dec)
         if num_layers > 2:
@@ -293,14 +293,14 @@ class DrugDiseaseModel(nn.Module):
 
     def __init__(self, num_nodes: int, num_relations: int, embedding_dim: int = 64, hidden_dim: int = 128,
                  dropout: float = 0.5, decoder_dropout: float = 0.0, num_bases: Optional[int] = None,
-                 num_layers: int = 2, num_blocks: Optional[int] = None):
+                 num_layers: int = 2, num_blocks: Optional[int] = None, aggr: str = "mean"):
         super().__init__()
         self.num_nodes = num_nodes
         self.num_relations = num_relations
         self.hidden_dim = hidden_dim
         self.encoder = DrugDiseaseRGCN(num_nodes=num_nodes, num_relations=num_relations,
                                        embedding_dim=embedding_dim, hidden_dim=hidden_dim, dropout=dropout,
-                                       num_bases=num_bases, num_layers=num_layers, num_blocks=num_blocks)
+                                       num_bases=num_bases, num_layers=num_layers, num_blocks=num_blocks, aggr=aggr)
         self.decoder = LinkPredictor(num_relations=num_relations, embedding_dim=hidden_dim, dropout=decoder_dropout)
 
     def forward(self, edge_index, edge_type, head_indices, tail_indices, relation_types) -> torch.Tensor:

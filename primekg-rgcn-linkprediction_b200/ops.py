@@ -191,6 +191,57 @@ def aggregate_bwd(g: RelGraph, gH: torch.Tensor, d: int, init: Optional[torch.Te
     return gX
 
 
+def aggregate_max_fwd(g: RelGraph, x: torch.Tensor, planes, x_root: Optional[torch.Tensor] = None):
+    """Max aggregation (``rgcn_aggregate_max_fwd``): writes H[i, r] = max_{j in N_r(i)} x[j] (0 for an empty segment) as
+    bf16 planes into the first R*d columns of ``planes`` = (hi, lo | None), x_root appended as block R when given, and
+    returns (Hmax, Hcnt) fp32 [n_dst, R*d]: the maxima and the tie counts the backward divides by."""
+    lib = _lib.load()
+    x = _f32c(x, "x")
+    if x.size(0) != g.n_src:
+        raise ValueError(f"x has {x.size(0)} rows, the graph gathers from {g.n_src}")
+    d = x.size(1)
+    hi, lo = planes
+    if hi.dtype != torch.bfloat16 or hi.size(0) != g.n_dst or hi.stride(1) != 1 or \
+            hi.size(1) < (g.R + (x_root is not None)) * d:
+        raise ValueError("planes must be bf16 [n_dst, >= R*d (+ d with x_root)] row-major")
+    if x_root is not None:
+        x_root = _f32c(x_root, "x_root")
+        if x_root.shape != (g.n_dst, d):
+            raise ValueError("x_root must be [n_dst, d]")
+    Hmax = torch.empty(g.n_dst, g.R * d, dtype=torch.float32, device=x.device)
+    Hcnt = torch.empty_like(Hmax)
+    ws = g.fwd.workspace(2 * d)                    # (max, ties) chunk partials of the hub segments
+    _lib.check(lib.rgcn_aggregate_max_fwd(g.fwd.ref, _ptr(x), x.stride(0), d, _ptr(hi), _ptr(lo), hi.stride(0),
+                                          2 if lo is not None else 1, _ptr(x_root), 0 if x_root is None else x_root.stride(0),
+                                          _ptr(Hmax), _ptr(Hcnt), Hmax.stride(0), _ptr(ws), 0 if ws is None else ws.numel() * 4,
+                                          _stream(x.device)), "rgcn_aggregate_max_fwd")
+    return Hmax, Hcnt
+
+
+def aggregate_max_bwd(g: RelGraph, gH: torch.Tensor, Hmax: torch.Tensor, Hcnt: torch.Tensor, x: torch.Tensor,
+                      init: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """gX[j] = init[j] + sum_r sum_{(j->i, r)} [x[j] == Hmax[i, r]] gH[i, r] / Hcnt[i, r] over the transposed CSR
+    (``rgcn_aggregate_max_bwd``; deterministic; NaN where Hmax is NaN, as torch's backward gives)."""
+    lib = _lib.load()
+    gH, x = _f32c(gH, "gH"), _f32c(x, "x")
+    d = x.size(1)
+    if gH.size(0) != g.n_dst or gH.size(1) < g.R * d or Hmax.shape != (g.n_dst, g.R * d) or Hcnt.shape != Hmax.shape:
+        raise ValueError("gH, Hmax and Hcnt must be [n_dst, R*d]")
+    if x.size(0) != g.n_src:
+        raise ValueError("x must be the layer input [n_src, d]")
+    if init is not None:
+        init = _f32c(init, "init")
+        if init.size(0) != g.n_src or init.size(1) < d:
+            raise ValueError("init must be [n_src, >= d]")
+    gX = torch.empty(g.n_src, d, dtype=torch.float32, device=x.device)
+    ws = g.bwd.workspace(d)
+    _lib.check(lib.rgcn_aggregate_max_bwd(g.bwd.ref, _ptr(gH), gH.stride(0), _ptr(Hmax), _ptr(Hcnt), Hmax.stride(0),
+                                          _ptr(x), x.stride(0), d, _ptr(init), 0 if init is None else init.stride(0),
+                                          _ptr(gX), gX.stride(0), _ptr(ws), 0 if ws is None else ws.numel() * 4,
+                                          _stream(x.device)), "rgcn_aggregate_max_bwd")
+    return gX
+
+
 def masked_planes_struct(mask: torch.Tensor, scale: float, planes, colsum: Optional[torch.Tensor]):
     """``rgcn_masked_planes_out`` for (mask, scale, (hi, lo | None), colsum | None); the tensors must outlive the call."""
     if _f32c(mask, "mask") is not mask:
